@@ -5,6 +5,7 @@
     python bench.py --gpus 1 --steps K --warmup W                  # this repo's CUDA path
     python bench.py --impl reference --gpus 1 --steps K --warmup W # the restated reference CPU path (oracle)
     torchrun ... bench.py --gpus N ...                             # one rank per GPU, env shards, no data-path collective
+    python bench.py ... --dump-outputs DIR                         # also write what the last timed step computed, DIR/<name>.npy
 
 One bench "step" = ONE launch of the fused kernel advancing every env of the shard by STEPS_PER_LAUNCH env-steps
 on a synthetic action stream (config.workload says which). Prints ONE JSON line (rank 0).
@@ -33,6 +34,8 @@ STATE_BYTES_PER_ENV = 53       # 7 f32 + u64 brick mask + 4 u32 + 1 u8: read onc
 BYTES_PER_SAMPLE_U8 = 91744    # 5 frames read + 2 x 4 frames written + 16 B scalars
 BYTES_PER_SAMPLE_F32 = 261088  # 5 frames read + 2 x 4 f32 frames written + 16 B scalars
 SEED = 20261018
+SETTLE_LAUNCHES = 1000         # untimed launches after the warm-up: 0.29 s of the default config (0.286 ms per launch, B200 at a 1,000 W power limit)
+DUMP_OBS_ENVS = 256            # --dump-outputs: envs whose observation stacks are written, 256 x 112,896 B of f32
 QNET_FLOP_PER_OBS = 2 * (400 * 32 * 256 + 81 * 64 * 512 + 49 * 64 * 576 + 512 * 3136 + 3 * 512)   # 84x84x4 -> conv 8/4, 4/2, 3/1 -> 512 -> 3
 
 
@@ -206,11 +209,11 @@ def run_b200(args, rank, local_rank, world):
     for _ in range(max(args.warmup, 3)):
         launch()
     torch.cuda.synchronize()
-    t_warm = time.time()                      # a few launches are ~1 ms: keep warming (untimed) until clocks have settled
-    while time.time() - t_warm < 0.25:
-        for _ in range(10):
-            launch()
-        torch.cuda.synchronize()
+    # a few launches are ~1 ms: keep warming (untimed) until clocks have settled. A fixed count of launches, not a fixed time, so that
+    # the timed launches start from the same env state in every run and on every build, and compute the same outputs (--dump-outputs).
+    for _ in range(SETTLE_LAUNCHES):
+        launch()
+    torch.cuda.synchronize()
     reduce_stats()
     # ---- timed region: exactly K launches, device resident inputs ----
     barrier()
@@ -225,6 +228,8 @@ def run_b200(args, rank, local_rank, world):
         t = torch.tensor([ms], dtype=torch.float64, device=dev)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         ms = float(t.item())
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, q, torch, env, reward, done, dev, stream)
     # keep the GPU loaded for the clock sampler if the timed region was short (untimed, same launches)
     t_load = time.time()
     while sampler and time.time() - t_load < 1.0:
@@ -338,6 +343,32 @@ def run_b200(args, rank, local_rank, world):
     if distributed:
         dist.barrier()
         dist.destroy_process_group()
+
+
+def dump_outputs(out_dir, q, torch, env, reward, done, dev, stream):
+    """--dump-outputs DIR: what the last timed launch handed its caller, as DIR/<name>.npy in f32 / f64, so that two builds run with
+    the same arguments can be compared output for output: reward and done [steps_per_launch][envs], the env state it advanced to
+    (one file per field, u32 fields as f64, the 64-bit brick masks as two f64 halves) and the 4-frame observation stacks
+    [envs][slot][y][x] of the first DUMP_OBS_ENVS of those envs. Beyond 4,096 envs, or 32 MiB of per-env arrays, the envs are a
+    fixed seeded sample, so the files stay under 64 MB together (at most 32 MiB + 28.9 MB of stacks). Rank 0's shard only."""
+    n, k = env.n_envs, reward.shape[0]
+    st = env.read_state()
+    state = {name: st[name] for name in ("ball_cx", "ball_cy", "ball_dx", "ball_dy", "pad_min_x", "pad_max_x", "pad_speed")}
+    state.update({name: st[name].astype(np.float64) for name in ("score", "episode_step", "episode", "err")})
+    state["finished"] = st["finished"].astype(np.float32)
+    state["bricks_lo"] = (st["bricks"] & np.uint64(0xFFFFFFFF)).astype(np.float64)
+    state["bricks_hi"] = (st["bricks"] >> np.uint64(32)).astype(np.float64)
+    per_env = 2 * 4 * k + sum(a.itemsize for a in state.values())
+    keep = max(1, min(n, 4096, (32 << 20) // per_env))
+    ids = np.arange(n) if keep == n else np.sort(np.random.default_rng(SEED).choice(n, keep, replace=False))
+    obs = torch.empty((n, 4, 84, 84), dtype=torch.uint8, device=dev)
+    env.obs_device(q.LAYOUT_U8_BHYX, obs.data_ptr(), stream)
+    out = {"reward": reward.cpu().numpy()[:, ids], "done": done.cpu().numpy()[:, ids].astype(np.float32),
+           "obs": obs[torch.from_numpy(ids[:DUMP_OBS_ENVS]).to(dev)].float().cpu().numpy()}
+    out.update(("state_" + name, a[ids]) for name, a in state.items())
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a))
 
 
 def measure_stats_reduce_every_step(q, torch, dist, env, launch, stream, rank, world, dev, barrier, steps):
@@ -779,7 +810,10 @@ def main():
     ap.add_argument("--no-extra", action="store_true", help="skip the secondary measurements")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-learner", action="store_true", help="skip the learner-in-the-loop section (profiling runs: it is thousands of library kernels)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed to DIR/<name>.npy (f32 / f64, under 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

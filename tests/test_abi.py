@@ -31,9 +31,10 @@ def test_library_exports_every_declared_symbol(qlb):
 def test_library_is_sm100a_with_bulk_copies(qlb):
     """The shipped binary carries sm_100a code and the TMA bulk-copy instructions (UBLKCP) of the render / gather path."""
     so = qlb.library_path()
-    out = subprocess.run(["cuobjdump", "-lelf", so], capture_output=True, text=True).stdout
+    cuobjdump = os.path.join(os.path.dirname(qlb._build._nvcc()), "cuobjdump")      # the toolkit that built the library
+    out = subprocess.run([cuobjdump, "-lelf", so], capture_output=True, text=True).stdout
     assert "sm_100a" in out
-    sass = subprocess.run(["cuobjdump", "-sass", so], capture_output=True, text=True).stdout
+    sass = subprocess.run([cuobjdump, "-sass", so], capture_output=True, text=True).stdout
     assert "UBLKCP" in sass, "no bulk async copies in SASS"
     assert "SYNCS" in sass, "no mbarrier ops in SASS"
     assert "FFMA" not in sass.split("env_reset_kernel")[0] or True   # (-fmad=false is checked below)
