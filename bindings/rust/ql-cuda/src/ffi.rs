@@ -103,6 +103,17 @@ pub struct qlc_qnet_weights {
     pub dense2_bias: *const f32,
 }
 
+/// Adam + clipnorm settings of qlc_qnet_train (default: the Keras model's 2.5e-4, 0.9, 0.999, 1e-7, clipnorm 1.0).
+#[repr(C)]
+#[derive(Clone, Copy, Debug)]
+pub struct qlc_adam_config {
+    pub lr: f32,
+    pub beta1: f32,
+    pub beta2: f32,
+    pub epsilon: f32,
+    pub clipnorm: f32,
+}
+
 #[repr(C)]
 #[derive(Clone, Copy, Default)]
 pub struct qlc_episode_stats {
@@ -178,5 +189,12 @@ extern "C" {
     pub fn qlc_qnet_error(qnet: *mut qlc_qnet, flag: *mut u32) -> i32;
     pub fn qlc_qnet_forward(qnet: *mut qlc_qnet, idx_dev: *const u32, n: u32, which: i32, q_dev: *mut f32, action_dev: *mut u8, max_q_dev: *mut f32, stream: *mut c_void) -> i32;
     pub fn qlc_qnet_forward_host(qnet: *mut qlc_qnet, idx_host: *const u32, n: u32, which: i32, q_host: *mut f32, action_host: *mut u8, max_q_host: *mut f32) -> i32;
+    pub fn qlc_qnet_set_adam(qnet: *mut qlc_qnet, cfg: *const qlc_adam_config) -> i32;
+    pub fn qlc_qnet_get_weights(qnet: *mut qlc_qnet, out_host: *const qlc_qnet_weights) -> i32;
+    pub fn qlc_qnet_train(qnet: *mut qlc_qnet, idx_dev: *const u32, batch: u32, n_batches: u32, target_dev: *const f32, target_net: *mut qlc_qnet,
+                          gamma: f32, loss_dev: *mut f32, stream: *mut c_void) -> i32;
+    pub fn qlc_qnet_train_host(qnet: *mut qlc_qnet, idx_host: *const u32, batch: u32, n_batches: u32, target_host: *const f32, target_net: *mut qlc_qnet,
+                               gamma: f32, loss_host: *mut f32) -> i32;
+    pub fn qlc_qnet_debug_grads(qnet: *mut qlc_qnet, idx_host: *const u32, n: u32, target_host: *const f32, grads_out_host: *const qlc_qnet_weights) -> i32;
     pub fn qlc_debug_gemm_bf16(a_host: *const f32, w_host: *const f32, bias_host: *const f32, relu: i32, out_host: *mut f32, m: u32, n: u32, k: u32) -> i32;
 }

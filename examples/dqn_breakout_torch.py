@@ -70,10 +70,14 @@ class TorchDQNModel:
 
 
 def run(n_envs=1024, iterations=200, batch=32, minibatches_per_call=None, seed=0, device=0, quiet=False, tensor_core_actor=False, actor_sync_every=10,
-        env_id_base=0, skip_model=False, random_phase_steps=None):
+        env_id_base=0, skip_model=False, random_phase_steps=None, tensor_core_learner=False, target_sync_every=250):
     """Device-resident variant of learner.SelfDrivingQLearner.learn_iteration: same rules, tensors never leave the GPU.
     skip_model: run the data path only (step, replay insert, sample + gather, TD-target inputs) without the network calls —
-    what is left of an iteration when the learner costs nothing (bench.py uses it to attribute the iteration time)."""
+    what is left of an iteration when the learner costs nothing (bench.py uses it to attribute the iteration time).
+    tensor_core_learner: the whole model on the library (torch_io.TensorCoreLearner): greedy actions and training on the
+    tcgen05 Q-network; minibatches are drawn by qlc_replay_sample into an index tensor (no gather, no state tensor) and
+    trained by qlc_qnet_train (one update per call on all of them, like the torch path) with the TD target from the target
+    network, which follows every `target_sync_every` iterations."""
     dev = torch.device("cuda", device)
     torch.cuda.set_device(dev)
     p = L.Parameter(history_buffer_len=n_envs * 128, epsilon_pure_random_steps=n_envs * 20 if random_phase_steps is None else random_phase_steps,
@@ -83,12 +87,16 @@ def run(n_envs=1024, iterations=200, batch=32, minibatches_per_call=None, seed=0
     rb = q.ReplayBuffer(env)
     model, target = TorchDQNModel(dev), TorchDQNModel(dev)
     target.load_from(model)
+    learner = tio.TensorCoreLearner(env, tio.keras_weights_from_torch(model.net), gamma=p.gamma.item()) if tensor_core_learner else None
     # optional: action selection on the library's tcgen05 Q-network, reading the frame ring directly (no f32 observation
     # is materialised); its weights follow the torch model every `actor_sync_every` iterations
     actor = tio.TensorCoreActor(env, model.net) if tensor_core_actor else None
     due_per_iter = n_envs // p.update_after_actions               # one minibatch per 4 env-steps (self_driving_tf_q_learner.rs:181)
     nb = minibatches_per_call or due_per_iter
-    sampler = tio.DeviceSampler(rb, batch, nb, q.LAYOUT_F32_BXYH)
+    if learner is None:
+        sampler = tio.DeviceSampler(rb, batch, nb, q.LAYOUT_F32_BXYH)
+    else:
+        idx = torch.empty((nb, batch), dtype=torch.int32, device=dev)
     gen = torch.Generator(device=dev); gen.manual_seed(seed)
     obs = None
     epsilon, delta = p.epsilon_max, p.epsilon_interval() / p.epsilon_greedy_steps
@@ -102,7 +110,9 @@ def run(n_envs=1024, iterations=200, batch=32, minibatches_per_call=None, seed=0
         random_mask = (eps > u) | (step_count + 1 + torch.arange(n_envs, device=dev) < p.epsilon_pure_random_steps)
         actions = a_rand
         if not skip_model and not bool(random_mask.all()):
-            if actor is not None:
+            if learner is not None:
+                greedy = learner.predict_action()[0]
+            elif actor is not None:
                 if it % actor_sync_every == 0:
                     actor.sync(model.net)
                 greedy = actor.predict_action()[0]
@@ -116,6 +126,11 @@ def run(n_envs=1024, iterations=200, batch=32, minibatches_per_call=None, seed=0
         step_count += n_envs
         if rb.len() > batch:
             for _ in range(max(1, due_per_iter // nb)):
+                if learner is not None:
+                    rb.sample_device(batch, nb, calls, idx.data_ptr(), tio._stream()); calls += nb
+                    if not skip_model:
+                        learner.train_indices(idx.view(1, -1))     # one update on the nb minibatches together, as the torch model trains them
+                    continue
                 s = sampler.sample(calls); calls += nb
                 st, nx = s.state.view(nb * batch, 84, 84, 4), s.state_next.view(nb * batch, 84, 84, 4)
                 if skip_model:
@@ -124,18 +139,26 @@ def run(n_envs=1024, iterations=200, batch=32, minibatches_per_call=None, seed=0
                 rwd, dn = s.reward.view(-1), s.done.view(-1)
                 updated_q = torch.where(dn != 0, rwd, rwd + p.gamma.item() * max_future)      # TD target (:192-199)
                 model.train(st, s.action.view(-1), updated_q)
+        if learner is not None and (it + 1) % target_sync_every == 0:
+            learner.sync_target()
         ended = done[0] != 0
         if bool(ended.any()):
             finished_returns.extend(returns[ended].tolist()); returns[ended] = 0
         if (it + 1) % 50 == 0 and not quiet:
             torch.cuda.synchronize()
             print("iter %d  env-steps %d  eps %.3f  loss %.4f  episodes %d  mean return %.2f  %.0f env-steps/s" % (
-                it + 1, step_count, epsilon, float(torch.stack(model.losses[-20:]).mean()) if model.losses else float("nan"),
+                it + 1, step_count, epsilon, float(torch.cat([x.reshape(-1) for x in (learner.losses if learner else model.losses)[-20:]]).mean())
+                if (learner.losses if learner else model.losses) else float("nan"),
                 len(finished_returns), float(np.mean(finished_returns[-500:])) if finished_returns else float("nan"), step_count / (time.time() - t0)), flush=True)
     torch.cuda.synchronize()
     stats = env.stats()
-    out = {"env_steps": step_count, "seconds": time.time() - t0, "episodes": int(stats["episodes"]), "train_calls": len(model.losses), "minibatches": calls,
-           "last_loss": float(model.losses[-1]) if model.losses else None, "epsilon": epsilon, "error_flags": env.error_flags()}
+    losses = model.losses if learner is None else learner.losses
+    out = {"env_steps": step_count, "seconds": time.time() - t0, "episodes": int(stats["episodes"]), "train_calls": len(losses), "minibatches": calls,
+           "last_loss": float(losses[-1].reshape(-1)[-1]) if losses else None, "epsilon": epsilon, "error_flags": env.error_flags()}
+    if learner is not None:
+        out["losses_finite"] = bool(all(torch.isfinite(x).all() for x in learner.losses))
+        out["qnet_error"] = learner.error()
+        learner.close()
     if actor is not None:
         actor.close()
     env.close()
@@ -147,6 +170,8 @@ if __name__ == "__main__":
     ap.add_argument("--envs", type=int, default=1024)
     ap.add_argument("--iterations", type=int, default=200)
     ap.add_argument("--batch", type=int, default=32)
+    ap.add_argument("--tensor-core-learner", action="store_true", help="the whole model on the library: greedy actions and training (qlc_qnet_train) "
+                    "on its tcgen05 Q-network, minibatches sampled as indices only")
     ap.add_argument("--tensor-core-actor", action="store_true", help="greedy actions from the library's tcgen05 Q-network (weights synced from the torch model)")
     args = ap.parse_args()
-    print(run(args.envs, args.iterations, args.batch, tensor_core_actor=args.tensor_core_actor))
+    print(run(args.envs, args.iterations, args.batch, tensor_core_actor=args.tensor_core_actor, tensor_core_learner=args.tensor_core_learner))

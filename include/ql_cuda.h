@@ -257,6 +257,25 @@ int32_t qlc_qnet_error(qlc_qnet* qnet, uint32_t* flag);
 int32_t qlc_qnet_forward(qlc_qnet* qnet, const uint32_t* idx_dev, uint32_t n, int32_t which, float* q_dev, uint8_t* action_dev, float* max_q_dev, void* stream);
 int32_t qlc_qnet_forward_host(qlc_qnet* qnet, const uint32_t* idx_host, uint32_t n, int32_t which, float* q_host, uint8_t* action_host, float* max_q_host);
 
+/* ---- Q-network training on the device: the reference's DeepQLearningModel::train (ml_model/model.rs:59-71) for the Keras
+ * model (Huber(delta 1) loss on Q(s)[a] averaged over the minibatch, clipnorm per variable, Adam). Master weights, Adam
+ * moments and gradients are f32; GEMM operands bf16 with f32 accumulation. Deterministic: the same inputs give the same
+ * weight bits. Adam moments are not part of qlc_env_save checkpoints; a resumed run restarts them. ---- */
+typedef struct qlc_adam_config { float lr, beta1, beta2, epsilon, clipnorm; } qlc_adam_config;   /* default 2.5e-4, 0.9, 0.999, 1e-7, 1.0; clipnorm <= 0: off */
+int32_t qlc_qnet_set_adam(qlc_qnet* qnet, const qlc_adam_config* cfg);           /* also resets m, v and the step count t (as qlc_qnet_set_weights does) */
+int32_t qlc_qnet_get_weights(qlc_qnet* qnet, const qlc_qnet_weights* out_host);  /* the f32 masters in the Keras layouts (writes through the pointers) */
+/* n_batches successive updates on the minibatches idx_dev[j * batch .. (j + 1) * batch) of replay transitions (state =
+ * which 0 of qlc_qnet_forward, action = record bits 0-1). Targets: target_dev [n_batches][batch] f32, or, when it is NULL,
+ * y = r + max_a Q_target(state_next) * gamma (y = r where done) from target_net (same env), evaluated once for the whole
+ * call. loss_dev (optional): [n_batches] Huber losses, before each update. Asynchronous on `stream`; MMA time-outs raise
+ * the sticky flag of qlc_qnet_error. */
+int32_t qlc_qnet_train(qlc_qnet* qnet, const uint32_t* idx_dev, uint32_t batch, uint32_t n_batches, const float* target_dev, qlc_qnet* target_net,
+                       float gamma, float* loss_dev, void* stream);
+int32_t qlc_qnet_train_host(qlc_qnet* qnet, const uint32_t* idx_host, uint32_t batch, uint32_t n_batches, const float* target_host, qlc_qnet* target_net,
+                            float gamma, float* loss_host);
+/* forward + backward only, for tests: the unclipped f32 gradients of the loss over n transitions with targets target_host [n] */
+int32_t qlc_qnet_debug_grads(qlc_qnet* qnet, const uint32_t* idx_host, uint32_t n, const float* target_host, const qlc_qnet_weights* grads_out_host);
+
 /* ---- checkpoint / resume of the env shard + replay ring (the reference checkpoints only the model:
  * q_learning_model.rs:191-202). qlc_env_load needs an env created with the same n_envs / env_id_base / seed /
  * replay_capacity / episode limits; a resumed run continues bit-identically. Synchronous. ---- */

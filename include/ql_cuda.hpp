@@ -283,6 +283,33 @@ public:
     TensorCoreQModel& operator=(const TensorCoreQModel&) = delete;
     void set_weights(const qlc_qnet_weights& weights) { check(qlc_qnet_set_weights(q_, &weights)); }
 
+    // The ten Keras arrays (f32 masters, layouts of qlc_qnet_weights) owned by the caller.
+    struct Weights {
+        std::vector<float> conv1_kernel = std::vector<float>(8 * 8 * 4 * 32), conv1_bias = std::vector<float>(32);
+        std::vector<float> conv2_kernel = std::vector<float>(4 * 4 * 32 * 64), conv2_bias = std::vector<float>(64);
+        std::vector<float> conv3_kernel = std::vector<float>(3 * 3 * 64 * 64), conv3_bias = std::vector<float>(64);
+        std::vector<float> dense1_kernel = std::vector<float>((size_t)3136 * 512), dense1_bias = std::vector<float>(512);
+        std::vector<float> dense2_kernel = std::vector<float>(512 * 3), dense2_bias = std::vector<float>(3);
+        qlc_qnet_weights view() const {
+            return {conv1_kernel.data(), conv1_bias.data(), conv2_kernel.data(), conv2_bias.data(), conv3_kernel.data(), conv3_bias.data(),
+                    dense1_kernel.data(), dense1_bias.data(), dense2_kernel.data(), dense2_bias.data()};
+        }
+    };
+    Weights weights() const {                                       // checkpoint / target sync (set_weights(w.view()))
+        Weights w;
+        const qlc_qnet_weights v = w.view();
+        check(qlc_qnet_get_weights(q_, &v));
+        return w;
+    }
+    // DeepQLearningModel::train (model.rs:59-71) on replay transitions by logical index (state and action read from the ring),
+    // one Keras-Adam update with the given TD targets; returns the Huber loss before the update.
+    float train_replay(const std::vector<uint32_t>& idx, const std::vector<float>& targets) {
+        if (idx.size() != targets.size() || idx.empty()) throw QlError("train_replay: one target per index, at least one index");
+        float loss = 0.0f;
+        check(qlc_qnet_train_host(q_, idx.data(), (uint32_t)idx.size(), 1, targets.data(), nullptr, 0.0f, &loss));
+        return loss;
+    }
+
     BreakoutAction predict_action(const BreakoutState& state) const {
         uint8_t a = 0;
         q_values(state, &a);

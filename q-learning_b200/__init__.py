@@ -52,6 +52,7 @@ ABI_SYMBOLS = [
     "qlc_stats_read", "qlc_stats_export", "qlc_stats_push", "qlc_stats_mean", "qlc_stats_min", "qlc_stats_window",
     "qlc_debug_collision_wall", "qlc_debug_collision_rect", "qlc_debug_collision_rect_batch", "qlc_debug_gemm_bf16",
     "qlc_qnet_create", "qlc_qnet_set_weights", "qlc_qnet_destroy", "qlc_qnet_error", "qlc_qnet_forward", "qlc_qnet_forward_host",
+    "qlc_qnet_set_adam", "qlc_qnet_get_weights", "qlc_qnet_train", "qlc_qnet_train_host", "qlc_qnet_debug_grads",
 ]
 
 
@@ -95,6 +96,10 @@ OBS_HANDLE_DTYPE = np.dtype([("time", np.uint64), ("k", np.uint32), ("env", np.u
 class QlcQnetWeights(C.Structure):
     _fields_ = [(n, C.c_void_p) for n in ("conv1_kernel", "conv1_bias", "conv2_kernel", "conv2_bias", "conv3_kernel", "conv3_bias",
                                            "dense1_kernel", "dense1_bias", "dense2_kernel", "dense2_bias")]
+
+
+class QlcAdamConfig(C.Structure):
+    _fields_ = [(n, C.c_float) for n in ("lr", "beta1", "beta2", "epsilon", "clipnorm")]
 
 
 QNET_SHAPES = {"conv1_kernel": (8, 8, 4, 32), "conv1_bias": (32,), "conv2_kernel": (4, 4, 32, 64), "conv2_bias": (64,),
@@ -184,6 +189,11 @@ def load_library(build_if_missing=True):
         "qlc_qnet_destroy": (i32, [vp]),
         "qlc_qnet_forward": (i32, [vp, vp, u32, i32, vp, vp, vp, vp]),
         "qlc_qnet_forward_host": (i32, [vp, vp, u32, i32, vp, vp, vp]),
+        "qlc_qnet_set_adam": (i32, [vp, C.POINTER(QlcAdamConfig)]),
+        "qlc_qnet_get_weights": (i32, [vp, C.POINTER(QlcQnetWeights)]),
+        "qlc_qnet_train": (i32, [vp, vp, u32, u32, vp, vp, C.c_float, vp, vp]),
+        "qlc_qnet_train_host": (i32, [vp, vp, u32, u32, vp, vp, C.c_float, vp]),
+        "qlc_qnet_debug_grads": (i32, [vp, vp, u32, vp, C.POINTER(QlcQnetWeights)]),
     }
     for name, (res, args) in sig.items():
         f = getattr(L, name)   # AttributeError if the library lacks a declared symbol
@@ -667,10 +677,10 @@ def debug_gemm_bf16(a, w, bias, relu=False):
 
 
 class QNetwork:
-    """Q-network forward on the tensor cores (tcgen05) for a BreakoutEnvironment: the inference half of the reference's
-    DeepQLearningModel (ml_model/model.rs:29-77) — predict_action for every env, batch_predict_max_future_reward for replay
-    samples — reading the u8 frames straight from the frame ring. `weights`: dict of f32 arrays in the Keras layouts
-    (QNET_SHAPES); bf16 operands, f32 accumulation."""
+    """Q-network on the tensor cores (tcgen05) for a BreakoutEnvironment: the reference's DeepQLearningModel
+    (ml_model/model.rs:29-77) — predict_action for every env, batch_predict_max_future_reward for replay samples, and
+    train on replay minibatches — reading the u8 frames straight from the frame ring. `weights`: dict of f32 arrays in the
+    Keras layouts (QNET_SHAPES); bf16 operands, f32 accumulation; f32 master weights and Adam moments for training."""
 
     def __init__(self, env, weights):
         self._env = env
@@ -729,3 +739,48 @@ class QNetwork:
 
     def forward_device(self, idx_ptr, n, which, q_ptr=None, action_ptr=None, max_q_ptr=None, stream=None):
         _check(self._L.qlc_qnet_forward(self._h, idx_ptr, n, which, q_ptr, action_ptr, max_q_ptr, stream))
+
+    def get_weights(self):
+        """The f32 master weights as a dict of arrays in the Keras layouts (QNET_SHAPES)."""
+        out = {name: np.empty(shape, dtype=np.float32) for name, shape in QNET_SHAPES.items()}
+        w, _ = self._pack(out)
+        _check(self._L.qlc_qnet_get_weights(self._h, C.byref(w)))
+        return out
+
+    def set_adam(self, lr=2.5e-4, beta1=0.9, beta2=0.999, epsilon=1e-7, clipnorm=1.0):
+        """Adam + per-variable clipnorm settings (clipnorm <= 0: no clipping); resets the moments and the step count."""
+        _check(self._L.qlc_qnet_set_adam(self._h, C.byref(QlcAdamConfig(lr, beta1, beta2, epsilon, clipnorm))))
+
+    def train(self, indices, targets=None, target_net=None, gamma=0.99, n_batches=1):
+        """`n_batches` successive updates on the replay transitions `indices` ([n_batches * batch], minibatch j = the j-th
+        slice). Targets: f32 [n_batches * batch], or None for y = r + max Q_target(state_next) * gamma (y = r where done)
+        from `target_net`. Returns the Huber loss of each minibatch (before its update) as f32 [n_batches]."""
+        idx = np.ascontiguousarray(indices, dtype=np.uint32).ravel()
+        if n_batches < 1 or idx.size % n_batches:
+            raise QlError("the number of indices must be a multiple of n_batches")
+        batch = idx.size // n_batches
+        tgt = None
+        if targets is not None:
+            tgt = np.ascontiguousarray(targets, dtype=np.float32).ravel()
+            if tgt.size != idx.size:
+                raise QlError("targets must have one value per index")
+        loss = np.empty(n_batches, dtype=np.float32)
+        _check(self._L.qlc_qnet_train_host(self._h, _np_ptr(idx), batch, n_batches, None if tgt is None else _np_ptr(tgt),
+                                           None if target_net is None else target_net._h, gamma, _np_ptr(loss)))
+        return loss
+
+    def train_device(self, idx_ptr, batch, n_batches, target_ptr=None, target_net=None, gamma=0.99, loss_ptr=None, stream=None):
+        """Device-pointer form of train (asynchronous on `stream`; time-outs surface through error())."""
+        _check(self._L.qlc_qnet_train(self._h, idx_ptr, batch, n_batches, target_ptr, None if target_net is None else target_net._h,
+                                      gamma, loss_ptr, stream))
+
+    def debug_grads(self, indices, targets):
+        """Forward + backward only: the unclipped f32 gradients of the loss on (indices, targets), Keras layouts."""
+        idx = np.ascontiguousarray(indices, dtype=np.uint32).ravel()
+        tgt = np.ascontiguousarray(targets, dtype=np.float32).ravel()
+        if tgt.size != idx.size:
+            raise QlError("targets must have one value per index")
+        out = {name: np.empty(shape, dtype=np.float32) for name, shape in QNET_SHAPES.items()}
+        w, _ = self._pack(out)
+        _check(self._L.qlc_qnet_debug_grads(self._h, _np_ptr(idx), idx.size, _np_ptr(tgt), C.byref(w)))
+        return out

@@ -4,12 +4,15 @@
 #include "kernels.cuh"
 #include "qnet.cuh"
 #include "qnet_conv.cuh"
+#include "qnet_train.cuh"
 #include "host_pool.h"
 #include "comm.h"
 
 #include <nvtx3/nvToolsExt.h>   // header-only; ranges cost a few ns unless a tool (ncu --nvtx, nsys) is attached
 
+#include <algorithm>
 #include <chrono>
+#include <cmath>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -1298,11 +1301,12 @@ int32_t qlc_debug_collision_rect_batch(const float* in_host, float* out_host, ui
 }
 }  // extern "C"
 
-template <int NT, class Loader>
-static cudaError_t launch_gemm_tc(const Loader& ld, const __nv_bfloat16* w, const float* bias, __nv_bfloat16* out, uint32_t m, uint32_t k, uint32_t n_total,
-                                  int relu, unsigned int* err, cudaStream_t s) {
+// gemm_tc_kernel over n_splits K slices (gridDim.z); persistent CTAs along M, as many as fit beside the other N tiles
+template <int NT, class Loader, class Epi>
+static cudaError_t launch_gemm(const Loader& ld, const __nv_bfloat16* w, const Epi& epi, uint32_t m, uint32_t k, uint32_t n_total, uint32_t n_splits,
+                               unsigned int* err, cudaStream_t s) {
     const size_t dyn = 2 * ((size_t)qnet::TILE_M * qnet::KC * 2 + (size_t)NT * qnet::KC * 2);
-    auto kern = qnet::gemm_tc_kernel<NT, Loader>;
+    auto kern = qnet::gemm_tc_kernel<NT, Loader, Epi>;
     static int occ_dev[64] = {}, sms_dev[64] = {};
     int cur_dev = 0; cudaGetDevice(&cur_dev);
     int &occ = occ_dev[cur_dev & 63], &sms = sms_dev[cur_dev & 63];
@@ -1319,11 +1323,16 @@ static cudaError_t launch_gemm_tc(const Loader& ld, const __nv_bfloat16* w, cons
         if (occ < 1) occ = 1;
     }
     const uint32_t n_mtiles = (m + qnet::TILE_M - 1) / qnet::TILE_M, n_ntiles = n_total / NT;
-    uint32_t gx = (uint32_t)(occ * sms) / n_ntiles;
+    uint32_t gx = (uint32_t)(occ * sms) / (n_ntiles * n_splits);
     if (gx < 1) gx = 1;
     if (gx > n_mtiles) gx = n_mtiles;
-    kern<<<dim3(gx, n_ntiles), 128, dyn, s>>>(ld, w, bias, out, m, k, n_total, relu, err);
+    kern<<<dim3(gx, n_ntiles, n_splits), 128, dyn, s>>>(ld, w, epi, m, k, n_total, err);
     return cudaGetLastError();
+}
+template <int NT, class Loader>
+static cudaError_t launch_gemm_tc(const Loader& ld, const __nv_bfloat16* w, const float* bias, __nv_bfloat16* out, uint32_t m, uint32_t k, uint32_t n_total,
+                                  int relu, unsigned int* err, cudaStream_t s) {
+    return launch_gemm<NT>(ld, w, qnet::EpiBiasAct{bias, out, n_total, relu}, m, k, n_total, 1u, err, s);
 }
 
 template <class G, class Out>
@@ -1355,9 +1364,32 @@ struct qlc_qnet {
     __nv_bfloat16 *a1p = nullptr, *a2p = nullptr, *a3p = nullptr;         // conv outputs in the next layer's operand (plane) layout
     unsigned long long* prof = nullptr;                                    // QLC_QNET_PROF: per-role cycle counters of CTA 0, printed after each forward
     int impl = 4;                                                          // how many convs run as shifted-window kernels (QLC_QNET_IMPL, A/B testing)
-    float* stage = nullptr; size_t stage_bytes = 0;
     uint32_t cap_items = 0;
+    // training (qlc_qnet_train): f32 masters of the 10 Keras variables back to back (b1..b5 point into it), their gradients,
+    // Adam moments; bf16 weight copies in the data-gradient GEMMs' operand layouts; scratch sized for train_cap items
+    float *master = nullptr, *grad = nullptr, *adam_m = nullptr, *adam_v = nullptr, *norm_partial = nullptr;
+    __nv_bfloat16 *w4k = nullptr, *w3r = nullptr, *w2r = nullptr;
+    qlc_adam_config adam{2.5e-4f, 0.9f, 0.999f, 1e-7f, 1.0f};
+    uint64_t adam_t = 0;                                                   // updates since set_weights / set_adam
+    uint32_t train_cap = 0, y_cap = 0;
+    float *t_q = nullptr, *t_dq = nullptr, *t_loss = nullptr, *t_dh = nullptr, *t_d3 = nullptr, *t_d2 = nullptr, *t_d1 = nullptr, *t_split = nullptr, *t_colsum = nullptr;
+    __nv_bfloat16 *t_dh_bf = nullptr, *t_d3_bf = nullptr, *t_d2_bf = nullptr, *t_pack = nullptr;
+    float *t_y = nullptr, *t_maxq = nullptr;
+    size_t split_floats = 0, pack_elems = 0;
 };
+
+// per-minibatch scratch of the backward (sized for train_cap items)
+static void qnet_free_scratch(qlc_qnet* q) {
+    void* p[] = {q->t_q, q->t_dq, q->t_loss, q->t_dh, q->t_d3, q->t_d2, q->t_d1, q->t_split, q->t_colsum, q->t_dh_bf, q->t_d3_bf, q->t_d2_bf, q->t_pack};
+    for (void* x : p) cudaFree(x);
+    q->t_q = q->t_dq = q->t_loss = q->t_dh = q->t_d3 = q->t_d2 = q->t_d1 = q->t_split = q->t_colsum = nullptr;
+    q->t_dh_bf = q->t_d3_bf = q->t_d2_bf = q->t_pack = nullptr; q->train_cap = 0; q->split_floats = 0; q->pack_elems = 0;
+}
+// TD targets and target-network max-Q of one call (sized for y_cap items)
+static void qnet_free_targets(qlc_qnet* q) {
+    cudaFree(q->t_y); cudaFree(q->t_maxq); q->t_y = q->t_maxq = nullptr; q->y_cap = 0;
+}
+static void qnet_free_train(qlc_qnet* q) { qnet_free_scratch(q); qnet_free_targets(q); }
 
 static void qnet_free_acts(qlc_qnet* q) {
     cudaFree(q->a1); cudaFree(q->a2); cudaFree(q->a3); cudaFree(q->a4); cudaFree(q->slot_frame); cudaFree(q->a1p); cudaFree(q->a2p); cudaFree(q->a3p); cudaFree(q->head_partial); cudaFree(q->head_count);
@@ -1373,10 +1405,13 @@ static void qnet_release_device(qlc_qnet* q) {
     cudaSetDevice(q->device);
     cudaDeviceSynchronize();
     qnet_free_acts(q);
+    qnet_free_train(q);
     cudaFree(q->w1); cudaFree(q->w2); cudaFree(q->w3); cudaFree(q->w4); cudaFree(q->w5); cudaFree(q->w1p); cudaFree(q->w2p); cudaFree(q->w3p); cudaFree(q->w4p); cudaFree(q->w4p256);
-    cudaFree(q->b1); cudaFree(q->b2); cudaFree(q->b3); cudaFree(q->b4); cudaFree(q->b5); cudaFree(q->err); cudaFree(q->stage); cudaFree(q->prof);
+    cudaFree(q->master); cudaFree(q->grad); cudaFree(q->adam_m); cudaFree(q->adam_v); cudaFree(q->norm_partial); cudaFree(q->w4k); cudaFree(q->w3r); cudaFree(q->w2r);
+    cudaFree(q->err); cudaFree(q->prof);
     q->w1 = q->w2 = q->w3 = q->w4 = q->w1p = q->w2p = q->w3p = q->w4p = q->w4p256 = nullptr; q->w5 = nullptr;
-    q->b1 = q->b2 = q->b3 = q->b4 = q->b5 = nullptr; q->err = nullptr; q->stage = nullptr; q->stage_bytes = 0; q->prof = nullptr;
+    q->master = q->grad = q->adam_m = q->adam_v = q->norm_partial = nullptr; q->w4k = q->w3r = q->w2r = nullptr;
+    q->b1 = q->b2 = q->b3 = q->b4 = q->b5 = nullptr; q->err = nullptr; q->prof = nullptr;
     q->env = nullptr;
 }
 
@@ -1410,36 +1445,74 @@ int32_t qlc_qnet_error(qlc_qnet* q, uint32_t* flag) {
     return QLC_OK;
 }
 
+static const float* const* weight_ptrs(const qlc_qnet_weights* w, const float* (&out)[qnet::NVARS]) {
+    const float* p[qnet::NVARS] = {w->conv1_kernel, w->conv1_bias, w->conv2_kernel, w->conv2_bias, w->conv3_kernel, w->conv3_bias, w->dense1_kernel, w->dense1_bias, w->dense2_kernel, w->dense2_bias};
+    for (int i = 0; i < qnet::NVARS; ++i) out[i] = p[i];
+    return out;
+}
+
+// operand-layout bf16 copies of the f32 masters (the forward's, and the backward's data-gradient weights), on `s`
+static cudaError_t qnet_prep_weights(qlc_qnet* q, cudaStream_t s) {
+    const float* m = q->master;
+    auto V = [&](int v) { return m + qnet::var_offset(v); };
+    qnet::prep_conv1_kernel<<<(32 * 256 + 255) / 256, 256, 0, s>>>(V(0), q->w1);
+    qnet::prep_conv1_planes_kernel<<<(32 * 256 + 255) / 256, 256, 0, s>>>(V(0), q->w1p);
+    qnet::prep_transpose_kernel<<<(512 * 64 + 255) / 256, 256, 0, s>>>(V(2), q->w2, 512, 64);             // [kh][kw][c][cout] = [K][N]
+    qnet::prep_conv2_planes_kernel<<<(512 * 64 + 255) / 256, 256, 0, s>>>(V(2), q->w2p);
+    qnet::prep_transpose_kernel<<<(576 * 64 + 255) / 256, 256, 0, s>>>(V(4), q->w3, 576, 64);
+    qnet::prep_conv3_planes_kernel<<<(576 * 64 + 255) / 256, 256, 0, s>>>(V(4), q->w3p);
+    qnet::prep_transpose_kernel<<<(3136 * 512 + 255) / 256, 256, 0, s>>>(V(6), q->w4, 3136, 512);
+    qnet::prep_dense_planes_kernel<128><<<(3136 * 512 + 255) / 256, 256, 0, s>>>(V(6), q->w4p);
+    qnet::prep_dense_planes_kernel<256><<<(3136 * 512 + 255) / 256, 256, 0, s>>>(V(6), q->w4p256);
+    qnet::prep_head_kernel<<<(3 * 512 + 255) / 256, 256, 0, s>>>(V(8), q->w5);
+    qnet::prep_dgrad_weights_kernel<16, 32, 64><<<(16 * 32 * 64 + 255) / 256, 256, 0, s>>>(V(2), q->w2r);
+    qnet::prep_dgrad_weights_kernel<9, 64, 64><<<(9 * 64 * 64 + 255) / 256, 256, 0, s>>>(V(4), q->w3r);
+    qnet::f32_to_bf16_kernel<<<1024, 256, 0, s>>>(V(6), q->w4k, (size_t)3136 * 512);
+    return cudaGetLastError();
+}
+
+static int32_t qnet_reset_adam(qlc_qnet* q) {
+    CUDA_TRY(cudaMemset(q->adam_m, 0, (size_t)qnet::N_PARAMS * 4));
+    CUDA_TRY(cudaMemset(q->adam_v, 0, (size_t)qnet::N_PARAMS * 4));
+    q->adam_t = 0;
+    return QLC_OK;
+}
+
 int32_t qlc_qnet_set_weights(qlc_qnet* q, const qlc_qnet_weights* w) {
     if (!q || !w) return fail(QLC_ERR_INVALID_ARG, "qnet/weights is null");
     if (!q->env) return fail(QLC_ERR_INVALID_ARG, "the environment of this Q-network has been destroyed");
-    const float* srcs[10] = {w->conv1_kernel, w->conv1_bias, w->conv2_kernel, w->conv2_bias, w->conv3_kernel, w->conv3_bias, w->dense1_kernel, w->dense1_bias, w->dense2_kernel, w->dense2_bias};
-    const size_t counts[10] = {8 * 8 * 4 * 32, 32, 4 * 4 * 32 * 64, 64, 3 * 3 * 64 * 64, 64, 3136 * 512, 512, 512 * 3, 3};
-    for (int i = 0; i < 10; ++i) if (!srcs[i]) return fail(QLC_ERR_INVALID_ARG, "a weight pointer is null");
+    const float* srcs[qnet::NVARS];
+    weight_ptrs(w, srcs);
+    for (int i = 0; i < qnet::NVARS; ++i) if (!srcs[i]) return fail(QLC_ERR_INVALID_ARG, "a weight pointer is null");
     int32_t rc = set_device(q->env); if (rc) return rc;
     CUDA_TRY(cudaDeviceSynchronize());
-    const size_t need = (size_t)3136 * 512 * 4;
-    if (q->stage_bytes < need) { cudaFree(q->stage); q->stage = nullptr; CUDA_TRY(cudaMalloc(&q->stage, need)); q->stage_bytes = need; }
-    float* biases[5] = {q->b1, q->b2, q->b3, q->b4, q->b5};
-    for (int l = 0; l < 5; ++l) {
-        CUDA_TRY(cudaMemcpy(q->stage, srcs[2 * l], counts[2 * l] * 4, cudaMemcpyHostToDevice));
-        switch (l) {
-            case 0: qnet::prep_conv1_kernel<<<(32 * 256 + 255) / 256, 256>>>(q->stage, q->w1);
-                    qnet::prep_conv1_planes_kernel<<<(32 * 256 + 255) / 256, 256>>>(q->stage, q->w1p); break;
-            case 1: qnet::prep_transpose_kernel<<<(512 * 64 + 255) / 256, 256>>>(q->stage, q->w2, 512, 64);             // [kh][kw][c][cout] = [K][N]
-                    qnet::prep_conv2_planes_kernel<<<(512 * 64 + 255) / 256, 256>>>(q->stage, q->w2p); break;
-            case 2: qnet::prep_transpose_kernel<<<(576 * 64 + 255) / 256, 256>>>(q->stage, q->w3, 576, 64);
-                    qnet::prep_conv3_planes_kernel<<<(576 * 64 + 255) / 256, 256>>>(q->stage, q->w3p); break;
-            case 3: qnet::prep_transpose_kernel<<<(3136 * 512 + 255) / 256, 256>>>(q->stage, q->w4, 3136, 512);
-                    qnet::prep_dense_planes_kernel<128><<<(3136 * 512 + 255) / 256, 256>>>(q->stage, q->w4p);
-                    qnet::prep_dense_planes_kernel<256><<<(3136 * 512 + 255) / 256, 256>>>(q->stage, q->w4p256); break;
-            default: qnet::prep_head_kernel<<<(3 * 512 + 255) / 256, 256>>>(q->stage, q->w5); break;
-        }
-        CUDA_TRY(cudaGetLastError());
-        CUDA_TRY(cudaDeviceSynchronize());
-        CUDA_TRY(cudaMemcpy(biases[l], srcs[2 * l + 1], counts[2 * l + 1] * 4, cudaMemcpyHostToDevice));
-    }
+    for (int v = 0; v < qnet::NVARS; ++v) CUDA_TRY(cudaMemcpy(q->master + qnet::var_offset(v), srcs[v], (size_t)qnet::var_size(v) * 4, cudaMemcpyHostToDevice));
+    CUDA_TRY(qnet_prep_weights(q, nullptr));
+    CUDA_TRY(cudaDeviceSynchronize());
+    return qnet_reset_adam(q);
+}
+
+int32_t qlc_qnet_get_weights(qlc_qnet* q, const qlc_qnet_weights* w) {
+    if (!q || !w) return fail(QLC_ERR_INVALID_ARG, "qnet/weights is null");
+    if (!q->env) return fail(QLC_ERR_INVALID_ARG, "the environment of this Q-network has been destroyed");
+    const float* dst[qnet::NVARS];
+    weight_ptrs(w, dst);
+    for (int i = 0; i < qnet::NVARS; ++i) if (!dst[i]) return fail(QLC_ERR_INVALID_ARG, "a weight pointer is null");
+    int32_t rc = set_device(q->env); if (rc) return rc;
+    CUDA_TRY(cudaDeviceSynchronize());
+    for (int v = 0; v < qnet::NVARS; ++v) CUDA_TRY(cudaMemcpy(const_cast<float*>(dst[v]), q->master + qnet::var_offset(v), (size_t)qnet::var_size(v) * 4, cudaMemcpyDeviceToHost));
     return QLC_OK;
+}
+
+int32_t qlc_qnet_set_adam(qlc_qnet* q, const qlc_adam_config* cfg) {
+    if (!q || !cfg) return fail(QLC_ERR_INVALID_ARG, "qnet/cfg is null");
+    if (!q->env) return fail(QLC_ERR_INVALID_ARG, "the environment of this Q-network has been destroyed");
+    if (!(cfg->lr >= 0.0f) || !(cfg->beta1 >= 0.0f && cfg->beta1 < 1.0f) || !(cfg->beta2 >= 0.0f && cfg->beta2 < 1.0f) || !(cfg->epsilon >= 0.0f) || cfg->clipnorm != cfg->clipnorm)
+        return fail(QLC_ERR_INVALID_ARG, "adam config out of range");
+    int32_t rc = set_device(q->env); if (rc) return rc;
+    CUDA_TRY(cudaDeviceSynchronize());
+    q->adam = *cfg;
+    return qnet_reset_adam(q);
 }
 
 int32_t qlc_qnet_create(qlc_env* env, const qlc_qnet_weights* w, qlc_qnet** out) {
@@ -1455,8 +1528,14 @@ int32_t qlc_qnet_create(qlc_env* env, const qlc_qnet_weights* w, qlc_qnet** out)
     A((void**)&q->w1p, 32 * 256 * 2); A((void**)&q->w2p, 64 * 512 * 2); A((void**)&q->w3p, 64 * 576 * 2); A((void**)&q->w4p, (size_t)512 * 3136 * 2); A((void**)&q->w4p256, (size_t)512 * 3136 * 2);
     if (const char* v = getenv("QLC_QNET_IMPL")) q->impl = atoi(v);
     if (getenv("QLC_QNET_PROF")) A((void**)&q->prof, 3 * 32 * 8);
-    A((void**)&q->b1, 32 * 4); A((void**)&q->b2, 64 * 4); A((void**)&q->b3, 64 * 4); A((void**)&q->b4, 512 * 4); A((void**)&q->b5, 3 * 4); A((void**)&q->err, 4);
-    if (e == cudaSuccess) e = cudaMemset(q->err, 0, 4);
+    A((void**)&q->master, (size_t)qnet::N_PARAMS * 4); A((void**)&q->grad, (size_t)qnet::N_PARAMS * 4);
+    A((void**)&q->adam_m, (size_t)qnet::N_PARAMS * 4); A((void**)&q->adam_v, (size_t)qnet::N_PARAMS * 4); A((void**)&q->norm_partial, qnet::NVARS * qnet::NORM_CHUNKS * 4);
+    A((void**)&q->w4k, (size_t)3136 * 512 * 2); A((void**)&q->w3r, 64 * 576 * 2); A((void**)&q->w2r, 32 * 1024 * 2); A((void**)&q->err, 4);
+    if (e == cudaSuccess) {
+        q->b1 = q->master + qnet::var_offset(1); q->b2 = q->master + qnet::var_offset(3); q->b3 = q->master + qnet::var_offset(5);
+        q->b4 = q->master + qnet::var_offset(7); q->b5 = q->master + qnet::var_offset(9);
+        e = cudaMemset(q->err, 0, 4);
+    }
     if (e != cudaSuccess) { qlc_qnet_destroy(q); return fail(QLC_ERR_CUDA, std::string("qnet alloc: ") + cudaGetErrorString(e)); }
     rc = qlc_qnet_set_weights(q, w);
     if (rc) { qlc_qnet_destroy(q); return rc; }
@@ -1464,8 +1543,11 @@ int32_t qlc_qnet_create(qlc_env* env, const qlc_qnet_weights* w, qlc_qnet** out)
     return QLC_OK;
 }
 
-int32_t qlc_qnet_forward(qlc_qnet* q, const uint32_t* idx_dev, uint32_t n, int32_t which, float* q_dev, uint8_t* action_dev, float* max_q_dev, void* stream) {
-    QLC_RANGE("qlc_qnet_forward");
+}  // extern "C"
+
+// the forward chain; hidden (training): keep the bf16 dense-1 activations in q->a4
+static int32_t qnet_forward(qlc_qnet* q, const uint32_t* idx_dev, uint32_t n, int32_t which, float* q_dev, uint8_t* action_dev, float* max_q_dev, bool hidden_out,
+                            void* stream) {
     if (!q) return fail(QLC_ERR_INVALID_ARG, "qnet is null");
     qlc_env* env = q->env;
     if (!env) return fail(QLC_ERR_INVALID_ARG, "the environment of this Q-network has been destroyed");
@@ -1533,7 +1615,7 @@ int32_t qlc_qnet_forward(qlc_qnet* q, const uint32_t* idx_dev, uint32_t n, int32
         const bool narrow = nt_force ? nt_force == 128 : m_tiles * 2u < (uint32_t)env->sm_count;
         // the head (Dense 512 -> 3, argmax, max) runs in the dense epilogue; rows_padded is that of the allocation (cap_items)
         const qnet::HeadArgs head{q->w5, q->b5, q->head_partial, q->head_count, ((q->cap_items + 127u) / 128u) * 128u, q_dev, action_dev, max_q_dev};
-        __nv_bfloat16* hidden = nullptr;                                   // the 512 hidden activations are not needed outside the kernel
+        __nv_bfloat16* hidden = hidden_out ? q->a4 : nullptr;             // the 512 hidden activations are only needed by training
         if (narrow)
             CUDA_TRY(launch_pdl(qnet::dense_tc_kernel<128>, dim3(m_tiles, 4), dim3(qnet::DenseGeomT<128>::THREADS), qnet::DenseGeomT<128>::SMEM_BYTES, s, (const uint8_t*)q->a3p,
                                 (const uint8_t*)q->w4p, (const float*)q->b4, hidden, n, q->err, head));
@@ -1557,6 +1639,13 @@ int32_t qlc_qnet_forward(qlc_qnet* q, const uint32_t* idx_dev, uint32_t n, int32
     return QLC_OK;
 }
 
+extern "C" int32_t qlc_qnet_forward(qlc_qnet* q, const uint32_t* idx_dev, uint32_t n, int32_t which, float* q_dev, uint8_t* action_dev, float* max_q_dev, void* stream) {
+    QLC_RANGE("qlc_qnet_forward");
+    return qnet_forward(q, idx_dev, n, which, q_dev, action_dev, max_q_dev, false, stream);
+}
+
+extern "C" {
+
 int32_t qlc_qnet_forward_host(qlc_qnet* q, const uint32_t* idx_host, uint32_t n, int32_t which, float* q_host, uint8_t* action_host, float* max_q_host) {
     QLC_RANGE("qlc_qnet_forward_host");
     if (!q) return fail(QLC_ERR_INVALID_ARG, "qnet is null");
@@ -1579,6 +1668,236 @@ int32_t qlc_qnet_forward_host(qlc_qnet* q, const uint32_t* idx_host, uint32_t n,
     uint32_t herr = 0;
     rc = qlc_qnet_error(q, &herr); if (rc) return rc;
     if (herr) return fail(QLC_ERR_CUDA, "qnet: an MMA completion barrier timed out");
+    return QLC_OK;
+}
+
+}  // extern "C"
+
+// ---------------- Q-network training (qnet_train.cuh, DESIGN §11) ----------------
+// K slices of a weight-gradient GEMM: enough CTAs for the machine (about two per SM), at least two 64-wide K chunks per slice
+struct SplitK { uint32_t splits, kc; };
+static SplitK pick_splits(uint32_t k_valid, uint32_t mn_tiles) {
+    const uint32_t chunks = (k_valid + qnet::KC - 1) / qnet::KC;
+    uint32_t sp = (296u + mn_tiles - 1u) / mn_tiles;
+    if (sp > 64u) sp = 64u;
+    if (sp > (chunks + 1u) / 2u) sp = (chunks + 1u) / 2u;
+    if (sp < 1u) sp = 1u;
+    const uint32_t per = (chunks + sp - 1u) / sp;
+    return SplitK{(chunks + per - 1u) / per, per * (uint32_t)qnet::KC};
+}
+// the four weight-gradient GEMMs of a minibatch of b items: {K valid, M x N tiles, N, M}
+struct WGradShape { uint32_t k_valid, mn_tiles, n, m; };
+static void wgrad_shapes(uint32_t b, WGradShape (&w)[4]) {
+    w[0] = {b, 25u * 2u, 512u, 3136u};          // dense 1 (N tiles of 256)
+    w[1] = {b * 49u, 5u, 64u, 576u};            // conv3
+    w[2] = {b * 81u, 4u, 64u, 512u};            // conv2
+    w[3] = {b * 400u, 2u, 32u, 256u};           // conv1
+}
+static uint32_t colsum_rows_per_split(uint32_t rows) { const uint32_t r = (rows + 63u) / 64u; return r < 256u ? 256u : r; }
+constexpr uint32_t COLSUM_MAX_SPLITS = 64, COLSUM_MAX_COLS = 1536;
+
+static int32_t qnet_train_alloc(qlc_qnet* q, uint32_t b) {
+    if (b <= q->train_cap) return QLC_OK;
+    CUDA_TRY(cudaDeviceSynchronize());
+    qnet_free_scratch(q);                   // a failed allocation below leaves train_cap = 0 and no stale pointers
+    WGradShape ws[4]; wgrad_shapes(b, ws);
+    size_t split_floats = 0, pack_elems = 0;
+    for (const WGradShape& w : ws) {
+        const SplitK sk = pick_splits(w.k_valid, w.mn_tiles);
+        split_floats = std::max(split_floats, (size_t)sk.splits * w.m * w.n);
+        pack_elems = std::max(pack_elems, (size_t)sk.splits * w.n * sk.kc);
+    }
+    const size_t n = b;
+    cudaError_t e = cudaSuccess;
+    auto A = [&](void** p, size_t bytes) { if (e == cudaSuccess) e = cudaMalloc(p, bytes); };
+    A((void**)&q->t_q, n * 3 * 4); A((void**)&q->t_dq, n * 3 * 4); A((void**)&q->t_loss, n * 4);
+    A((void**)&q->t_dh, n * 512 * 4); A((void**)&q->t_dh_bf, n * 512 * 2);
+    A((void**)&q->t_d3, n * 3136 * 4); A((void**)&q->t_d3_bf, n * 3136 * 2);
+    A((void**)&q->t_d2, n * 5184 * 4); A((void**)&q->t_d2_bf, n * 5184 * 2);
+    A((void**)&q->t_d1, n * 12800 * 4);
+    A((void**)&q->t_split, split_floats * 4); A((void**)&q->t_pack, pack_elems * 2);
+    A((void**)&q->t_colsum, (size_t)COLSUM_MAX_SPLITS * COLSUM_MAX_COLS * 4);
+    if (e != cudaSuccess) { cudaGetLastError(); qnet_free_scratch(q); return fail(QLC_ERR_CUDA, std::string("qnet training scratch: ") + cudaGetErrorString(e)); }
+    q->split_floats = split_floats; q->pack_elems = pack_elems; q->train_cap = b;
+    return QLC_OK;
+}
+
+// out[c] = sum over rows of x [rows][c] (fixed order) / div
+static cudaError_t launch_colsum(qlc_qnet* q, const float* x, uint32_t rows, uint32_t c, float div, float* out, cudaStream_t s) {
+    const uint32_t rps = colsum_rows_per_split(rows), splits = (rows + rps - 1) / rps;
+    cudaError_t e = launch_pdl(qnet::colsum_partial_kernel, dim3((c + 31) / 32, splits), dim3(32, 8), 0, s, x, rows, c, rps, q->t_colsum);
+    if (e != cudaSuccess) return e;
+    return launch_pdl(qnet::colsum_final_kernel, dim3((c + 255) / 256), dim3(256), 0, s, (const float*)q->t_colsum, splits, c, div, out);
+}
+// dW [m][n] (Keras layout, into the gradient block) = A^T(loader) * dZ [k_valid rows][n] over K slices
+template <int NT, class Loader>
+static cudaError_t launch_wgrad(qlc_qnet* q, const WGradShape& w, Loader ld, const float* dz, float* out, cudaStream_t s) {
+    const SplitK sk = pick_splits(w.k_valid, w.mn_tiles);
+    ld.k_valid = w.k_valid; ld.kc = sk.kc;
+    const size_t pack = (size_t)sk.splits * w.n * sk.kc;
+    cudaError_t e = launch_pdl(qnet::pack_splits_kernel, dim3((uint32_t)std::min<size_t>((pack + 255) / 256, 4096)), dim3(256), 0, s, dz, w.k_valid, w.n, sk.kc, sk.splits, q->t_pack);
+    if (e != cudaSuccess) return e;
+    e = launch_gemm<NT>(ld, (const __nv_bfloat16*)q->t_pack, qnet::EpiF32{q->t_split, w.m, w.n}, w.m, sk.kc, w.n, sk.splits, q->err, s);
+    if (e != cudaSuccess) return e;
+    const uint32_t mn = w.m * w.n;
+    return launch_pdl(qnet::reduce_splits_kernel, dim3(std::min<uint32_t>((mn + 255) / 256, 2048)), dim3(256), 0, s, (const float*)q->t_split, sk.splits, mn, out);
+}
+
+// forward + backward of one minibatch (idx_dev [b], targets y_dev [b]) into q->grad; loss_dev (optional) gets the mean Huber
+// loss; apply: clip + Adam + operand copies of the new weights
+static int32_t qnet_train_step(qlc_qnet* q, const uint32_t* idx_dev, uint32_t b, const float* y_dev, float* loss_dev, bool apply, cudaStream_t s) {
+    using namespace qnet;
+    qlc_env* env = q->env;
+    int32_t rc = qnet_train_alloc(q, b); if (rc) return rc;
+    rc = qnet_forward(q, idx_dev, b, 0, q->t_q, nullptr, nullptr, true, s); if (rc) return rc;
+    float* const g = q->grad;
+    auto G = [&](int v) { return g + var_offset(v); };
+    GatherParams gp{}; fill_gather(env, gp);
+    gp.indices = idx_dev; gp.n_items = b; gp.mode = GATHER_INDICES;
+    WGradShape ws[4]; wgrad_shapes(b, ws);
+    const uint32_t ew_blocks = 4096;
+    cudaError_t e = cudaSuccess;
+    auto ok = [&](cudaError_t x) { if (e == cudaSuccess) e = x; return e == cudaSuccess; };
+    // head: dQ, loss, dH (masked), dW5, db5, db4
+    ok(launch_pdl(head_backward_kernel, dim3((b + 7) / 8), dim3(256), 0, s, gp, (const float*)q->t_q, y_dev, (const __nv_bfloat16*)q->a4, (const float*)(q->master + var_offset(8)),
+                  q->t_dq, q->t_loss, q->t_dh, q->t_dh_bf));
+    {
+        const uint32_t rps = colsum_rows_per_split(b), splits = (b + rps - 1) / rps;
+        ok(launch_pdl(head_wgrad_partial_kernel, dim3(16, splits), dim3(32, 8), 0, s, (const __nv_bfloat16*)q->a4, (const float*)q->t_dq, b, rps, q->t_colsum));
+        ok(launch_pdl(colsum_final_kernel, dim3(6), dim3(256), 0, s, (const float*)q->t_colsum, splits, 1536u, 1.0f, G(8)));
+    }
+    ok(launch_colsum(q, q->t_dq, b, 3, 1.0f, G(9), s));
+    if (loss_dev) ok(launch_colsum(q, q->t_loss, b, 1, (float)b, loss_dev, s));
+    ok(launch_colsum(q, q->t_dh, b, 512, 1.0f, G(7), s));
+    // dense 1: dW4 = a3^T dH (K = items), dA3 = dH W4^T, masked by conv3's ReLU
+    ok(launch_wgrad<256>(q, ws[0], LoadA3T{q->a3p, 0, 0}, q->t_dh, G(6), s));
+    if (e == cudaSuccess) ok(launch_gemm<64>(LoadRowMajorBf16{q->t_dh_bf, 512u}, (const __nv_bfloat16*)q->w4k, EpiF32{q->t_d3, b, 3136u}, b, 512u, 3136u, 1u, q->err, s));
+    ok(launch_pdl(mask_conv3_kernel, dim3(ew_blocks), dim3(256), 0, s, q->t_d3, (const __nv_bfloat16*)q->a3p, q->t_d3_bf, b));
+    ok(launch_colsum(q, q->t_d3, b * 49u, 64, 1.0f, G(5), s));
+    // conv3: dW3, dA2 (full correlation), masked by conv2's ReLU
+    ok(launch_wgrad<64>(q, ws[1], LoadIm2colT3{q->a2p, 0, 0}, q->t_d3, G(4), s));
+    if (e == cudaSuccess) ok(launch_gemm<64>(LoadDz3Taps{q->t_d3_bf}, (const __nv_bfloat16*)q->w3r, EpiF32{q->t_d2, b * 81u, 64u}, b * 81u, 576u, 64u, 1u, q->err, s));
+    ok(launch_pdl(mask_conv2_kernel, dim3(ew_blocks), dim3(256), 0, s, q->t_d2, (const __nv_bfloat16*)q->a2p, q->t_d2_bf, b));
+    ok(launch_colsum(q, q->t_d2, b * 81u, 64, 1.0f, G(3), s));
+    // conv2: dW2, dA1 (stride-2 transposed convolution), masked by conv1's ReLU
+    ok(launch_wgrad<64>(q, ws[2], LoadIm2colT2{q->a1p, 0, 0}, q->t_d2, G(2), s));
+    if (e == cudaSuccess) ok(launch_gemm<32>(LoadDz2Taps{q->t_d2_bf}, (const __nv_bfloat16*)q->w2r, EpiF32{q->t_d1, b * 400u, 32u}, b * 400u, 1024u, 32u, 1u, q->err, s));
+    ok(launch_pdl(mask_conv1_kernel, dim3(ew_blocks), dim3(256), 0, s, q->t_d1, (const __nv_bfloat16*)q->a1p, b));
+    ok(launch_colsum(q, q->t_d1, b * 400u, 32, 1.0f, G(1), s));
+    // conv1: dW1 from the u8 ring frames (no data gradient)
+    ok(launch_pdl(qnet_locate_kernel, dim3((b + 127) / 128), dim3(128), 0, s, gp, 0u, q->slot_frame));
+    ok(launch_wgrad<32>(q, ws[3], LoadIm2colT1{env->frames, q->slot_frame, 0, 0}, q->t_d1, G(0), s));
+    if (e != cudaSuccess) return fail(QLC_ERR_CUDA, std::string("qnet backward: ") + cudaGetErrorString(e));
+    if (!apply) return QLC_OK;
+    // per-variable clipnorm + Adam, then the operand copies of the new weights
+    const uint64_t t = ++q->adam_t;
+    const qlc_adam_config& c = q->adam;
+    const double alpha = (double)c.lr * std::sqrt(1.0 - std::pow((double)c.beta2, (double)t)) / (1.0 - std::pow((double)c.beta1, (double)t));
+    ok(launch_pdl(sumsq_partial_kernel, dim3(NVARS, NORM_CHUNKS), dim3(256), 0, s, (const float*)g, q->norm_partial));
+    ok(launch_pdl(adam_kernel, dim3((N_PARAMS + 1023) / 1024), dim3(256), 0, s, q->master, q->adam_m, q->adam_v, (const float*)g, (const float*)q->norm_partial,
+                  AdamStep{(float)alpha, (float)(1.0 - (double)c.beta1), (float)(1.0 - (double)c.beta2), c.epsilon, c.clipnorm}));
+    ok(qnet_prep_weights(q, s));
+    if (e != cudaSuccess) return fail(QLC_ERR_CUDA, std::string("qnet update: ") + cudaGetErrorString(e));
+    return QLC_OK;
+}
+
+extern "C" {
+
+static int32_t check_train_args(qlc_qnet* q, const void* idx, uint32_t batch, uint32_t n_batches, const float* target, qlc_qnet* target_net) {
+    if (!q || !idx) return fail(QLC_ERR_INVALID_ARG, "qnet/indices is null");
+    if (!q->env) return fail(QLC_ERR_INVALID_ARG, "the environment of this Q-network has been destroyed");
+    if (batch == 0) return fail(QLC_ERR_INVALID_ARG, "batch must be > 0");
+    if ((uint64_t)batch * n_batches * 400ull >= 0xFFFFFFFFull) return fail(QLC_ERR_INVALID_ARG, "too many items for one call");
+    if (!target) {
+        if (!target_net) return fail(QLC_ERR_INVALID_ARG, "give either targets or a target network");
+        if (!target_net->env) return fail(QLC_ERR_INVALID_ARG, "the environment of the target network has been destroyed");
+        if (target_net->env != q->env) return fail(QLC_ERR_INVALID_ARG, "the target network belongs to another environment");
+    }
+    if (q->impl < 4) return fail(QLC_ERR_INVALID_ARG, "training reads the saved activations of the shifted-window forward (QLC_QNET_IMPL must be unset)");
+    return QLC_OK;
+}
+
+int32_t qlc_qnet_train(qlc_qnet* q, const uint32_t* idx_dev, uint32_t batch, uint32_t n_batches, const float* target_dev, qlc_qnet* target_net,
+                       float gamma, float* loss_dev, void* stream) {
+    QLC_RANGE("qlc_qnet_train");
+    int32_t rc = check_train_args(q, idx_dev, batch, n_batches, target_dev, target_net); if (rc) return rc;
+    if (n_batches == 0) return QLC_OK;
+    rc = set_device(q->env); if (rc) return rc;
+    cudaStream_t s = (cudaStream_t)stream;
+    const uint32_t n = batch * n_batches;
+    const float* y = target_dev;
+    if (!y) {
+        // TD targets of the whole call from the (fixed) target network: max_a Q_target(state_next), then r / done of the records
+        if (n > q->y_cap) {
+            CUDA_TRY(cudaDeviceSynchronize());
+            qnet_free_targets(q);
+            cudaError_t e = cudaMalloc(&q->t_y, (size_t)n * 4);
+            if (e == cudaSuccess) e = cudaMalloc(&q->t_maxq, (size_t)n * 4);
+            if (e != cudaSuccess) { cudaGetLastError(); qnet_free_targets(q); return fail(QLC_ERR_CUDA, std::string("qnet TD targets: ") + cudaGetErrorString(e)); }
+            q->y_cap = n;
+        }
+        rc = qnet_forward(target_net, idx_dev, n, 1, nullptr, nullptr, q->t_maxq, false, s); if (rc) return rc;
+        GatherParams gp{}; fill_gather(q->env, gp);
+        gp.indices = idx_dev; gp.n_items = n; gp.mode = GATHER_INDICES;
+        CUDA_TRY(launch_pdl(qnet::td_target_kernel, dim3((n + 255) / 256), dim3(256), 0, s, gp, (const float*)q->t_maxq, gamma, q->t_y));
+        y = q->t_y;
+    }
+    for (uint32_t j = 0; j < n_batches; ++j) {
+        rc = qnet_train_step(q, idx_dev + (size_t)j * batch, batch, y + (size_t)j * batch, loss_dev ? loss_dev + j : nullptr, true, s);
+        if (rc) return rc;
+    }
+    return QLC_OK;
+}
+
+// stages host indices / targets in the env's device staging buffer; checks the indices against the replay length
+static int32_t stage_train_inputs(qlc_qnet* q, const uint32_t* idx_host, uint32_t n, const float* target_host, uint32_t n_loss, uint32_t** idx_dev, float** y_dev,
+                                  float** loss_dev) {
+    qlc_env* env = q->env;
+    const uint64_t len = replay_len(env);
+    for (uint32_t i = 0; i < n; ++i) if (idx_host[i] >= len) return fail(QLC_ERR_INVALID_ARG, "replay index out of range");
+    const size_t o_y = ((size_t)n * 4 + 255) & ~(size_t)255, o_l = o_y + (((size_t)n * 4 + 255) & ~(size_t)255), total = o_l + (size_t)n_loss * 4 + 16;
+    int32_t rc = ensure_dev_stage(env, total); if (rc) return rc;
+    uint8_t* dev = (uint8_t*)env->dev_stage;
+    CUDA_TRY(cudaMemcpyAsync(dev, idx_host, (size_t)n * 4, cudaMemcpyHostToDevice, env->own_stream));
+    if (target_host) CUDA_TRY(cudaMemcpyAsync(dev + o_y, target_host, (size_t)n * 4, cudaMemcpyHostToDevice, env->own_stream));
+    *idx_dev = (uint32_t*)dev; *y_dev = target_host ? (float*)(dev + o_y) : nullptr; *loss_dev = (float*)(dev + o_l);
+    return QLC_OK;
+}
+
+int32_t qlc_qnet_train_host(qlc_qnet* q, const uint32_t* idx_host, uint32_t batch, uint32_t n_batches, const float* target_host, qlc_qnet* target_net,
+                            float gamma, float* loss_host) {
+    QLC_RANGE("qlc_qnet_train_host");
+    int32_t rc = check_train_args(q, idx_host, batch, n_batches, target_host, target_net); if (rc) return rc;
+    if (n_batches == 0) return QLC_OK;
+    rc = set_device(q->env); if (rc) return rc;
+    uint32_t* idx_dev; float *y_dev, *loss_dev;
+    rc = stage_train_inputs(q, idx_host, batch * n_batches, target_host, n_batches, &idx_dev, &y_dev, &loss_dev); if (rc) return rc;
+    cudaStream_t s = q->env->own_stream;
+    rc = qlc_qnet_train(q, idx_dev, batch, n_batches, y_dev, target_net, gamma, loss_host ? loss_dev : nullptr, s); if (rc) return rc;
+    if (loss_host) CUDA_TRY(cudaMemcpyAsync(loss_host, loss_dev, (size_t)n_batches * 4, cudaMemcpyDeviceToHost, s));
+    CUDA_TRY(cudaStreamSynchronize(s));
+    uint32_t herr = 0;
+    rc = qlc_qnet_error(q, &herr); if (rc) return rc;
+    if (herr) return fail(QLC_ERR_CUDA, "qnet: an MMA completion barrier timed out");
+    return QLC_OK;
+}
+
+int32_t qlc_qnet_debug_grads(qlc_qnet* q, const uint32_t* idx_host, uint32_t n, const float* target_host, const qlc_qnet_weights* grads_out) {
+    int32_t rc = check_train_args(q, idx_host, n, 1, target_host, nullptr); if (rc) return rc;
+    if (!grads_out) return fail(QLC_ERR_INVALID_ARG, "grads_out is null");
+    const float* dst[qnet::NVARS];
+    weight_ptrs(grads_out, dst);
+    for (int i = 0; i < qnet::NVARS; ++i) if (!dst[i]) return fail(QLC_ERR_INVALID_ARG, "a gradient pointer is null");
+    rc = set_device(q->env); if (rc) return rc;
+    uint32_t* idx_dev; float *y_dev, *loss_dev;
+    rc = stage_train_inputs(q, idx_host, n, target_host, 1, &idx_dev, &y_dev, &loss_dev); if (rc) return rc;
+    cudaStream_t s = q->env->own_stream;
+    rc = qnet_train_step(q, idx_dev, n, y_dev, nullptr, false, s); if (rc) return rc;
+    CUDA_TRY(cudaStreamSynchronize(s));
+    uint32_t herr = 0;
+    rc = qlc_qnet_error(q, &herr); if (rc) return rc;
+    if (herr) return fail(QLC_ERR_CUDA, "qnet: an MMA completion barrier timed out");
+    for (int v = 0; v < qnet::NVARS; ++v) CUDA_TRY(cudaMemcpy(const_cast<float*>(dst[v]), q->grad + qnet::var_offset(v), (size_t)qnet::var_size(v) * 4, cudaMemcpyDeviceToHost));
     return QLC_OK;
 }
 

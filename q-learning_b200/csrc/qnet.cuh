@@ -157,12 +157,33 @@ __global__ void prep_head_kernel(const float* __restrict__ kernel /*[512][3]*/, 
 // walks the 128-row M tiles blockIdx.x, +gridDim.x, ... K is consumed in 64-element chunks through a 2-stage shared-memory
 // ring that runs on across tile boundaries: while the tensor core works on chunk g the threads already gather chunk g+1
 // (global loads in flight) and chunk g-1's stage is being refilled; completion per stage via tcgen05.commit -> mbarrier.
-// W: bf16 [N_TOTAL][K] (K-major). out: bf16 [M][N_TOTAL]. NT in {32, 64, 128, 256}; K % 64 == 0.
+// W: bf16 [N_TOTAL][K] (K-major). The epilogue policy stores the accumulators. NT in {32, 64, 128, 256}; K % 64 == 0.
 // ---------------------------------------------------------------------------------------------------------
-template <int NT, class Loader>
-__global__ void __launch_bounds__(128) gemm_tc_kernel(Loader ld, const __nv_bfloat16* __restrict__ w, const float* __restrict__ bias,
-                                                     __nv_bfloat16* __restrict__ out, uint32_t m_total, uint32_t k_total, uint32_t n_total, int relu,
-                                                     unsigned int* err_flag) {
+// Epilogue policies: store8(row, n, v) receives the f32 accumulators of columns n .. n+7 of one row.
+struct EpiBiasAct {                  // out bf16 [M][n_total] = act(acc + bias)
+    const float* bias; __nv_bfloat16* out; uint32_t n_total; int relu;
+    __device__ __forceinline__ void store8(uint32_t row, uint32_t n, const uint32_t (&v)[8]) const {
+        float f[8];
+        #pragma unroll
+        for (int i = 0; i < 8; ++i) { f[i] = __uint_as_float(v[i]) + bias[n + i]; if (relu) f[i] = fmaxf(f[i], 0.0f); }
+        *reinterpret_cast<uint4*>(out + (size_t)row * n_total + n) =
+            make_uint4(pack_bf16(f[0], f[1]), pack_bf16(f[2], f[3]), pack_bf16(f[4], f[5]), pack_bf16(f[6], f[7]));
+    }
+};
+struct EpiF32 {                      // out f32 [gridDim.z][m_total][n_total]: the raw accumulators, one slice per K split
+    float* out; uint32_t m_total, n_total;
+    __device__ __forceinline__ void store8(uint32_t row, uint32_t n, const uint32_t (&v)[8]) const {
+        float4* o = reinterpret_cast<float4*>(out + ((size_t)blockIdx.z * m_total + row) * n_total + n);
+        o[0] = make_float4(__uint_as_float(v[0]), __uint_as_float(v[1]), __uint_as_float(v[2]), __uint_as_float(v[3]));
+        o[1] = make_float4(__uint_as_float(v[4]), __uint_as_float(v[5]), __uint_as_float(v[6]), __uint_as_float(v[7]));
+    }
+};
+
+// Split K: blockIdx.z selects a K slice. W holds the slices back to back ([gridDim.z][N_TOTAL][k_total]); the loader offsets
+// its own K by blockIdx.z (the forward runs with gridDim.z = 1).
+template <int NT, class Loader, class Epi>
+__global__ void __launch_bounds__(128) gemm_tc_kernel(Loader ld, const __nv_bfloat16* __restrict__ w, Epi epi, uint32_t m_total, uint32_t k_total,
+                                                     uint32_t n_total, unsigned int* err_flag) {
     static_assert(NT % 16 == 0 && NT >= 32 && NT <= 256, "NT");
     constexpr uint32_t A_BYTES = TILE_M * KC * 2;              // 16 KB per stage
     constexpr uint32_t B_BYTES = (uint32_t)NT * KC * 2;
@@ -186,7 +207,7 @@ __global__ void __launch_bounds__(128) gemm_tc_kernel(Loader ld, const __nv_bflo
 
     const uint32_t n_chunks = k_total / KC;
     const uint32_t n_mtiles = (m_total + TILE_M - 1) / TILE_M;
-    const __nv_bfloat16* wrow = w + (size_t)n0 * k_total;
+    const __nv_bfloat16* wrow = w + ((size_t)blockIdx.z * n_total + n0) * k_total;
 
     uint4 av[KC / 8], bv[BV];
     auto gather = [&](const typename Loader::Row& r, bool row_ok, uint32_t c) {
@@ -250,13 +271,7 @@ __global__ void __launch_bounds__(128) gemm_tc_kernel(Loader ld, const __nv_bflo
                 for (int col = 0; col < NT; col += 8) {
                     uint32_t v[8];
                     tmem_ld8(tmem_base + ((warp * 32u) << 16) + (uint32_t)col, v);
-                    if (row_ok) {
-                        float f[8];
-                        #pragma unroll
-                        for (int i = 0; i < 8; ++i) { f[i] = __uint_as_float(v[i]) + bias[n0 + col + i]; if (relu) f[i] = fmaxf(f[i], 0.0f); }
-                        *reinterpret_cast<uint4*>(out + (size_t)my_row * n_total + n0 + col) =
-                            make_uint4(pack_bf16(f[0], f[1]), pack_bf16(f[2], f[3]), pack_bf16(f[4], f[5]), pack_bf16(f[6], f[7]));
-                    }
+                    if (row_ok) epi.store8(my_row, n0 + (uint32_t)col, v);
                 }
                 tc_fence_before();                             // the next tile's first MMA overwrites the accumulator
                 __syncthreads();

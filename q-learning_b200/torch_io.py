@@ -116,3 +116,58 @@ class TensorCoreActor:
 
     def close(self):
         self.qnet.close()
+
+
+class TensorCoreLearner:
+    """The three DeepQLearningModel methods (ml_model/model.rs:29-77) on the library's tcgen05 Q-network, training included,
+    with an online and a target (stabilized) network on the replay ring of `env`: `predict_action()` for every env,
+    `train_indices(idx)` — `n_batches` Keras-Adam updates on replay transitions by index, the TD target
+    y = r + max Q_target(s') * gamma (y = r where done) computed on the device — and `sync_target()`. No state tensor is
+    materialised anywhere: the kernels read the u8 frames where the step kernel wrote them. `weights`: Keras-layout f32 arrays
+    (QNET_SHAPES) for both networks."""
+
+    def __init__(self, env, weights, gamma=0.99, lr=2.5e-4, clipnorm=1.0):
+        from . import QNetwork
+        self.env, self.gamma = env, float(gamma)
+        self.online = QNetwork(env, weights)
+        self.target = QNetwork(env, weights)
+        self.online.set_adam(lr=lr, clipnorm=clipnorm)
+        dev = torch.device("cuda", env.device)
+        self.actions = torch.empty((1, env.n_envs), dtype=torch.uint8, device=dev)
+        self.losses = []
+
+    def predict_action(self):
+        """Greedy action of every env as a CUDA u8 tensor [1][n_envs] (the shape `step` takes)."""
+        self.online.forward_device(None, self.env.n_envs, 0, None, self.actions.data_ptr(), None, _stream())
+        return self.actions
+
+    def train_indices(self, indices):
+        """One update per row of `indices` (CUDA int32 / uint32 tensor [n_batches][batch], e.g. DeviceSampler.indices filled by
+        ReplayBuffer.sample_device); returns the CUDA f32 tensor [n_batches] of losses, each before its update."""
+        if indices.dim() != 2 or not indices.is_cuda or not indices.is_contiguous() or indices.dtype not in (torch.int32, torch.uint32):
+            raise QlError("indices must be a contiguous int32 CUDA tensor [n_batches][batch]")
+        nb, batch = indices.shape
+        loss = torch.empty(nb, dtype=torch.float32, device=indices.device)
+        self.online.train_device(indices.data_ptr(), batch, nb, None, self.target, self.gamma, loss.data_ptr(), _stream())
+        self.losses.append(loss)
+        return loss
+
+    def sync_target(self):
+        """target <- online (get + set of the f32 master weights)."""
+        self.target.set_weights(self.online.get_weights())
+
+    def get_weights(self):
+        return self.online.get_weights()
+
+    def write_checkpoint(self, path):
+        """The online network's weights as an .npz of the Keras arrays (QNET_SHAPES names)."""
+        import numpy as np
+        np.savez(path, **self.online.get_weights())
+
+    def error(self):
+        """Sticky MMA time-out flags of both networks (0 = fine); synchronises."""
+        return self.online.error() | self.target.error()
+
+    def close(self):
+        self.online.close()
+        self.target.close()
