@@ -1318,7 +1318,6 @@ static cudaError_t launch_gemm(const Loader& ld, const __nv_bfloat16* w, const E
         if (e != cudaSuccess) return e;
         int dev = 0; cudaGetDevice(&dev); cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
         const int tmem_limit = 512 / (NT <= 32 ? 32 : (NT <= 64 ? 64 : (NT <= 128 ? 128 : 256)));   // TMEM columns per SM
-        if (getenv("QLC_DEBUG_OCC")) fprintf(stderr, "gemm_tc NT=%d dyn=%zu occ(api)=%d tmem_limit=%d sms=%d\n", NT, dyn, occ, tmem_limit, sms);
         if (occ > tmem_limit) occ = tmem_limit;
         if (occ < 1) occ = 1;
     }
@@ -1328,11 +1327,6 @@ static cudaError_t launch_gemm(const Loader& ld, const __nv_bfloat16* w, const E
     if (gx > n_mtiles) gx = n_mtiles;
     kern<<<dim3(gx, n_ntiles, n_splits), 128, dyn, s>>>(ld, w, epi, m, k, n_total, err);
     return cudaGetLastError();
-}
-template <int NT, class Loader>
-static cudaError_t launch_gemm_tc(const Loader& ld, const __nv_bfloat16* w, const float* bias, __nv_bfloat16* out, uint32_t m, uint32_t k, uint32_t n_total,
-                                  int relu, unsigned int* err, cudaStream_t s) {
-    return launch_gemm<NT>(ld, w, qnet::EpiBiasAct{bias, out, n_total, relu}, m, k, n_total, 1u, err, s);
 }
 
 template <class G, class Out>
@@ -1356,14 +1350,13 @@ extern "C" {
 struct qlc_qnet {
     qlc_env* env = nullptr;                                                 // NULL once the env has been destroyed: every call but destroy fails
     int device = 0;
-    __nv_bfloat16 *w1 = nullptr, *w2 = nullptr, *w3 = nullptr, *w4 = nullptr; float* w5 = nullptr;
+    float* w5 = nullptr;
     float *b1 = nullptr, *b2 = nullptr, *b3 = nullptr, *b4 = nullptr, *b5 = nullptr;
     __nv_bfloat16 *w1p = nullptr, *w2p = nullptr, *w3p = nullptr, *w4p = nullptr, *w4p256 = nullptr;   // operand-layout weights (dense: N tiles of 128 and of 256): planes [K/8][N][8]
-    __nv_bfloat16 *a1 = nullptr, *a2 = nullptr, *a3 = nullptr, *a4 = nullptr; uint32_t* slot_frame = nullptr; unsigned int* err = nullptr;
+    __nv_bfloat16* a4 = nullptr; uint32_t* slot_frame = nullptr; unsigned int* err = nullptr;
     float4* head_partial = nullptr; uint32_t* head_count = nullptr;       // dense epilogue -> fused head (per-N-tile partials, per-row tickets)
     __nv_bfloat16 *a1p = nullptr, *a2p = nullptr, *a3p = nullptr;         // conv outputs in the next layer's operand (plane) layout
     unsigned long long* prof = nullptr;                                    // QLC_QNET_PROF: per-role cycle counters of CTA 0, printed after each forward
-    int impl = 4;                                                          // how many convs run as shifted-window kernels (QLC_QNET_IMPL, A/B testing)
     uint32_t cap_items = 0;
     // training (qlc_qnet_train): f32 masters of the 10 Keras variables back to back (b1..b5 point into it), their gradients,
     // Adam moments; bf16 weight copies in the data-gradient GEMMs' operand layouts; scratch sized for train_cap items
@@ -1392,8 +1385,8 @@ static void qnet_free_targets(qlc_qnet* q) {
 static void qnet_free_train(qlc_qnet* q) { qnet_free_scratch(q); qnet_free_targets(q); }
 
 static void qnet_free_acts(qlc_qnet* q) {
-    cudaFree(q->a1); cudaFree(q->a2); cudaFree(q->a3); cudaFree(q->a4); cudaFree(q->slot_frame); cudaFree(q->a1p); cudaFree(q->a2p); cudaFree(q->a3p); cudaFree(q->head_partial); cudaFree(q->head_count);
-    q->a1 = q->a2 = q->a3 = q->a4 = q->a1p = q->a2p = q->a3p = nullptr; q->head_partial = nullptr; q->head_count = nullptr; q->slot_frame = nullptr; q->cap_items = 0;
+    cudaFree(q->a4); cudaFree(q->slot_frame); cudaFree(q->a1p); cudaFree(q->a2p); cudaFree(q->a3p); cudaFree(q->head_partial); cudaFree(q->head_count);
+    q->a4 = q->a1p = q->a2p = q->a3p = nullptr; q->head_partial = nullptr; q->head_count = nullptr; q->slot_frame = nullptr; q->cap_items = 0;
 }
 
 }  // extern "C"
@@ -1406,10 +1399,10 @@ static void qnet_release_device(qlc_qnet* q) {
     cudaDeviceSynchronize();
     qnet_free_acts(q);
     qnet_free_train(q);
-    cudaFree(q->w1); cudaFree(q->w2); cudaFree(q->w3); cudaFree(q->w4); cudaFree(q->w5); cudaFree(q->w1p); cudaFree(q->w2p); cudaFree(q->w3p); cudaFree(q->w4p); cudaFree(q->w4p256);
+    cudaFree(q->w5); cudaFree(q->w1p); cudaFree(q->w2p); cudaFree(q->w3p); cudaFree(q->w4p); cudaFree(q->w4p256);
     cudaFree(q->master); cudaFree(q->grad); cudaFree(q->adam_m); cudaFree(q->adam_v); cudaFree(q->norm_partial); cudaFree(q->w4k); cudaFree(q->w3r); cudaFree(q->w2r);
     cudaFree(q->err); cudaFree(q->prof);
-    q->w1 = q->w2 = q->w3 = q->w4 = q->w1p = q->w2p = q->w3p = q->w4p = q->w4p256 = nullptr; q->w5 = nullptr;
+    q->w1p = q->w2p = q->w3p = q->w4p = q->w4p256 = nullptr; q->w5 = nullptr;
     q->master = q->grad = q->adam_m = q->adam_v = q->norm_partial = nullptr; q->w4k = q->w3r = q->w2r = nullptr;
     q->b1 = q->b2 = q->b3 = q->b4 = q->b5 = nullptr; q->err = nullptr; q->prof = nullptr;
     q->env = nullptr;
@@ -1455,13 +1448,9 @@ static const float* const* weight_ptrs(const qlc_qnet_weights* w, const float* (
 static cudaError_t qnet_prep_weights(qlc_qnet* q, cudaStream_t s) {
     const float* m = q->master;
     auto V = [&](int v) { return m + qnet::var_offset(v); };
-    qnet::prep_conv1_kernel<<<(32 * 256 + 255) / 256, 256, 0, s>>>(V(0), q->w1);
     qnet::prep_conv1_planes_kernel<<<(32 * 256 + 255) / 256, 256, 0, s>>>(V(0), q->w1p);
-    qnet::prep_transpose_kernel<<<(512 * 64 + 255) / 256, 256, 0, s>>>(V(2), q->w2, 512, 64);             // [kh][kw][c][cout] = [K][N]
     qnet::prep_conv2_planes_kernel<<<(512 * 64 + 255) / 256, 256, 0, s>>>(V(2), q->w2p);
-    qnet::prep_transpose_kernel<<<(576 * 64 + 255) / 256, 256, 0, s>>>(V(4), q->w3, 576, 64);
     qnet::prep_conv3_planes_kernel<<<(576 * 64 + 255) / 256, 256, 0, s>>>(V(4), q->w3p);
-    qnet::prep_transpose_kernel<<<(3136 * 512 + 255) / 256, 256, 0, s>>>(V(6), q->w4, 3136, 512);
     qnet::prep_dense_planes_kernel<128><<<(3136 * 512 + 255) / 256, 256, 0, s>>>(V(6), q->w4p);
     qnet::prep_dense_planes_kernel<256><<<(3136 * 512 + 255) / 256, 256, 0, s>>>(V(6), q->w4p256);
     qnet::prep_head_kernel<<<(3 * 512 + 255) / 256, 256, 0, s>>>(V(8), q->w5);
@@ -1524,9 +1513,8 @@ int32_t qlc_qnet_create(qlc_env* env, const qlc_qnet_weights* w, qlc_qnet** out)
     env->qnets.push_back(q);
     cudaError_t e = cudaSuccess;
     auto A = [&](void** p, size_t bytes) { if (e == cudaSuccess) e = cudaMalloc(p, bytes); };
-    A((void**)&q->w1, 32 * 256 * 2); A((void**)&q->w2, 64 * 512 * 2); A((void**)&q->w3, 64 * 576 * 2); A((void**)&q->w4, (size_t)512 * 3136 * 2); A((void**)&q->w5, 3 * 512 * 4);
+    A((void**)&q->w5, 3 * 512 * 4);
     A((void**)&q->w1p, 32 * 256 * 2); A((void**)&q->w2p, 64 * 512 * 2); A((void**)&q->w3p, 64 * 576 * 2); A((void**)&q->w4p, (size_t)512 * 3136 * 2); A((void**)&q->w4p256, (size_t)512 * 3136 * 2);
-    if (const char* v = getenv("QLC_QNET_IMPL")) q->impl = atoi(v);
     if (getenv("QLC_QNET_PROF")) A((void**)&q->prof, 3 * 32 * 8);
     A((void**)&q->master, (size_t)qnet::N_PARAMS * 4); A((void**)&q->grad, (size_t)qnet::N_PARAMS * 4);
     A((void**)&q->adam_m, (size_t)qnet::N_PARAMS * 4); A((void**)&q->adam_v, (size_t)qnet::N_PARAMS * 4); A((void**)&q->norm_partial, qnet::NVARS * qnet::NORM_CHUNKS * 4);
@@ -1559,8 +1547,7 @@ static int32_t qnet_forward(qlc_qnet* q, const uint32_t* idx_dev, uint32_t n, in
     if (n > q->cap_items) {
         CUDA_TRY(cudaDeviceSynchronize());
         qnet_free_acts(q);
-        CUDA_TRY(cudaMalloc(&q->a1, (size_t)n * 400 * 32 * 2)); CUDA_TRY(cudaMalloc(&q->a2, (size_t)n * 81 * 64 * 2));
-        CUDA_TRY(cudaMalloc(&q->a3, (size_t)n * 49 * 64 * 2)); CUDA_TRY(cudaMalloc(&q->a4, (size_t)n * 512 * 2)); CUDA_TRY(cudaMalloc(&q->slot_frame, (size_t)n * 16));
+        CUDA_TRY(cudaMalloc(&q->a4, (size_t)n * 512 * 2)); CUDA_TRY(cudaMalloc(&q->slot_frame, (size_t)n * 16));
         const size_t a1p_bytes = (size_t)((n + qnet::Conv2Geom::B - 1) / qnet::Conv2Geom::B) * qnet::Conv2Geom::STAGE_BYTES;
         const size_t a2p_bytes = (size_t)((n + qnet::Conv3Geom::B - 1) / qnet::Conv3Geom::B) * qnet::Conv3Geom::STAGE_BYTES;
         CUDA_TRY(cudaMalloc(&q->a1p, a1p_bytes)); CUDA_TRY(cudaMalloc(&q->a2p, a2p_bytes));
@@ -1574,59 +1561,34 @@ static int32_t qnet_forward(qlc_qnet* q, const uint32_t* idx_dev, uint32_t n, in
     }
     GatherParams g{}; fill_gather(env, g);
     g.indices = idx_dev; g.n_items = n; g.mode = idx_dev ? GATHER_INDICES : GATHER_CURRENT;
-    cudaError_t e;
-    const int impl = q->impl;
-    if (impl >= 1) {
-        // conv1's loader works out where each item's four frames are (the gather kernels' locate()) - no separate kernel
-        qnet::ConvArgs a{(const uint8_t*)q->w1p, q->b1, env->frames, g, which ? 1u : 0u, n, q->err, q->prof};
-        e = impl >= 2 ? launch_conv_sw<qnet::Conv1Geom>(a, qnet::OutConv2Planes{q->a1p}, s) : launch_conv_sw<qnet::Conv1Geom>(a, qnet::OutXYC{q->a1, 20, 20, 32}, s);
-    } else {
-        CUDA_TRY(launch_pdl(qnet::qnet_locate_kernel, dim3((n + 127) / 128), dim3(128), 0, s, g, which ? 1u : 0u, q->slot_frame));
-        qnet::LoadConv1FromRing l1{env->frames, q->slot_frame};
-        e = launch_gemm_tc<32>(l1, q->w1, q->b1, q->a1, n * 400u, 256u, 32u, 1, q->err, s);
-    }
+    // conv1's loader works out where each item's four frames are (the gather kernels' locate()) - no separate kernel
+    const qnet::ConvArgs c1{(const uint8_t*)q->w1p, q->b1, env->frames, g, which ? 1u : 0u, n, q->err, q->prof};
+    cudaError_t e = launch_conv_sw<qnet::Conv1Geom>(c1, qnet::OutConv2Planes{q->a1p}, s);
     if (e != cudaSuccess) return fail(QLC_ERR_CUDA, std::string("conv1: ") + cudaGetErrorString(e));
-    if (impl >= 2) {
-        qnet::ConvArgs a{(const uint8_t*)q->w2p, q->b2, (const uint8_t*)q->a1p, GatherParams{}, 0u, n, q->err, q->prof ? q->prof + 32 : nullptr};
-        e = impl >= 3 ? launch_conv_sw<qnet::Conv2Geom>(a, qnet::OutConv3Planes{q->a2p}, s) : launch_conv_sw<qnet::Conv2Geom>(a, qnet::OutXYC{q->a2, 9, 9, 64}, s);
-    } else {
-        qnet::LoadConvNHWC l2{q->a1, 20, 20, 32, 9, 9, 4, 4, 2};
-        e = launch_gemm_tc<64>(l2, q->w2, q->b2, q->a2, n * 81u, 512u, 64u, 1, q->err, s);
-    }
+    const qnet::ConvArgs c2{(const uint8_t*)q->w2p, q->b2, (const uint8_t*)q->a1p, GatherParams{}, 0u, n, q->err, q->prof ? q->prof + 32 : nullptr};
+    e = launch_conv_sw<qnet::Conv2Geom>(c2, qnet::OutConv3Planes{q->a2p}, s);
     if (e != cudaSuccess) return fail(QLC_ERR_CUDA, std::string("conv2: ") + cudaGetErrorString(e));
-    if (impl >= 3) {
-        qnet::ConvArgs a{(const uint8_t*)q->w3p, q->b3, (const uint8_t*)q->a2p, GatherParams{}, 0u, n, q->err, q->prof ? q->prof + 64 : nullptr};
-        e = impl >= 4 ? launch_conv_sw<qnet::Conv3Geom>(a, qnet::OutDensePlanes{q->a3p}, s) : launch_conv_sw<qnet::Conv3Geom>(a, qnet::OutXYC{q->a3, 7, 7, 64}, s);
-    } else {
-        qnet::LoadConvNHWC l3{q->a2, 9, 9, 64, 7, 7, 3, 3, 1};
-        e = launch_gemm_tc<64>(l3, q->w3, q->b3, q->a3, n * 49u, 576u, 64u, 1, q->err, s);
-    }
+    const qnet::ConvArgs c3{(const uint8_t*)q->w3p, q->b3, (const uint8_t*)q->a2p, GatherParams{}, 0u, n, q->err, q->prof ? q->prof + 64 : nullptr};
+    e = launch_conv_sw<qnet::Conv3Geom>(c3, qnet::OutDensePlanes{q->a3p}, s);
     if (e != cudaSuccess) return fail(QLC_ERR_CUDA, std::string("conv3: ") + cudaGetErrorString(e));
-    if (impl >= 4) {
-        static bool attr_set[64] = {};
-        if (!attr_set[env->cfg.device & 63]) {
-            CUDA_TRY(cudaFuncSetAttribute(qnet::dense_tc_kernel<128>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)qnet::DenseGeomT<128>::SMEM_BYTES));
-            CUDA_TRY(cudaFuncSetAttribute(qnet::dense_tc_kernel<256>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)qnet::DenseGeomT<256>::SMEM_BYTES));
-            attr_set[env->cfg.device & 63] = true;
-        }
-        // N tiles of 128 while (M tiles x 2) CTAs would leave SMs idle (the layer is bound by per-SM L2 ingest), 256 beyond
-        const uint32_t m_tiles = (n + 127) / 128;
-        static const int nt_force = getenv("QLC_QNET_DENSE_NT") ? atoi(getenv("QLC_QNET_DENSE_NT")) : 0;
-        const bool narrow = nt_force ? nt_force == 128 : m_tiles * 2u < (uint32_t)env->sm_count;
-        // the head (Dense 512 -> 3, argmax, max) runs in the dense epilogue; rows_padded is that of the allocation (cap_items)
-        const qnet::HeadArgs head{q->w5, q->b5, q->head_partial, q->head_count, ((q->cap_items + 127u) / 128u) * 128u, q_dev, action_dev, max_q_dev};
-        __nv_bfloat16* hidden = hidden_out ? q->a4 : nullptr;             // the 512 hidden activations are only needed by training
-        if (narrow)
-            CUDA_TRY(launch_pdl(qnet::dense_tc_kernel<128>, dim3(m_tiles, 4), dim3(qnet::DenseGeomT<128>::THREADS), qnet::DenseGeomT<128>::SMEM_BYTES, s, (const uint8_t*)q->a3p,
-                                (const uint8_t*)q->w4p, (const float*)q->b4, hidden, n, q->err, head));
-        else
-            CUDA_TRY(launch_pdl(qnet::dense_tc_kernel<256>, dim3(m_tiles, 2), dim3(qnet::DenseGeomT<256>::THREADS), qnet::DenseGeomT<256>::SMEM_BYTES, s, (const uint8_t*)q->a3p,
-                                (const uint8_t*)q->w4p256, (const float*)q->b4, hidden, n, q->err, head));
-    } else {
-        qnet::LoadRowMajorBf16 l4{q->a3, 3136u};
-        e = launch_gemm_tc<128>(l4, q->w4, q->b4, q->a4, n, 3136u, 512u, 1, q->err, s); if (e != cudaSuccess) return fail(QLC_ERR_CUDA, std::string("dense1: ") + cudaGetErrorString(e));
-        qnet::head_kernel<<<(n + 7) / 8, 256, 0, s>>>(q->a4, q->w5, q->b5, q_dev, action_dev, max_q_dev, n);
+    static bool attr_set[64] = {};
+    if (!attr_set[env->cfg.device & 63]) {
+        CUDA_TRY(cudaFuncSetAttribute(qnet::dense_tc_kernel<128>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)qnet::DenseGeomT<128>::SMEM_BYTES));
+        CUDA_TRY(cudaFuncSetAttribute(qnet::dense_tc_kernel<256>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)qnet::DenseGeomT<256>::SMEM_BYTES));
+        attr_set[env->cfg.device & 63] = true;
     }
+    // N tiles of 128 while (M tiles x 2) CTAs would leave SMs idle (the layer is bound by per-SM L2 ingest), 256 beyond
+    const uint32_t m_tiles = (n + 127) / 128;
+    const bool narrow = m_tiles * 2u < (uint32_t)env->sm_count;
+    // the head (Dense 512 -> 3, argmax, max) runs in the dense epilogue; rows_padded is that of the allocation (cap_items)
+    const qnet::HeadArgs head{q->w5, q->b5, q->head_partial, q->head_count, ((q->cap_items + 127u) / 128u) * 128u, q_dev, action_dev, max_q_dev};
+    __nv_bfloat16* hidden = hidden_out ? q->a4 : nullptr;                 // the 512 hidden activations are only needed by training
+    if (narrow)
+        CUDA_TRY(launch_pdl(qnet::dense_tc_kernel<128>, dim3(m_tiles, 4), dim3(qnet::DenseGeomT<128>::THREADS), qnet::DenseGeomT<128>::SMEM_BYTES, s, (const uint8_t*)q->a3p,
+                            (const uint8_t*)q->w4p, (const float*)q->b4, hidden, n, q->err, head));
+    else
+        CUDA_TRY(launch_pdl(qnet::dense_tc_kernel<256>, dim3(m_tiles, 2), dim3(qnet::DenseGeomT<256>::THREADS), qnet::DenseGeomT<256>::SMEM_BYTES, s, (const uint8_t*)q->a3p,
+                            (const uint8_t*)q->w4p256, (const float*)q->b4, hidden, n, q->err, head));
     CUDA_TRY(cudaGetLastError());
     if (q->prof) {
         unsigned long long h[96];
@@ -1813,7 +1775,6 @@ static int32_t check_train_args(qlc_qnet* q, const void* idx, uint32_t batch, ui
         if (!target_net->env) return fail(QLC_ERR_INVALID_ARG, "the environment of the target network has been destroyed");
         if (target_net->env != q->env) return fail(QLC_ERR_INVALID_ARG, "the target network belongs to another environment");
     }
-    if (q->impl < 4) return fail(QLC_ERR_INVALID_ARG, "training reads the saved activations of the shifted-window forward (QLC_QNET_IMPL must be unset)");
     return QLC_OK;
 }
 
@@ -1919,13 +1880,14 @@ int32_t qlc_debug_gemm_bf16(const float* a_host, const float* w_host, const floa
     if (e == cudaSuccess) {
         qnet::f32_to_bf16_kernel<<<256, 256>>>(da, ba, (size_t)m * k);
         qnet::f32_to_bf16_kernel<<<256, 256>>>(dw, bw, (size_t)n * k);
-        qnet::LoadRowMajorBf16 ld{ba, k};
+        const qnet::LoadRowMajorBf16 ld{ba, k};
+        const qnet::EpiBiasAct epi{db, bo, n, relu};
         switch (n) {
-            case 32: e = launch_gemm_tc<32>(ld, bw, db, bo, m, k, n, relu, derr, nullptr); break;
-            case 64: e = launch_gemm_tc<64>(ld, bw, db, bo, m, k, n, relu, derr, nullptr); break;
-            case 128: e = launch_gemm_tc<128>(ld, bw, db, bo, m, k, n, relu, derr, nullptr); break;
-            case 256: e = launch_gemm_tc<256>(ld, bw, db, bo, m, k, n, relu, derr, nullptr); break;
-            default: e = launch_gemm_tc<128>(ld, bw, db, bo, m, k, n, relu, derr, nullptr); break;      // 512 = 4 N tiles of 128
+            case 32: e = launch_gemm<32>(ld, bw, epi, m, k, n, 1u, derr, nullptr); break;
+            case 64: e = launch_gemm<64>(ld, bw, epi, m, k, n, 1u, derr, nullptr); break;
+            case 128: e = launch_gemm<128>(ld, bw, epi, m, k, n, 1u, derr, nullptr); break;
+            case 256: e = launch_gemm<256>(ld, bw, epi, m, k, n, 1u, derr, nullptr); break;
+            default: e = launch_gemm<128>(ld, bw, epi, m, k, n, 1u, derr, nullptr); break;      // 512 = 4 N tiles of 128
         }
     }
     unsigned int herr = 0;

@@ -1,15 +1,15 @@
-// qnet.cuh — Q-network forward on the 5th-generation tensor cores (SURVEY.md §8f-3: the only tensor-core-worthy piece
-// next to the hot path; closes the actor loop on the GPU). Architecture = the reference's Keras model
-// (/root/reference/src/ql-with-tensorflow/python_model/create_ql_model_breakout_84x84x4_3_32.py:17-33):
+// qnet.cuh — tcgen05 (5th-generation tensor core) helpers and gemm_tc_kernel, the GEMM engine of the Q-network's backward
+// pass (qnet_train.cuh: weight gradients with split K, data gradients) and of the qlc_debug_gemm_bf16 test hook. The forward
+// runs on the shifted-window convolutions and the bulk-copy fed dense layer of qnet_conv.cuh, which share the helpers.
+// Architecture = the reference's Keras model (/root/reference/src/ql-with-tensorflow/python_model/create_ql_model_breakout_84x84x4_3_32.py:17-33):
 //   Conv(32, 8x8, stride 4) -> Conv(64, 4x4, stride 2) -> Conv(64, 3x3, stride 1) -> Dense 512 -> Dense 3, ReLU between.
-// Every layer is an implicit GEMM  C[M x N] = act(A[M x K] * W[N x K]^T + bias)  with M = (env, output pixel), bf16 operands,
-// f32 accumulation in TMEM:
-//   * one CTA (128 threads) owns a 128-row tile of M and all N columns (N <= 512 = the whole TMEM);
-//   * A is gathered by the threads (im2col on the fly; conv1 reads the u8 frames STRAIGHT from the replay frame ring, with
-//     the ring-slot rotation and episode-start zero fill of the reference's FrameRingBuffer) into the canonical K-major,
-//     non-swizzled core-matrix layout (8 rows x 16 bytes per core matrix), W likewise;
+// gemm_tc_kernel: C[M x N] = A[M x K] * W[N x K]^T, bf16 operands, f32 accumulation in TMEM:
+//   * one CTA (128 threads) owns a 128-row tile of M and one N tile of NT <= 256 columns;
+//   * the threads gather A through a loader policy, and W, into the canonical K-major, non-swizzled core-matrix layout
+//     (8 rows x 16 bytes per core matrix);
 //   * one elected thread issues tcgen05.mma (cta_group::1, kind::f16, M = 128) from shared-memory descriptors, completion
-//     via tcgen05.commit -> mbarrier; the epilogue reads TMEM with tcgen05.ld (32x32b), adds bias, applies ReLU, writes bf16.
+//     via tcgen05.commit -> mbarrier; the epilogue reads TMEM with tcgen05.ld (32x32b) and hands the f32 accumulators to an
+//     epilogue policy.
 #pragma once
 #include <stdint.h>
 #include <cuda_runtime.h>
@@ -79,49 +79,12 @@ __device__ __forceinline__ uint32_t pack_bf16(float a, float b) {
 }
 
 // ---- A-operand loaders: prepare(row) hoists the per-row index math, load8() returns 8 consecutive K elements (16 B) ----
-struct LoadRowMajorBf16 {            // plain GEMM: A bf16 [M][K] row-major (Dense layers, and conv outputs flattened)
+struct LoadRowMajorBf16 {            // plain GEMM: A bf16 [M][K] row-major (dH of the dA3 GEMM, the debug hook)
     const __nv_bfloat16* a; uint32_t k_total;
     struct Row { const __nv_bfloat16* p; };
     __device__ __forceinline__ Row prepare(uint32_t row) const { return Row{a + (size_t)row * k_total}; }
     __device__ __forceinline__ uint4 load8(const Row& r, uint32_t kchunk) const { return __ldg(reinterpret_cast<const uint4*>(r.p + (size_t)kchunk * 8)); }
 };
-struct LoadConvNHWC {                // conv over bf16 activations [B][H][W][C] (C % 8 == 0), K order (kh, kw, c)
-    const __nv_bfloat16* act; int H, W, C, OH, OW, KH, KW, stride;
-    struct Row { const __nv_bfloat16* p; };
-    __device__ __forceinline__ Row prepare(uint32_t row) const {
-        const int per = OH * OW;
-        const int b = row / per, pos = row - b * per;
-        const int oh = pos / OW, ow = pos - oh * OW;
-        return Row{act + (((size_t)b * H + oh * stride) * W + ow * stride) * C};
-    }
-    __device__ __forceinline__ uint4 load8(const Row& r, uint32_t kchunk) const {
-        const int k = kchunk * 8;
-        const int kk = k / C, c = k - kk * C;
-        const int kh = kk / KW, kw = kk - kh * KW;
-        return __ldg(reinterpret_cast<const uint4*>(r.p + ((size_t)kh * W + kw) * C + c));
-    }
-};
-struct LoadConv1FromRing {           // conv1 straight from the u8 frame ring: K order (slot, kw, kh), kh fastest = 8 bytes of a frame row
-    const uint8_t* frames; const uint32_t* slot_frame;   // slot_frame[item][4]: frame number in the ring of ring-slot h, ~0u = all zero
-    struct Row { uint32_t b, off; };
-    __device__ __forceinline__ Row prepare(uint32_t row) const {
-        const uint32_t b = row / 400u, pos = row - b * 400u;
-        const uint32_t ox = pos / 20u, oy = pos - ox * 20u;            // output pixel (x, y): reference tensor layout is [x][y][slot]
-        return Row{b, 4u * oy * FRAME_W + 4u * ox};
-    }
-    __device__ __forceinline__ uint4 load8(const Row& r, uint32_t kchunk) const {
-        const uint32_t h = kchunk >> 3, kw = kchunk & 7u;              // ring slot, y offset
-        const uint32_t fi = __ldg(slot_frame + r.b * 4u + h);
-        if (fi == 0xFFFFFFFFu) return make_uint4(0u, 0u, 0u, 0u);      // slot not written yet in this episode
-        const uint8_t* f = frames + (size_t)fi * FRAME_BYTES + r.off + kw * FRAME_W;
-        const uint32_t lo = __ldg(reinterpret_cast<const uint32_t*>(f)), hi = __ldg(reinterpret_cast<const uint32_t*>(f + 4));
-        uint4 o;
-        o.x = pack_bf16((float)(lo & 0xFFu), (float)((lo >> 8) & 0xFFu));  o.y = pack_bf16((float)((lo >> 16) & 0xFFu), (float)(lo >> 24));
-        o.z = pack_bf16((float)(hi & 0xFFu), (float)((hi >> 8) & 0xFFu));  o.w = pack_bf16((float)((hi >> 16) & 0xFFu), (float)(hi >> 24));
-        return o;
-    }
-};
-
 // which frame of the ring holds ring-slot h of item b's state (obs mode: indices == NULL, item = env at the current time;
 // replay mode: logical transition index, which = 0 state / 1 next) — same rules as the gather kernels (locate()).
 __global__ void qnet_locate_kernel(GatherParams g, uint32_t which, uint32_t* slot_frame) {
@@ -132,20 +95,7 @@ __global__ void qnet_locate_kernel(GatherParams g, uint32_t which, uint32_t* slo
     reinterpret_cast<uint4*>(slot_frame)[b] = slot_frames(g, b, which);
 }
 
-// weight preparation: Keras layouts (f32) -> bf16 [N][K] K-major in the K order each loader uses
-__global__ void prep_conv1_kernel(const float* __restrict__ kernel /*[8][8][4][32] = [kh(x)][kw(y)][slot][cout]*/, __nv_bfloat16* __restrict__ w /*[32][256]*/) {
-    const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= 32 * 256) return;
-    const int co = i / 256, k = i % 256;
-    const int s = k / 64, kw = (k / 8) % 8, kh = k % 8;
-    w[i] = __float2bfloat16_rn(kernel[((kh * 8 + kw) * 4 + s) * 32 + co]);
-}
-__global__ void prep_transpose_kernel(const float* __restrict__ kernel /*[K][N]*/, __nv_bfloat16* __restrict__ w /*[N][K]*/, int K, int N) {
-    const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= K * N) return;
-    const int n = i / K, k = i % K;
-    w[i] = __float2bfloat16_rn(kernel[(size_t)k * N + n]);
-}
+// the head weights of the dense epilogue: Keras [512][3] -> [3][512] f32
 __global__ void prep_head_kernel(const float* __restrict__ kernel /*[512][3]*/, float* __restrict__ w /*[3][512]*/) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= 3 * 512) return;
@@ -180,7 +130,7 @@ struct EpiF32 {                      // out f32 [gridDim.z][m_total][n_total]: t
 };
 
 // Split K: blockIdx.z selects a K slice. W holds the slices back to back ([gridDim.z][N_TOTAL][k_total]); the loader offsets
-// its own K by blockIdx.z (the forward runs with gridDim.z = 1).
+// its own K by blockIdx.z (the data-gradient GEMMs run with gridDim.z = 1).
 template <int NT, class Loader, class Epi>
 __global__ void __launch_bounds__(128) gemm_tc_kernel(Loader ld, const __nv_bfloat16* __restrict__ w, Epi epi, uint32_t m_total, uint32_t k_total,
                                                      uint32_t n_total, unsigned int* err_flag) {
@@ -281,25 +231,6 @@ __global__ void __launch_bounds__(128) gemm_tc_kernel(Loader ld, const __nv_bflo
         }
     }
     if (warp == 0) tmem_dealloc(tmem_base, TMEM_COLS);
-}
-
-// Dense 512 -> 3 + argmax (tiny: CUDA cores). act bf16 [M][512], w f32 [3][512]; q f32 [M][3]; action u8 [M]
-__global__ void head_kernel(const __nv_bfloat16* __restrict__ act, const float* __restrict__ w, const float* __restrict__ bias, float* __restrict__ q,
-                            uint8_t* __restrict__ action, float* __restrict__ max_q, uint32_t m_total) {
-    const uint32_t row = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5), lane = threadIdx.x & 31u;
-    if (row >= m_total) return;
-    float s0 = 0.0f, s1 = 0.0f, s2 = 0.0f;
-    for (int k = lane; k < 512; k += 32) {
-        const float a = __bfloat162float(act[(size_t)row * 512 + k]);
-        s0 += a * w[k]; s1 += a * w[512 + k]; s2 += a * w[1024 + k];
-    }
-    for (int o = 16; o; o >>= 1) { s0 += __shfl_down_sync(~0u, s0, o); s1 += __shfl_down_sync(~0u, s1, o); s2 += __shfl_down_sync(~0u, s2, o); }
-    if (lane == 0) {
-        s0 += bias[0]; s1 += bias[1]; s2 += bias[2];
-        if (q) { q[(size_t)row * 3] = s0; q[(size_t)row * 3 + 1] = s1; q[(size_t)row * 3 + 2] = s2; }
-        if (action) action[row] = (uint8_t)(s1 > s0 ? (s2 > s1 ? 2 : 1) : (s2 > s0 ? 2 : 0));     // first maximum, like tf.argmax
-        if (max_q) max_q[row] = fmaxf(s0, fmaxf(s1, s2));                                          // tf.reduce_max
-    }
 }
 
 __global__ void f32_to_bf16_kernel(const float* __restrict__ in, __nv_bfloat16* __restrict__ out, size_t n) {

@@ -111,12 +111,6 @@ __host__ __device__ __forceinline__ size_t plane_elem_offset(uint32_t item, uint
 }
 
 // ---- epilogue targets: where the bf16 outputs of pixel (ox, oy) of an item go ---------------------------------
-struct OutXYC {                      // [item][ox][oy][c]: the Keras tensor order (H = x), used for Flatten -> Dense and by the plain GEMM loaders
-    __nv_bfloat16* out; int ow, oh, n;
-    __device__ __forceinline__ void store8(uint32_t item, uint32_t ox, uint32_t oy, uint32_t c0, uint4 v) const {
-        *reinterpret_cast<uint4*>(out + (((size_t)item * ow + ox) * oh + oy) * n + c0) = v;
-    }
-};
 struct OutConv2Planes {              // conv1 -> conv2 input: space-to-depth by 2, channel = (oy&1, ox&1, c), row = (oy/2)*10 + ox/2
     __nv_bfloat16* out;
     __device__ __forceinline__ void store8(uint32_t item, uint32_t ox, uint32_t oy, uint32_t c0, uint4 v) const {
@@ -548,7 +542,7 @@ __global__ void prep_dense_planes_kernel(const float* __restrict__ kernel, __nv_
     w[i] = __float2bfloat16_rn(kernel[(size_t)(j * 8 + e) * 512 + tile * NT + nt]);
 }
 
-// Dense 512 -> 3 + argmax, one warp per row with 16-byte loads (replaces head_kernel's 2-byte loads)
+// Dense 512 -> 3 + argmax over bf16 activations [M][512], one warp per row with 16-byte loads
 __global__ void __launch_bounds__(256) head_vec_kernel(const __nv_bfloat16* __restrict__ act, const float* __restrict__ w /*[3][512]*/, const float* __restrict__ bias,
                                                        float* __restrict__ q, uint8_t* __restrict__ action, float* __restrict__ max_q, uint32_t m_total) {
     __shared__ float sw[3 * 512];
