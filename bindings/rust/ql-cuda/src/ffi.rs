@@ -88,6 +88,12 @@ pub struct qlc_qnet {
     _private: [u8; 0],
 }
 
+/// proportional prioritized replay: a sum tree over an env's replay ring
+#[repr(C)]
+pub struct qlc_per {
+    _private: [u8; 0],
+}
+
 /// host f32 arrays in the Keras layouts
 #[repr(C)]
 pub struct qlc_qnet_weights {
@@ -196,5 +202,15 @@ extern "C" {
     pub fn qlc_qnet_train_host(qnet: *mut qlc_qnet, idx_host: *const u32, batch: u32, n_batches: u32, target_host: *const f32, target_net: *mut qlc_qnet,
                                gamma: f32, loss_host: *mut f32) -> i32;
     pub fn qlc_qnet_debug_grads(qnet: *mut qlc_qnet, idx_host: *const u32, n: u32, target_host: *const f32, grads_out_host: *const qlc_qnet_weights) -> i32;
+    pub fn qlc_qnet_train_weighted(qnet: *mut qlc_qnet, idx_dev: *const u32, weight_dev: *const f32, batch: u32, n_batches: u32, target_dev: *const f32,
+                                   target_net: *mut qlc_qnet, gamma: f32, loss_dev: *mut f32, td_dev: *mut f32, stream: *mut c_void) -> i32;
+    pub fn qlc_qnet_debug_grads_weighted(qnet: *mut qlc_qnet, idx_host: *const u32, n: u32, target_host: *const f32, weight_host: *const f32,
+                                         grads_out_host: *const qlc_qnet_weights, td_out_host: *mut f32) -> i32;
+    pub fn qlc_per_create(env: *mut qlc_env, alpha: f32, epsilon: f32, out: *mut *mut qlc_per) -> i32;
+    pub fn qlc_per_destroy(per: *mut qlc_per) -> i32;
+    pub fn qlc_per_sample(per: *mut qlc_per, batch: u32, n_batches: u32, call_index: u64, beta: f32, idx_dev: *mut u32, weight_dev: *mut f32,
+                          stream: *mut c_void) -> i32;
+    pub fn qlc_per_update(per: *mut qlc_per, idx_dev: *const u32, td_dev: *const f32, n: u32, stream: *mut c_void) -> i32;
+    pub fn qlc_per_read_host(per: *mut qlc_per, leaves_host: *mut f32, total_host: *mut f64, max_priority_host: *mut f32) -> i32;
     pub fn qlc_debug_gemm_bf16(a_host: *const f32, w_host: *const f32, bias_host: *const f32, relu: i32, out_host: *mut f32, m: u32, n: u32, k: u32) -> i32;
 }

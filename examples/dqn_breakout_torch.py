@@ -70,14 +70,19 @@ class TorchDQNModel:
 
 
 def run(n_envs=1024, iterations=200, batch=32, minibatches_per_call=None, seed=0, device=0, quiet=False, tensor_core_actor=False, actor_sync_every=10,
-        env_id_base=0, skip_model=False, random_phase_steps=None, tensor_core_learner=False, target_sync_every=250):
+        env_id_base=0, skip_model=False, random_phase_steps=None, tensor_core_learner=False, target_sync_every=250, prioritized=False):
     """Device-resident variant of learner.SelfDrivingQLearner.learn_iteration: same rules, tensors never leave the GPU.
     skip_model: run the data path only (step, replay insert, sample + gather, TD-target inputs) without the network calls —
     what is left of an iteration when the learner costs nothing (bench.py uses it to attribute the iteration time).
     tensor_core_learner: the whole model on the library (torch_io.TensorCoreLearner): greedy actions and training on the
     tcgen05 Q-network; minibatches are drawn by qlc_replay_sample into an index tensor (no gather, no state tensor) and
     trained by qlc_qnet_train (one update per call on all of them, like the torch path) with the TD target from the target
-    network, which follows every `target_sync_every` iterations."""
+    network, which follows every `target_sync_every` iterations.
+    prioritized (with tensor_core_learner): proportional prioritized replay (alpha 0.6) instead of uniform minibatches — one
+    stratified minibatch of the same nb * batch items per iteration, importance weights with beta annealed linearly from 0.4 to
+    1.0 over the run, priorities updated from the TD errors of the update."""
+    if prioritized and not tensor_core_learner:
+        raise ValueError("prioritized replay runs on the tensor-core learner (tensor_core_learner=True)")
     dev = torch.device("cuda", device)
     torch.cuda.set_device(dev)
     p = L.Parameter(history_buffer_len=n_envs * 128, epsilon_pure_random_steps=n_envs * 20 if random_phase_steps is None else random_phase_steps,
@@ -87,7 +92,8 @@ def run(n_envs=1024, iterations=200, batch=32, minibatches_per_call=None, seed=0
     rb = q.ReplayBuffer(env)
     model, target = TorchDQNModel(dev), TorchDQNModel(dev)
     target.load_from(model)
-    learner = tio.TensorCoreLearner(env, tio.keras_weights_from_torch(model.net), gamma=p.gamma.item()) if tensor_core_learner else None
+    learner = tio.TensorCoreLearner(env, tio.keras_weights_from_torch(model.net), gamma=p.gamma.item(), per_alpha=0.6 if prioritized else None) \
+        if tensor_core_learner else None
     # optional: action selection on the library's tcgen05 Q-network, reading the frame ring directly (no f32 observation
     # is materialised); its weights follow the torch model every `actor_sync_every` iterations
     actor = tio.TensorCoreActor(env, model.net) if tensor_core_actor else None
@@ -126,6 +132,11 @@ def run(n_envs=1024, iterations=200, batch=32, minibatches_per_call=None, seed=0
         step_count += n_envs
         if rb.len() > batch:
             for _ in range(max(1, due_per_iter // nb)):
+                if prioritized:
+                    if not skip_model:
+                        learner.train_prioritized(nb * batch, 1, calls, 0.4 + 0.6 * it / max(1, iterations - 1))
+                    calls += nb
+                    continue
                 if learner is not None:
                     rb.sample_device(batch, nb, calls, idx.data_ptr(), tio._stream()); calls += nb
                     if not skip_model:
@@ -158,6 +169,9 @@ def run(n_envs=1024, iterations=200, batch=32, minibatches_per_call=None, seed=0
     if learner is not None:
         out["losses_finite"] = bool(all(torch.isfinite(x).all() for x in learner.losses))
         out["qnet_error"] = learner.error()
+        if learner.per is not None:
+            out["per_leaves"], out["per_total"], out["per_max"] = learner.per.read()      # logical order; the ring is at env.time()
+            out["env_time"] = env.time()
         learner.close()
     if actor is not None:
         actor.close()
@@ -173,5 +187,9 @@ if __name__ == "__main__":
     ap.add_argument("--tensor-core-learner", action="store_true", help="the whole model on the library: greedy actions and training (qlc_qnet_train) "
                     "on its tcgen05 Q-network, minibatches sampled as indices only")
     ap.add_argument("--tensor-core-actor", action="store_true", help="greedy actions from the library's tcgen05 Q-network (weights synced from the torch model)")
+    ap.add_argument("--prioritized", action="store_true", help="with --tensor-core-learner: proportional prioritized replay (alpha 0.6, beta 0.4 -> 1.0)")
     args = ap.parse_args()
-    print(run(args.envs, args.iterations, args.batch, tensor_core_actor=args.tensor_core_actor, tensor_core_learner=args.tensor_core_learner))
+    if args.prioritized and not args.tensor_core_learner:
+        ap.error("--prioritized needs --tensor-core-learner")
+    print(run(args.envs, args.iterations, args.batch, tensor_core_actor=args.tensor_core_actor, tensor_core_learner=args.tensor_core_learner,
+              prioritized=args.prioritized))

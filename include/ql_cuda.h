@@ -275,6 +275,38 @@ int32_t qlc_qnet_train_host(qlc_qnet* qnet, const uint32_t* idx_host, uint32_t b
                             float gamma, float* loss_host);
 /* forward + backward only, for tests: the unclipped f32 gradients of the loss over n transitions with targets target_host [n] */
 int32_t qlc_qnet_debug_grads(qlc_qnet* qnet, const uint32_t* idx_host, uint32_t n, const float* target_host, const qlc_qnet_weights* grads_out_host);
+/* qlc_qnet_train with per-item loss weights: minibatch loss = mean of w * Huber(Q(s)[a] - y). weight_dev [n_batches][batch] (NULL = 1:
+ * exactly qlc_qnet_train's arithmetic); td_dev [n_batches][batch] out (NULL = not written) gets Q(s)[a] - y from the forward that
+ * precedes each item's own update - what qlc_per_update takes. */
+int32_t qlc_qnet_train_weighted(qlc_qnet* qnet, const uint32_t* idx_dev, const float* weight_dev, uint32_t batch, uint32_t n_batches,
+                                const float* target_dev, qlc_qnet* target_net, float gamma, float* loss_dev, float* td_dev, void* stream);
+/* test hook, like qlc_qnet_debug_grads: unclipped gradients of the weighted loss (weight_host NULL = 1), and the TD errors
+ * td_out_host [n] (may be NULL) */
+int32_t qlc_qnet_debug_grads_weighted(qlc_qnet* qnet, const uint32_t* idx_host, uint32_t n, const float* target_host,
+                                      const float* weight_host, const qlc_qnet_weights* grads_out_host, float* td_out_host);
+
+/* ---- proportional prioritized replay (Schaul et al., ICLR 2016) on the device: a sum tree over the replay ring (DESIGN.md §13).
+ * Priorities p = (|delta| + epsilon)^alpha, one per transition; a transition enters the replay at the running maximum priority
+ * (which starts at 1.0 and never decreases). The tree follows the ring lazily: every call first catches up with the steps taken
+ * since the previous one, so qlc_env_step is unchanged and nothing is read back to the host. Sample, train and update must see
+ * the same env time: a step in between shifts the logical indices (as it does between qlc_replay_sample and qlc_qnet_train).
+ * Priorities are not part of qlc_env_save checkpoints; after qlc_env_load every transition restarts at the running maximum.
+ * Deterministic: the same calls give the same indices, weights and tree bits. ---- */
+typedef struct qlc_per qlc_per;
+/* 0 <= alpha <= 1, epsilon > 0 (finite); the env's replay_capacity > 0 */
+int32_t qlc_per_create(qlc_env* env, float alpha, float epsilon, qlc_per** out);
+/* valid before or after qlc_env_destroy; afterwards every other call fails */
+int32_t qlc_per_destroy(qlc_per* per);
+/* n_batches stratified minibatches drawn with replacement, P(i) = p_i / total: idx_dev [n_batches][batch] u32 logical indices
+ * (0 = oldest), weight_dev [n_batches][batch] f32 importance weights (p_min / p_i)^beta, p_min the smallest priority in the item's
+ * minibatch (may be NULL); 0 <= beta <= 1. Minibatch m uses the Philox stream (seed, call_index + m, 'PRIO'). Asynchronous. */
+int32_t qlc_per_sample(qlc_per* per, uint32_t batch, uint32_t n_batches, uint64_t call_index, float beta,
+                       uint32_t* idx_dev, float* weight_dev, void* stream);
+/* priorities of n transitions from their TD errors td_dev [n]: an index given twice keeps its largest priority, indices >= len
+ * are ignored, a non-finite delta gives the running maximum. Asynchronous. */
+int32_t qlc_per_update(qlc_per* per, const uint32_t* idx_dev, const float* td_dev, uint32_t n, void* stream);
+/* synchronous; leaves_host [len] in logical order (may be NULL), total = root, max = running max priority (either may be NULL) */
+int32_t qlc_per_read_host(qlc_per* per, float* leaves_host, double* total_host, float* max_priority_host);
 
 /* ---- checkpoint / resume of the env shard + replay ring (the reference checkpoints only the model:
  * q_learning_model.rs:191-202). qlc_env_load needs an env created with the same n_envs / env_id_base / seed /

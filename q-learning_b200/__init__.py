@@ -53,6 +53,8 @@ ABI_SYMBOLS = [
     "qlc_debug_collision_wall", "qlc_debug_collision_rect", "qlc_debug_collision_rect_batch", "qlc_debug_gemm_bf16",
     "qlc_qnet_create", "qlc_qnet_set_weights", "qlc_qnet_destroy", "qlc_qnet_error", "qlc_qnet_forward", "qlc_qnet_forward_host",
     "qlc_qnet_set_adam", "qlc_qnet_get_weights", "qlc_qnet_train", "qlc_qnet_train_host", "qlc_qnet_debug_grads",
+    "qlc_qnet_train_weighted", "qlc_qnet_debug_grads_weighted",
+    "qlc_per_create", "qlc_per_destroy", "qlc_per_sample", "qlc_per_update", "qlc_per_read_host",
 ]
 
 
@@ -194,6 +196,13 @@ def load_library(build_if_missing=True):
         "qlc_qnet_train": (i32, [vp, vp, u32, u32, vp, vp, C.c_float, vp, vp]),
         "qlc_qnet_train_host": (i32, [vp, vp, u32, u32, vp, vp, C.c_float, vp]),
         "qlc_qnet_debug_grads": (i32, [vp, vp, u32, vp, C.POINTER(QlcQnetWeights)]),
+        "qlc_qnet_train_weighted": (i32, [vp, vp, vp, u32, u32, vp, vp, C.c_float, vp, vp, vp]),
+        "qlc_qnet_debug_grads_weighted": (i32, [vp, vp, u32, vp, vp, C.POINTER(QlcQnetWeights), vp]),
+        "qlc_per_create": (i32, [vp, C.c_float, C.c_float, C.POINTER(vp)]),
+        "qlc_per_destroy": (i32, [vp]),
+        "qlc_per_sample": (i32, [vp, u32, u32, u64, C.c_float, vp, vp, vp]),
+        "qlc_per_update": (i32, [vp, vp, vp, u32, vp]),
+        "qlc_per_read_host": (i32, [vp, vp, C.POINTER(C.c_double), C.POINTER(C.c_float)]),
     }
     for name, (res, args) in sig.items():
         f = getattr(L, name)   # AttributeError if the library lacks a declared symbol
@@ -784,3 +793,66 @@ class QNetwork:
         w, _ = self._pack(out)
         _check(self._L.qlc_qnet_debug_grads(self._h, _np_ptr(idx), idx.size, _np_ptr(tgt), C.byref(w)))
         return out
+
+    def train_weighted_device(self, idx_ptr, weight_ptr, batch, n_batches, target_ptr=None, target_net=None, gamma=0.99, loss_ptr=None, td_ptr=None,
+                              stream=None):
+        """train_device with per-item loss weights (weight_ptr None = 1: train_device's arithmetic) and, if td_ptr is given, the
+        TD errors Q(s)[a] - y of every item written there (what PrioritizedReplay.update_device takes)."""
+        _check(self._L.qlc_qnet_train_weighted(self._h, idx_ptr, weight_ptr, batch, n_batches, target_ptr, None if target_net is None else target_net._h,
+                                               gamma, loss_ptr, td_ptr, stream))
+
+    def debug_grads_weighted(self, indices, targets, weights):
+        """Forward + backward only of the loss mean(w * Huber): (gradients in the Keras layouts, TD errors f32 [n])."""
+        idx = np.ascontiguousarray(indices, dtype=np.uint32).ravel()
+        tgt = np.ascontiguousarray(targets, dtype=np.float32).ravel()
+        wt = np.ascontiguousarray(weights, dtype=np.float32).ravel()
+        if tgt.size != idx.size or wt.size != idx.size:
+            raise QlError("targets and weights must have one value per index")
+        out = {name: np.empty(shape, dtype=np.float32) for name, shape in QNET_SHAPES.items()}
+        w, _ = self._pack(out)
+        td = np.empty(idx.size, dtype=np.float32)
+        _check(self._L.qlc_qnet_debug_grads_weighted(self._h, _np_ptr(idx), idx.size, _np_ptr(tgt), _np_ptr(wt), C.byref(w), _np_ptr(td)))
+        return out, td
+
+
+class PrioritizedReplay:
+    """Proportional prioritized replay (Schaul et al., ICLR 2016) over the replay ring of a BreakoutEnvironment: a sum tree on the
+    device, p = (|delta| + epsilon)^alpha, new transitions at the running maximum priority. Sampling is stratified with
+    replacement and returns logical replay indices (the ones QNetwork.train_device takes) and importance weights."""
+
+    def __init__(self, env, alpha=0.6, epsilon=1e-6):
+        self._env = env
+        self._L = env._L
+        self.alpha, self.epsilon = float(alpha), float(epsilon)
+        h = C.c_void_p()
+        _check(self._L.qlc_per_create(env._h, self.alpha, self.epsilon, C.byref(h)))
+        self._h = h
+
+    def close(self):
+        if getattr(self, "_h", None):
+            self._L.qlc_per_destroy(self._h)
+            self._h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def sample_device(self, batch, n_batches, call_index, beta, idx_ptr, weight_ptr=None, stream=None):
+        """n_batches minibatches of `batch` indices (u32 [n_batches][batch] at idx_ptr) and weights (f32, weight_ptr may be None).
+        Asynchronous on `stream`."""
+        _check(self._L.qlc_per_sample(self._h, batch, n_batches, call_index, beta, idx_ptr, weight_ptr, stream))
+
+    def update_device(self, idx_ptr, td_ptr, n, stream=None):
+        """New priorities of the n transitions idx_ptr (u32) from their TD errors td_ptr (f32). Asynchronous on `stream`."""
+        _check(self._L.qlc_per_update(self._h, idx_ptr, td_ptr, n, stream))
+
+    def read(self):
+        """(leaves f32 [len] in logical order, total f64 = the root, running max priority f32); synchronises."""
+        n = C.c_uint64(0)
+        _check(self._L.qlc_replay_len(self._env._h, C.byref(n)))
+        leaves = np.empty(n.value, dtype=np.float32)
+        total, mx = C.c_double(0), C.c_float(0)
+        _check(self._L.qlc_per_read_host(self._h, _np_ptr(leaves) if leaves.size else None, C.byref(total), C.byref(mx)))
+        return leaves, total.value, mx.value

@@ -18,6 +18,7 @@ HEADERS = [
     os.path.join(_HERE, "csrc", "qnet.cuh"),
     os.path.join(_HERE, "csrc", "qnet_conv.cuh"),
     os.path.join(_HERE, "csrc", "qnet_train.cuh"),
+    os.path.join(_HERE, "csrc", "per.cuh"),
     os.path.join(_HERE, "csrc", "host_pool.h"),
     os.path.join(_HERE, "csrc", "comm.h"),
     os.path.join(os.path.dirname(_HERE), "include", "ql_cuda.h"),

@@ -330,7 +330,7 @@ __device__ __forceinline__ void time_step(Env& e, uint32_t action, MoveCache& mc
 }
 
 // ---- Philox-4x32-10 (Salmon et al., SC'11) and the random inputs derived from it ----
-constexpr uint32_t STREAM_RESET = 0x52455345u, STREAM_SAMPLE = 0x53414D50u, STREAM_ACTION = 0x41435449u;
+constexpr uint32_t STREAM_RESET = 0x52455345u, STREAM_SAMPLE = 0x53414D50u, STREAM_ACTION = 0x41435449u, STREAM_PRIORITY = 0x5052494Fu;
 
 __device__ __forceinline__ uint4 philox4x32_10(uint4 c, uint2 k) {
     #pragma unroll

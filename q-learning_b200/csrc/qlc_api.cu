@@ -5,6 +5,7 @@
 #include "qnet.cuh"
 #include "qnet_conv.cuh"
 #include "qnet_train.cuh"
+#include "per.cuh"
 #include "host_pool.h"
 #include "comm.h"
 
@@ -89,6 +90,8 @@ struct qlc_env {
     int persistent = 1;                        // QLC_PERSISTENT=0: one CTA per env batch
     std::vector<void*> allocs;
     std::vector<struct qlc_qnet*> qnets;       // Q-networks created on this env: invalidated (not dangling) when the env goes first
+    std::vector<struct qlc_per*> pers;         // prioritized-replay trees over this env's ring: the same
+    uint64_t generation = 0;                   // raised by qlc_env_load: the ring's contents were replaced (the trees rebuild)
     // episode-statistics reduction over the env shards (qlc_comm_init / qlc_stats_allreduce): NCCL on a side stream, off the step path
     struct Comm {
         qlc_comm::Comm nccl = nullptr; int rank = 0, world = 1;
@@ -106,6 +109,7 @@ struct qlc_env {
     }* comm = nullptr;
 };
 static void qnet_release_device(struct qlc_qnet* q);
+static void per_release_device(struct qlc_per* p);
 
 static int32_t ensure_pin(qlc_env* env, size_t bytes) {
     if (bytes <= env->pin_bytes) return QLC_OK;
@@ -263,6 +267,7 @@ int32_t qlc_env_destroy(qlc_env* env) {
 #endif
     qlc_comm_destroy(env);
     for (struct qlc_qnet* q : env->qnets) qnet_release_device(q);      // their handles stay valid for qlc_qnet_destroy, every other call fails
+    for (struct qlc_per* p : env->pers) per_release_device(p);         // likewise for qlc_per_destroy
     for (void* p : env->allocs) cudaFree(p);
     if (env->pin) cudaFreeHost(env->pin);
     if (env->dev_stage) cudaFree(env->dev_stage);
@@ -1256,6 +1261,7 @@ int32_t qlc_env_load(qlc_env* env, const char* path) {
         }
     }
     fclose(f);
+    ++env->generation;                               // the ring may have been (partly) overwritten, whether or not the load succeeds
     if (ok) ok = cudaMemcpy(env->stats, &h.stats, sizeof h.stats, cudaMemcpyHostToDevice) == cudaSuccess;
     if (!ok) return fail(QLC_ERR_CUDA, std::string("reading checkpoint failed (the env state is now undefined): ") + path);
     env->t = h.t; env->window = window;
@@ -1705,9 +1711,10 @@ static cudaError_t launch_wgrad(qlc_qnet* q, const WGradShape& w, Loader ld, con
     return launch_pdl(qnet::reduce_splits_kernel, dim3(std::min<uint32_t>((mn + 255) / 256, 2048)), dim3(256), 0, s, (const float*)q->t_split, sk.splits, mn, out);
 }
 
-// forward + backward of one minibatch (idx_dev [b], targets y_dev [b]) into q->grad; loss_dev (optional) gets the mean Huber
-// loss; apply: clip + Adam + operand copies of the new weights
-static int32_t qnet_train_step(qlc_qnet* q, const uint32_t* idx_dev, uint32_t b, const float* y_dev, float* loss_dev, bool apply, cudaStream_t s) {
+// forward + backward of one minibatch (idx_dev [b], targets y_dev [b], loss weights w_dev [b] or NULL = 1) into q->grad; loss_dev
+// (optional) gets the mean weighted Huber loss, td_dev (optional) Q(s)[a] - y; apply: clip + Adam + operand copies of the new weights
+static int32_t qnet_train_step(qlc_qnet* q, const uint32_t* idx_dev, uint32_t b, const float* y_dev, const float* w_dev, float* loss_dev, float* td_dev,
+                               bool apply, cudaStream_t s) {
     using namespace qnet;
     qlc_env* env = q->env;
     int32_t rc = qnet_train_alloc(q, b); if (rc) return rc;
@@ -1721,8 +1728,8 @@ static int32_t qnet_train_step(qlc_qnet* q, const uint32_t* idx_dev, uint32_t b,
     cudaError_t e = cudaSuccess;
     auto ok = [&](cudaError_t x) { if (e == cudaSuccess) e = x; return e == cudaSuccess; };
     // head: dQ, loss, dH (masked), dW5, db5, db4
-    ok(launch_pdl(head_backward_kernel, dim3((b + 7) / 8), dim3(256), 0, s, gp, (const float*)q->t_q, y_dev, (const __nv_bfloat16*)q->a4, (const float*)(q->master + var_offset(8)),
-                  q->t_dq, q->t_loss, q->t_dh, q->t_dh_bf));
+    ok(launch_pdl(head_backward_kernel, dim3((b + 7) / 8), dim3(256), 0, s, gp, (const float*)q->t_q, y_dev, w_dev, (const __nv_bfloat16*)q->a4,
+                  (const float*)(q->master + var_offset(8)), q->t_dq, q->t_loss, q->t_dh, q->t_dh_bf, td_dev));
     {
         const uint32_t rps = colsum_rows_per_split(b), splits = (b + rps - 1) / rps;
         ok(launch_pdl(head_wgrad_partial_kernel, dim3(16, splits), dim3(32, 8), 0, s, (const __nv_bfloat16*)q->a4, (const float*)q->t_dq, b, rps, q->t_colsum));
@@ -1778,9 +1785,9 @@ static int32_t check_train_args(qlc_qnet* q, const void* idx, uint32_t batch, ui
     return QLC_OK;
 }
 
-int32_t qlc_qnet_train(qlc_qnet* q, const uint32_t* idx_dev, uint32_t batch, uint32_t n_batches, const float* target_dev, qlc_qnet* target_net,
-                       float gamma, float* loss_dev, void* stream) {
-    QLC_RANGE("qlc_qnet_train");
+int32_t qlc_qnet_train_weighted(qlc_qnet* q, const uint32_t* idx_dev, const float* weight_dev, uint32_t batch, uint32_t n_batches, const float* target_dev,
+                                qlc_qnet* target_net, float gamma, float* loss_dev, float* td_dev, void* stream) {
+    QLC_RANGE("qlc_qnet_train_weighted");
     int32_t rc = check_train_args(q, idx_dev, batch, n_batches, target_dev, target_net); if (rc) return rc;
     if (n_batches == 0) return QLC_OK;
     rc = set_device(q->env); if (rc) return rc;
@@ -1804,24 +1811,35 @@ int32_t qlc_qnet_train(qlc_qnet* q, const uint32_t* idx_dev, uint32_t batch, uin
         y = q->t_y;
     }
     for (uint32_t j = 0; j < n_batches; ++j) {
-        rc = qnet_train_step(q, idx_dev + (size_t)j * batch, batch, y + (size_t)j * batch, loss_dev ? loss_dev + j : nullptr, true, s);
+        const size_t o = (size_t)j * batch;
+        rc = qnet_train_step(q, idx_dev + o, batch, y + o, weight_dev ? weight_dev + o : nullptr, loss_dev ? loss_dev + j : nullptr,
+                             td_dev ? td_dev + o : nullptr, true, s);
         if (rc) return rc;
     }
     return QLC_OK;
 }
 
-// stages host indices / targets in the env's device staging buffer; checks the indices against the replay length
-static int32_t stage_train_inputs(qlc_qnet* q, const uint32_t* idx_host, uint32_t n, const float* target_host, uint32_t n_loss, uint32_t** idx_dev, float** y_dev,
-                                  float** loss_dev) {
+int32_t qlc_qnet_train(qlc_qnet* q, const uint32_t* idx_dev, uint32_t batch, uint32_t n_batches, const float* target_dev, qlc_qnet* target_net,
+                       float gamma, float* loss_dev, void* stream) {
+    return qlc_qnet_train_weighted(q, idx_dev, nullptr, batch, n_batches, target_dev, target_net, gamma, loss_dev, nullptr, stream);
+}
+
+// stages host indices / targets / loss weights (may be NULL) in the env's device staging buffer, with room for n_loss losses and
+// n TD errors; checks the indices against the replay length
+static int32_t stage_train_inputs(qlc_qnet* q, const uint32_t* idx_host, uint32_t n, const float* target_host, const float* weight_host, uint32_t n_loss,
+                                  uint32_t** idx_dev, float** y_dev, float** w_dev, float** loss_dev, float** td_dev) {
     qlc_env* env = q->env;
     const uint64_t len = replay_len(env);
     for (uint32_t i = 0; i < n; ++i) if (idx_host[i] >= len) return fail(QLC_ERR_INVALID_ARG, "replay index out of range");
-    const size_t o_y = ((size_t)n * 4 + 255) & ~(size_t)255, o_l = o_y + (((size_t)n * 4 + 255) & ~(size_t)255), total = o_l + (size_t)n_loss * 4 + 16;
+    const size_t arr = ((size_t)n * 4 + 255) & ~(size_t)255;
+    const size_t o_y = arr, o_w = 2 * arr, o_td = 3 * arr, o_l = 4 * arr, total = o_l + (size_t)n_loss * 4 + 16;
     int32_t rc = ensure_dev_stage(env, total); if (rc) return rc;
     uint8_t* dev = (uint8_t*)env->dev_stage;
     CUDA_TRY(cudaMemcpyAsync(dev, idx_host, (size_t)n * 4, cudaMemcpyHostToDevice, env->own_stream));
     if (target_host) CUDA_TRY(cudaMemcpyAsync(dev + o_y, target_host, (size_t)n * 4, cudaMemcpyHostToDevice, env->own_stream));
-    *idx_dev = (uint32_t*)dev; *y_dev = target_host ? (float*)(dev + o_y) : nullptr; *loss_dev = (float*)(dev + o_l);
+    if (weight_host) CUDA_TRY(cudaMemcpyAsync(dev + o_w, weight_host, (size_t)n * 4, cudaMemcpyHostToDevice, env->own_stream));
+    *idx_dev = (uint32_t*)dev; *y_dev = target_host ? (float*)(dev + o_y) : nullptr; *w_dev = weight_host ? (float*)(dev + o_w) : nullptr;
+    *loss_dev = (float*)(dev + o_l); *td_dev = (float*)(dev + o_td);
     return QLC_OK;
 }
 
@@ -1831,8 +1849,8 @@ int32_t qlc_qnet_train_host(qlc_qnet* q, const uint32_t* idx_host, uint32_t batc
     int32_t rc = check_train_args(q, idx_host, batch, n_batches, target_host, target_net); if (rc) return rc;
     if (n_batches == 0) return QLC_OK;
     rc = set_device(q->env); if (rc) return rc;
-    uint32_t* idx_dev; float *y_dev, *loss_dev;
-    rc = stage_train_inputs(q, idx_host, batch * n_batches, target_host, n_batches, &idx_dev, &y_dev, &loss_dev); if (rc) return rc;
+    uint32_t* idx_dev; float *y_dev, *w_dev, *loss_dev, *td_dev;
+    rc = stage_train_inputs(q, idx_host, batch * n_batches, target_host, nullptr, n_batches, &idx_dev, &y_dev, &w_dev, &loss_dev, &td_dev); if (rc) return rc;
     cudaStream_t s = q->env->own_stream;
     rc = qlc_qnet_train(q, idx_dev, batch, n_batches, y_dev, target_net, gamma, loss_host ? loss_dev : nullptr, s); if (rc) return rc;
     if (loss_host) CUDA_TRY(cudaMemcpyAsync(loss_host, loss_dev, (size_t)n_batches * 4, cudaMemcpyDeviceToHost, s));
@@ -1843,23 +1861,29 @@ int32_t qlc_qnet_train_host(qlc_qnet* q, const uint32_t* idx_host, uint32_t batc
     return QLC_OK;
 }
 
-int32_t qlc_qnet_debug_grads(qlc_qnet* q, const uint32_t* idx_host, uint32_t n, const float* target_host, const qlc_qnet_weights* grads_out) {
+int32_t qlc_qnet_debug_grads_weighted(qlc_qnet* q, const uint32_t* idx_host, uint32_t n, const float* target_host, const float* weight_host,
+                                      const qlc_qnet_weights* grads_out, float* td_out_host) {
     int32_t rc = check_train_args(q, idx_host, n, 1, target_host, nullptr); if (rc) return rc;
     if (!grads_out) return fail(QLC_ERR_INVALID_ARG, "grads_out is null");
     const float* dst[qnet::NVARS];
     weight_ptrs(grads_out, dst);
     for (int i = 0; i < qnet::NVARS; ++i) if (!dst[i]) return fail(QLC_ERR_INVALID_ARG, "a gradient pointer is null");
     rc = set_device(q->env); if (rc) return rc;
-    uint32_t* idx_dev; float *y_dev, *loss_dev;
-    rc = stage_train_inputs(q, idx_host, n, target_host, 1, &idx_dev, &y_dev, &loss_dev); if (rc) return rc;
+    uint32_t* idx_dev; float *y_dev, *w_dev, *loss_dev, *td_dev;
+    rc = stage_train_inputs(q, idx_host, n, target_host, weight_host, 1, &idx_dev, &y_dev, &w_dev, &loss_dev, &td_dev); if (rc) return rc;
     cudaStream_t s = q->env->own_stream;
-    rc = qnet_train_step(q, idx_dev, n, y_dev, nullptr, false, s); if (rc) return rc;
+    rc = qnet_train_step(q, idx_dev, n, y_dev, w_dev, nullptr, td_out_host ? td_dev : nullptr, false, s); if (rc) return rc;
     CUDA_TRY(cudaStreamSynchronize(s));
     uint32_t herr = 0;
     rc = qlc_qnet_error(q, &herr); if (rc) return rc;
     if (herr) return fail(QLC_ERR_CUDA, "qnet: an MMA completion barrier timed out");
     for (int v = 0; v < qnet::NVARS; ++v) CUDA_TRY(cudaMemcpy(const_cast<float*>(dst[v]), q->grad + qnet::var_offset(v), (size_t)qnet::var_size(v) * 4, cudaMemcpyDeviceToHost));
+    if (td_out_host) CUDA_TRY(cudaMemcpy(td_out_host, td_dev, (size_t)n * 4, cudaMemcpyDeviceToHost));
     return QLC_OK;
+}
+
+int32_t qlc_qnet_debug_grads(qlc_qnet* q, const uint32_t* idx_host, uint32_t n, const float* target_host, const qlc_qnet_weights* grads_out) {
+    return qlc_qnet_debug_grads_weighted(q, idx_host, n, target_host, nullptr, grads_out, nullptr);
 }
 
 // test hook: out[M][N] = act(bf16(a)[M][K] * bf16(w)[N][K]^T + bias) through the tcgen05 GEMM kernel (host f32 in / out)
@@ -1907,6 +1931,189 @@ int32_t qlc_debug_collision_wall(int32_t which, float cx, float cy, float radius
 int32_t qlc_debug_collision_rect(float cx, float cy, float radius, float mvx, float mvy, float min_x, float min_y, float max_x, float max_y,
                                  int32_t* some, float* way, float* approximation, float* nx, float* ny, uint32_t* err) {
     return run_debug(3, cx, cy, radius, mvx, mvy, min_x, min_y, max_x, max_y, some, way, approximation, nx, ny, err);
+}
+
+}  // extern "C"
+
+// ---------------- prioritized replay: a sum tree over the replay ring (per.cuh, DESIGN.md §13) ----------------
+struct qlc_per {
+    qlc_env* env = nullptr;                    // NULL once the env has been destroyed: every call but destroy fails
+    int device = 0;
+    float alpha = 0.6f, epsilon = 1e-6f;
+    per::Tree tree{};
+    void* block = nullptr;                     // one allocation: leaves, node levels, running max
+    bool synced = false;                       // the leaves describe the ring at (synced_t, synced_gen)
+    uint64_t synced_t = 0, synced_gen = 0;
+};
+
+static void per_release_device(qlc_per* p) {
+    if (!p->env) return;
+    cudaSetDevice(p->device);
+    cudaDeviceSynchronize();
+    cudaFree(p->block);
+    p->block = nullptr; p->tree = per::Tree{}; p->env = nullptr;
+}
+
+static uint32_t per_grid(const qlc_env* env, uint64_t items, uint32_t threads) {
+    const uint64_t want = (items + threads - 1) / threads, most = (uint64_t)env->sm_count * 8u;
+    return (uint32_t)(want < 1 ? 1 : (want > most ? most : want));
+}
+
+// Brings the leaves up to the env's time: rows whose time entered the replay get the running max, rows whose time left it 0;
+// then their ancestors are re-summed. A load (new generation) or a jump of time_slots steps or more rewrites every row.
+static int32_t per_sync(qlc_per* p, cudaStream_t s) {
+    qlc_env* env = p->env;
+    const uint64_t t = env->t, oldest = t > env->t_cap ? t - env->t_cap : 0;
+    if (p->synced && p->synced_gen == env->generation && p->synced_t == t) return QLC_OK;
+    const uint32_t ts = env->time_slots, n_envs = env->cfg.n_envs;
+    per::Intervals slots{};
+    auto add_times = [&](uint64_t a, uint64_t b) {       // times [a, b), b - a < time_slots, as ring-slot intervals
+        if (b <= a) return;
+        const uint64_t s0 = a % ts, n = b - a;
+        if (s0 + n <= ts) { slots.lo[slots.n] = s0; slots.hi[slots.n++] = s0 + n; }
+        else { slots.lo[slots.n] = s0; slots.hi[slots.n++] = ts; slots.lo[slots.n] = 0; slots.hi[slots.n++] = s0 + n - ts; }
+    };
+    if (!p->synced || p->synced_gen != env->generation || t < p->synced_t || t - p->synced_t >= ts) {
+        slots.n = 1; slots.lo[0] = 0; slots.hi[0] = ts;
+    } else {
+        const uint64_t t0 = p->synced_t, oldest0 = t0 > env->t_cap ? t0 - env->t_cap : 0;
+        add_times(oldest0, oldest);                        // left the replay
+        add_times(t0, t);                                  // written since the last sync
+    }
+    per::Intervals iv = slots;
+    uint64_t total = 0;
+    for (uint32_t k = 0; k < iv.n; ++k) { iv.lo[k] *= n_envs; iv.hi[k] *= n_envs; total += iv.hi[k] - iv.lo[k]; }
+    CUDA_TRY(launch_pdl(per::per_sync_leaves_kernel, dim3(per_grid(env, total, 256)), dim3(256), 0, s, p->tree, iv, total, t, oldest));
+    for (uint32_t level = 1; level <= p->tree.depth; ++level) {
+        per::Intervals nv = iv;
+        total = 0;
+        for (uint32_t k = 0; k < nv.n; ++k) {
+            nv.lo[k] = iv.lo[k] >> (per::LOG_FAN * level); nv.hi[k] = ((iv.hi[k] - 1) >> (per::LOG_FAN * level)) + 1;
+            total += nv.hi[k] - nv.lo[k];
+        }
+        CUDA_TRY(launch_pdl(per::per_resum_intervals_kernel, dim3(per_grid(env, total, 256)), dim3(256), 0, s, p->tree, level, nv, total));
+    }
+    p->synced = true; p->synced_t = t; p->synced_gen = env->generation;
+    return QLC_OK;
+}
+
+extern "C" {
+
+int32_t qlc_per_create(qlc_env* env, float alpha, float epsilon, qlc_per** out) {
+    if (!(alpha >= 0.0f && alpha <= 1.0f)) return fail(QLC_ERR_INVALID_ARG, "alpha must be in [0, 1]");
+    if (!(epsilon > 0.0f) || !std::isfinite(epsilon)) return fail(QLC_ERR_INVALID_ARG, "epsilon must be finite and > 0");
+    if (!env || !out) return fail(QLC_ERR_INVALID_ARG, "env/out is null");
+    *out = nullptr;
+    int ndev = 0;                                      // before anything reads the env
+
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) return fail(QLC_ERR_NO_DEVICE, "no CUDA device: ql_cuda has no CPU fallback");
+    if (env->cfg.replay_capacity == 0) return fail(QLC_ERR_INVALID_ARG, "the env keeps no replay (replay_capacity == 0)");
+    int32_t rc = set_device(env); if (rc) return rc;
+    qlc_per* p = new qlc_per();
+    p->device = env->cfg.device; p->alpha = alpha; p->epsilon = epsilon;
+    per::Tree& t = p->tree;
+    t.n_envs = env->cfg.n_envs; t.time_slots = env->time_slots;
+    uint64_t cnt = (uint64_t)env->time_slots * env->cfg.n_envs;
+    t.count[0] = cnt;
+    while (cnt > 1 || t.depth == 0) { cnt = (cnt + per::FAN - 1) / per::FAN; t.count[++t.depth] = cnt; }
+    auto padded = [](uint64_t n, size_t elem) { return ((((n + per::FAN - 1) / per::FAN) * per::FAN * elem) + 255) & ~(size_t)255; };
+    size_t bytes = padded(t.count[0], 4);
+    for (uint32_t k = 1; k <= t.depth; ++k) bytes += padded(t.count[k], 8);
+    bytes += 256;
+    cudaError_t e = cudaMalloc(&p->block, bytes);
+    if (e == cudaSuccess) e = cudaMemset(p->block, 0, bytes);
+    if (e == cudaSuccess) {
+        uint8_t* b = (uint8_t*)p->block;
+        t.leaves = (float*)b; b += padded(t.count[0], 4);
+        for (uint32_t k = 1; k <= t.depth; ++k) { t.node[k] = (double*)b; b += padded(t.count[k], 8); }
+        t.max_bits = (unsigned int*)b;
+        const float one = 1.0f;
+        e = cudaMemcpy(t.max_bits, &one, 4, cudaMemcpyHostToDevice);
+    }
+    if (e != cudaSuccess) { cudaGetLastError(); cudaFree(p->block); delete p; return fail(QLC_ERR_CUDA, std::string("prioritized replay alloc: ") + cudaGetErrorString(e)); }
+    p->env = env;
+    env->pers.push_back(p);
+    *out = p;
+    return QLC_OK;
+}
+
+int32_t qlc_per_destroy(qlc_per* p) {
+    if (!p) return QLC_OK;
+    if (qlc_env* env = p->env) {
+        for (size_t i = 0; i < env->pers.size(); ++i)
+            if (env->pers[i] == p) { env->pers.erase(env->pers.begin() + i); break; }
+        per_release_device(p);
+    }
+    delete p;
+    return QLC_OK;
+}
+
+static int32_t check_per(qlc_per* p) {
+    if (!p) return fail(QLC_ERR_INVALID_ARG, "per is null");
+    if (!p->env) return fail(QLC_ERR_INVALID_ARG, "the environment of this prioritized replay has been destroyed");
+    return QLC_OK;
+}
+
+int32_t qlc_per_sample(qlc_per* p, uint32_t batch, uint32_t n_batches, uint64_t call_index, float beta, uint32_t* idx_dev, float* weight_dev, void* stream) {
+    QLC_RANGE("qlc_per_sample");
+    if (batch == 0) return fail(QLC_ERR_INVALID_ARG, "batch must be > 0");
+    if (!(beta >= 0.0f && beta <= 1.0f)) return fail(QLC_ERR_INVALID_ARG, "beta must be in [0, 1]");
+    if ((uint64_t)batch * n_batches > 0x3FFFFFFFull) return fail(QLC_ERR_INVALID_ARG, "too many items for one call");
+    int32_t rc = check_per(p); if (rc) return rc;
+    if (!idx_dev) return fail(QLC_ERR_INVALID_ARG, "idx is null");
+    qlc_env* env = p->env;
+    const uint64_t len = replay_len(env);
+    if (len == 0) return fail(QLC_ERR_NOT_ENOUGH, "the replay is empty");
+    if (len >= 0xFFFFFFFFull) return fail(QLC_ERR_INVALID_ARG, "replay longer than 2^32-2 transitions");
+    if (n_batches == 0) return QLC_OK;
+    rc = set_device(env); if (rc) return rc;
+    cudaStream_t s = (cudaStream_t)stream;
+    rc = per_sync(p, s); if (rc) return rc;
+    const uint32_t n = batch * n_batches;
+    const uint64_t oldest = env->t > env->t_cap ? env->t - env->t_cap : 0;
+    CUDA_TRY(launch_pdl(per::per_sample_kernel, dim3((n + 127) / 128), dim3(128), 0, s, p->tree, batch, n, call_index, env->cfg.seed, env->t, oldest,
+                        idx_dev, weight_dev));
+    if (weight_dev) CUDA_TRY(launch_pdl(per::per_weight_kernel, dim3(n_batches), dim3(256), 0, s, weight_dev, batch, beta));
+    return QLC_OK;
+}
+
+int32_t qlc_per_update(qlc_per* p, const uint32_t* idx_dev, const float* td_dev, uint32_t n, void* stream) {
+    QLC_RANGE("qlc_per_update");
+    int32_t rc = check_per(p); if (rc) return rc;
+    if (!idx_dev || !td_dev) return fail(QLC_ERR_INVALID_ARG, "idx/td is null");
+    qlc_env* env = p->env;
+    const uint64_t len = replay_len(env);
+    if (len >= 0xFFFFFFFFull) return fail(QLC_ERR_INVALID_ARG, "replay longer than 2^32-2 transitions");
+    rc = set_device(env); if (rc) return rc;
+    cudaStream_t s = (cudaStream_t)stream;
+    rc = per_sync(p, s); if (rc) return rc;
+    if (n == 0) return QLC_OK;
+    const uint64_t oldest = env->t > env->t_cap ? env->t - env->t_cap : 0;
+    const dim3 grid((n + 255) / 256);
+    CUDA_TRY(launch_pdl(per::per_update_clear_kernel, grid, dim3(256), 0, s, p->tree, idx_dev, td_dev, n, (uint32_t)len, oldest, p->alpha, p->epsilon));
+    CUDA_TRY(launch_pdl(per::per_update_set_kernel, grid, dim3(256), 0, s, p->tree, idx_dev, td_dev, n, (uint32_t)len, oldest, p->alpha, p->epsilon));
+    for (uint32_t level = 1; level <= p->tree.depth; ++level)
+        CUDA_TRY(launch_pdl(per::per_resum_items_kernel, grid, dim3(256), 0, s, p->tree, level, idx_dev, n, (uint32_t)len, oldest));
+    return QLC_OK;
+}
+
+int32_t qlc_per_read_host(qlc_per* p, float* leaves_host, double* total_host, float* max_priority_host) {
+    int32_t rc = check_per(p); if (rc) return rc;
+    qlc_env* env = p->env;
+    rc = set_device(env); if (rc) return rc;
+    CUDA_TRY(cudaDeviceSynchronize());
+    rc = per_sync(p, env->own_stream); if (rc) return rc;
+    CUDA_TRY(cudaStreamSynchronize(env->own_stream));
+    if (leaves_host) {
+        // logical order = rows of times t_oldest .. t - 1, contiguous in the ring up to one wrap
+        const uint64_t n_envs = env->cfg.n_envs, rows = replay_len(env) / n_envs, ts = env->time_slots;
+        const uint64_t s0 = (env->t > env->t_cap ? env->t - env->t_cap : 0) % ts, first = std::min(rows, ts - s0);
+        CUDA_TRY(cudaMemcpy(leaves_host, p->tree.leaves + s0 * n_envs, first * n_envs * 4, cudaMemcpyDeviceToHost));
+        if (rows > first) CUDA_TRY(cudaMemcpy(leaves_host + first * n_envs, p->tree.leaves, (rows - first) * n_envs * 4, cudaMemcpyDeviceToHost));
+    }
+    if (total_host) CUDA_TRY(cudaMemcpy(total_host, p->tree.node[p->tree.depth], 8, cudaMemcpyDeviceToHost));
+    if (max_priority_host) CUDA_TRY(cudaMemcpy(max_priority_host, p->tree.max_bits, 4, cudaMemcpyDeviceToHost));
+    return QLC_OK;
 }
 
 }  // extern "C"

@@ -201,11 +201,14 @@ __global__ void td_target_kernel(GatherParams g, const float* __restrict__ max_q
     y[i] = ((rec >> 2) & 1u) ? r : r + fut;
 }
 
-// ---- head backward (CUDA cores, one warp per item): Huber(delta 1) on Q(s)[a] averaged over the batch ----
-// dq [B][3] (only column a is non-zero), loss_i [B], dH = (dq . W5^T) masked by h > 0: f32 [B][512] and bf16 [B][512]
+// ---- head backward (CUDA cores, one warp per item): Huber(delta 1) on Q(s)[a], weighted by w [B] (NULL = 1), averaged over
+// the batch ----
+// dq [B][3] (only column a is non-zero), loss_i [B], dH = (dq . W5^T) masked by h > 0: f32 [B][512] and bf16 [B][512];
+// td [B] (optional) = Q(s)[a] - y. A weight of 1.0 multiplies exactly, so the unweighted update keeps its bits.
 __global__ void __launch_bounds__(256) head_backward_kernel(GatherParams g, const float* __restrict__ q, const float* __restrict__ y,
-                                                            const __nv_bfloat16* __restrict__ h, const float* __restrict__ w5 /*Keras [512][3]*/,
-                                                            float* __restrict__ dq, float* __restrict__ loss_i, float* __restrict__ dh, __nv_bfloat16* __restrict__ dh_bf) {
+                                                            const float* __restrict__ w, const __nv_bfloat16* __restrict__ h,
+                                                            const float* __restrict__ w5 /*Keras [512][3]*/, float* __restrict__ dq, float* __restrict__ loss_i,
+                                                            float* __restrict__ dh, __nv_bfloat16* __restrict__ dh_bf, float* __restrict__ td) {
     pdl_launch_dependents(); pdl_wait();
     const uint32_t b = blockIdx.x * 8u + (threadIdx.x >> 5), lane = threadIdx.x & 31u;
     if (b >= g.n_items) return;
@@ -214,9 +217,11 @@ __global__ void __launch_bounds__(256) head_backward_kernel(GatherParams g, cons
     const uint32_t a = rec & 3u;
     const float d = q[(size_t)b * 3 + a] - y[b];
     const float ad = fabsf(d);
-    const float g_a = fminf(fmaxf(d, -1.0f), 1.0f) / (float)g.n_items;
+    const float wb = w ? w[b] : 1.0f;
+    const float g_a = (fminf(fmaxf(d, -1.0f), 1.0f) * wb) / (float)g.n_items;
     if (lane == 0) {
-        loss_i[b] = ad <= 1.0f ? 0.5f * (d * d) : ad - 0.5f;
+        loss_i[b] = wb * (ad <= 1.0f ? 0.5f * (d * d) : ad - 0.5f);
+        if (td) td[b] = d;
         #pragma unroll
         for (uint32_t j = 0; j < 3; ++j) dq[(size_t)b * 3 + j] = j == a ? g_a : 0.0f;
     }

@@ -124,14 +124,17 @@ class TensorCoreLearner:
     `train_indices(idx)` — `n_batches` Keras-Adam updates on replay transitions by index, the TD target
     y = r + max Q_target(s') * gamma (y = r where done) computed on the device — and `sync_target()`. No state tensor is
     materialised anywhere: the kernels read the u8 frames where the step kernel wrote them. `weights`: Keras-layout f32 arrays
-    (QNET_SHAPES) for both networks."""
+    (QNET_SHAPES) for both networks. `per_alpha` (not None): prioritized replay over the same ring (PrioritizedReplay), used by
+    `train_prioritized()`."""
 
-    def __init__(self, env, weights, gamma=0.99, lr=2.5e-4, clipnorm=1.0):
-        from . import QNetwork
+    def __init__(self, env, weights, gamma=0.99, lr=2.5e-4, clipnorm=1.0, per_alpha=None, per_epsilon=1e-6):
+        from . import PrioritizedReplay, QNetwork
         self.env, self.gamma = env, float(gamma)
         self.online = QNetwork(env, weights)
         self.target = QNetwork(env, weights)
         self.online.set_adam(lr=lr, clipnorm=clipnorm)
+        self.per = None if per_alpha is None else PrioritizedReplay(env, per_alpha, per_epsilon)
+        self._per_bufs = None
         dev = torch.device("cuda", env.device)
         self.actions = torch.empty((1, env.n_envs), dtype=torch.uint8, device=dev)
         self.losses = []
@@ -152,6 +155,25 @@ class TensorCoreLearner:
         self.losses.append(loss)
         return loss
 
+    def train_prioritized(self, batch, n_batches, call_index, beta):
+        """`n_batches` updates on minibatches of `batch` transitions drawn by priority, each weighted by its importance weights
+        (exponent `beta`); the TD errors of the updates become the new priorities. Sample, train and update are queued on the
+        current stream without a host synchronisation; returns the CUDA f32 tensor [n_batches] of weighted losses."""
+        if self.per is None:
+            raise QlError("this learner was created without per_alpha")
+        dev = torch.device("cuda", self.env.device)
+        if self._per_bufs is None or self._per_bufs[0].shape != (n_batches, batch):
+            self._per_bufs = (torch.empty((n_batches, batch), dtype=torch.int32, device=dev), torch.empty((n_batches, batch), dtype=torch.float32, device=dev),
+                              torch.empty((n_batches, batch), dtype=torch.float32, device=dev))
+        idx, w, td = self._per_bufs
+        s = _stream()
+        loss = torch.empty(n_batches, dtype=torch.float32, device=dev)
+        self.per.sample_device(batch, n_batches, call_index, beta, idx.data_ptr(), w.data_ptr(), s)
+        self.online.train_weighted_device(idx.data_ptr(), w.data_ptr(), batch, n_batches, None, self.target, self.gamma, loss.data_ptr(), td.data_ptr(), s)
+        self.per.update_device(idx.data_ptr(), td.data_ptr(), batch * n_batches, s)
+        self.losses.append(loss)
+        return loss
+
     def sync_target(self):
         """target <- online (get + set of the f32 master weights)."""
         self.target.set_weights(self.online.get_weights())
@@ -169,5 +191,7 @@ class TensorCoreLearner:
         return self.online.error() | self.target.error()
 
     def close(self):
+        if self.per is not None:
+            self.per.close()
         self.online.close()
         self.target.close()
