@@ -1440,6 +1440,7 @@ int32_t qlc_qnet_error(qlc_qnet* q, uint32_t* flag) {
         // a pass that gave up may have left per-row tickets of the fused head behind: start the next one clean
         if (q->head_count) CUDA_TRY(cudaMemset(q->head_count, 0, (size_t)((q->cap_items + 127u) / 128u) * 128u * 4));
         CUDA_TRY(cudaMemset(q->err, 0, 4));
+        CUDA_TRY(cudaDeviceSynchronize());              // legacy-stream memsets: done before work on a non-blocking stream
     }
     return QLC_OK;
 }
@@ -1469,6 +1470,7 @@ static cudaError_t qnet_prep_weights(qlc_qnet* q, cudaStream_t s) {
 static int32_t qnet_reset_adam(qlc_qnet* q) {
     CUDA_TRY(cudaMemset(q->adam_m, 0, (size_t)qnet::N_PARAMS * 4));
     CUDA_TRY(cudaMemset(q->adam_v, 0, (size_t)qnet::N_PARAMS * 4));
+    CUDA_TRY(cudaDeviceSynchronize());                  // legacy-stream memsets: done before an update on a non-blocking stream
     q->adam_t = 0;
     return QLC_OK;
 }
@@ -1551,6 +1553,8 @@ static int32_t qnet_forward(qlc_qnet* q, const uint32_t* idx_dev, uint32_t n, in
     if ((uint64_t)n * 400ull >= 0xFFFFFFFFull) return fail(QLC_ERR_INVALID_ARG, "too many items for one forward pass");
     cudaStream_t s = (cudaStream_t)stream;
     if (n > q->cap_items) {
+        // the new buffers are cleared on `s`: a plain cudaMemset runs on the legacy stream, which a non-blocking stream (the
+        // env's own) does not wait for, and could then zero conv outputs and head tickets under this pass's kernels
         CUDA_TRY(cudaDeviceSynchronize());
         qnet_free_acts(q);
         CUDA_TRY(cudaMalloc(&q->a4, (size_t)n * 512 * 2)); CUDA_TRY(cudaMalloc(&q->slot_frame, (size_t)n * 16));
@@ -1558,11 +1562,11 @@ static int32_t qnet_forward(qlc_qnet* q, const uint32_t* idx_dev, uint32_t n, in
         const size_t a2p_bytes = (size_t)((n + qnet::Conv3Geom::B - 1) / qnet::Conv3Geom::B) * qnet::Conv3Geom::STAGE_BYTES;
         CUDA_TRY(cudaMalloc(&q->a1p, a1p_bytes)); CUDA_TRY(cudaMalloc(&q->a2p, a2p_bytes));
         const size_t a3p_bytes = (size_t)((n + 127) / 128) * qnet::DenseGeom::A_TILE_BYTES;
-        CUDA_TRY(cudaMalloc(&q->a3p, a3p_bytes)); CUDA_TRY(cudaMemset(q->a3p, 0, a3p_bytes));
+        CUDA_TRY(cudaMalloc(&q->a3p, a3p_bytes)); CUDA_TRY(cudaMemsetAsync(q->a3p, 0, a3p_bytes, s));
         const size_t rows_padded = (size_t)((n + 127) / 128) * 128;
         CUDA_TRY(cudaMalloc(&q->head_partial, 4 * rows_padded * sizeof(float4))); CUDA_TRY(cudaMalloc(&q->head_count, rows_padded * 4));
-        CUDA_TRY(cudaMemset(q->head_count, 0, rows_padded * 4));
-        CUDA_TRY(cudaMemset(q->a1p, 0, a1p_bytes)); CUDA_TRY(cudaMemset(q->a2p, 0, a2p_bytes));     // rows of a partial last batch are read (never used)
+        CUDA_TRY(cudaMemsetAsync(q->head_count, 0, rows_padded * 4, s));
+        CUDA_TRY(cudaMemsetAsync(q->a1p, 0, a1p_bytes, s)); CUDA_TRY(cudaMemsetAsync(q->a2p, 0, a2p_bytes, s));     // rows of a partial last batch are read (never used)
         q->cap_items = n;
     }
     GatherParams g{}; fill_gather(env, g);
