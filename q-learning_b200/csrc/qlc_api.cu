@@ -2034,6 +2034,7 @@ int32_t qlc_per_create(qlc_env* env, float alpha, float epsilon, qlc_per** out) 
         const float one = 1.0f;
         e = cudaMemcpy(t.max_bits, &one, 4, cudaMemcpyHostToDevice);
     }
+    if (e == cudaSuccess) e = cudaDeviceSynchronize();   // legacy-stream init: done before a sync or sample on a non-blocking stream
     if (e != cudaSuccess) { cudaGetLastError(); cudaFree(p->block); delete p; return fail(QLC_ERR_CUDA, std::string("prioritized replay alloc: ") + cudaGetErrorString(e)); }
     p->env = env;
     env->pers.push_back(p);
