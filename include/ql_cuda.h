@@ -5,6 +5,11 @@
  * every call returns an int32 status (QLC_OK = 0), the text of the last failure is qlc_last_error_string().
  * A handle is NOT thread-safe: one host thread and one CUDA stream per handle / per GPU
  * (the reference learner is single-threaded behind Arc<RwLock<E>>: self_driving_tf_q_learner.rs:74,171).
+ * Stream order: every call is ordered after all work that earlier calls on the same handle (or on its env, for Q-network and
+ * prioritized-replay handles) queued, whether on the caller's stream or on the library's own stream (the *_host calls, submitted
+ * host steps). So a host-buffer call after qlc_env_step on the caller's stream sees the step, and a device-pointer call after
+ * qlc_env_step_host_submit sees the submitted steps. This holds for one caller stream per handle: work on a second caller
+ * stream is not ordered by the library.
  *
  * Reference interfaces replaced (paths relative to /root/reference/src):
  *   Environment trait ................. ql/src/prelude.rs:21-63

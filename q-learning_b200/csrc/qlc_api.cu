@@ -75,6 +75,8 @@ struct qlc_env {
     uint32_t t_cap = 0;                        // replay capacity in time steps
     uint64_t t = 0;                            // env-steps taken per env (global time)
     cudaStream_t own_stream = nullptr;         // used by the *_host entry points
+    cudaEvent_t caller_done = nullptr;         // recorded after the launches of every asynchronous call; own_stream waits for it
+    bool submits_pending = false;              // submitted host steps may still be running on own_stream
     // pinned staging for the host-buffer entry points
     void* pin = nullptr; size_t pin_bytes = 0;
     std::vector<qlc_host::StreamPiece> stream_pieces;
@@ -172,6 +174,27 @@ float qlc_env_goal_mean(void) { return 59.0f; }   // (bricks.len() - 1) as f32, 
 
 static int32_t set_device(const qlc_env* env) { CUDA_TRY(cudaSetDevice(env->cfg.device)); return QLC_OK; }
 
+// Stream order (ql_cuda.h): the caller's stream and own_stream are not ordered by CUDA (own_stream is non-blocking), and the
+// device-pointer calls resolve times and indices against env->t when they are queued. So an asynchronous call first waits for
+// the newest submitted host step still in flight and ends with a record of caller_done on the caller's stream; a host-buffer
+// call first makes own_stream wait for caller_done. An event stays valid after the caller destroys its stream; a remembered
+// stream handle would not.
+}  // extern "C"
+template <class F>
+static int32_t on_caller_stream(qlc_env* env, void* stream, F&& launches) {
+    const cudaStream_t s = (cudaStream_t)stream;
+    int32_t rc = set_device(env); if (rc) return rc;
+    if (env->submits_pending) CUDA_TRY(cudaStreamWaitEvent(s, env->submit_done[(env->submit_seq - 1) % 8], 0));   // in order: older ones are done too
+    rc = launches(); if (rc) return rc;
+    CUDA_TRY(cudaEventRecord(env->caller_done, s));
+    return QLC_OK;
+}
+extern "C" {
+static int32_t after_caller_stream(qlc_env* env) {
+    CUDA_TRY(cudaStreamWaitEvent(env->own_stream, env->caller_done, 0));
+    return QLC_OK;
+}
+
 static int32_t launch_reset(qlc_env* env, const uint8_t* mask_dev, const float* dir_dev, int first_time, cudaStream_t s) {
     const uint32_t n = env->cfg.n_envs;
     env_reset_kernel<<<(n + 255) / 256, 256, 0, s>>>(env->st, n, env->cfg.env_id_base, env->cfg.seed, mask_dev, dir_dev, first_time);
@@ -238,6 +261,8 @@ int32_t qlc_env_create(const qlc_config* cfg, qlc_env** out) {
 #undef TRY_ALLOC
     cudaError_t ce = cudaStreamCreateWithFlags(&env->own_stream, cudaStreamNonBlocking);
     if (ce != cudaSuccess) { qlc_env_destroy(env); return fail(QLC_ERR_CUDA, std::string("cudaStreamCreate: ") + cudaGetErrorString(ce)); }
+    ce = cudaEventCreateWithFlags(&env->caller_done, cudaEventDisableTiming);
+    if (ce != cudaSuccess) { qlc_env_destroy(env); return fail(QLC_ERR_CUDA, std::string("cudaEventCreate: ") + cudaGetErrorString(ce)); }
     DeviceStats init{0ull, 0ull, 0xFFFFFFFFu, 0u};
     ce = cudaMemcpy(env->stats, &init, sizeof init, cudaMemcpyHostToDevice);
     if (ce != cudaSuccess) { qlc_env_destroy(env); return fail(QLC_ERR_CUDA, std::string("stats init: ") + cudaGetErrorString(ce)); }
@@ -274,6 +299,7 @@ int32_t qlc_env_destroy(qlc_env* env) {
     for (cudaEvent_t ev : env->submit_done) if (ev) cudaEventDestroy(ev);
     for (cudaEvent_t ev : env->h2d_done) if (ev) cudaEventDestroy(ev);
     for (cudaEvent_t ev : env->piece_ev) if (ev) cudaEventDestroy(ev);
+    if (env->caller_done) cudaEventDestroy(env->caller_done);
     if (env->copy_stream) cudaStreamDestroy(env->copy_stream);
     if (env->own_stream) cudaStreamDestroy(env->own_stream);
     delete env;
@@ -434,14 +460,14 @@ static int32_t step_split(qlc_env* env, const uint8_t* actions_dev, uint8_t* act
 int32_t qlc_env_step(qlc_env* env, const uint8_t* actions_dev, uint32_t n_steps, float* reward_dev, uint8_t* done_dev, void* stream) {
     QLC_RANGE("qlc_env_step");
     if (!env || !actions_dev) return fail(QLC_ERR_INVALID_ARG, "env/actions is null");
-    return step_split(env, actions_dev, nullptr, n_steps, reward_dev, done_dev, stream);
+    return on_caller_stream(env, stream, [&] { return step_split(env, actions_dev, nullptr, n_steps, reward_dev, done_dev, stream); });
 }
 
 // the learner's pure-random phase: the uniform action of every env and step is drawn inside the step kernel
 int32_t qlc_env_step_random(qlc_env* env, uint32_t n_steps, uint8_t* actions_out_dev, float* reward_dev, uint8_t* done_dev, void* stream) {
     QLC_RANGE("qlc_env_step_random");
     if (!env) return fail(QLC_ERR_INVALID_ARG, "env is null");
-    return step_split(env, nullptr, actions_out_dev, n_steps, reward_dev, done_dev, stream);
+    return on_caller_stream(env, stream, [&] { return step_split(env, nullptr, actions_out_dev, n_steps, reward_dev, done_dev, stream); });
 }
 
 static bool is_pinned(const void* p) {
@@ -460,6 +486,7 @@ static int32_t step_host_impl(qlc_env* env, const uint8_t* actions_host, uint32_
     // page-locked caller buffers (qlc_host_alloc / cudaHostRegister) are used in place; pageable ones are staged
     const bool pin_a = is_pinned(actions_host), pin_r = !reward_host || is_pinned(reward_host), pin_d = !done_host || is_pinned(done_host);
     if (!wait && !(pin_a && pin_r && pin_d)) return fail(QLC_ERR_INVALID_ARG, "qlc_env_step_host_submit needs page-locked buffers (qlc_host_alloc)");
+    rc = after_caller_stream(env); if (rc) return rc;
     // the asynchronous form keeps several steps in flight: each gets its own slice of the device staging ring
     const size_t off_r = (n + 15) & ~(size_t)15, off_d = off_r + n * 4, total = (off_d + n + 255) & ~(size_t)255;
     const uint32_t slot = wait ? 0u : (uint32_t)(env->submit_seq % 2u);
@@ -499,7 +526,7 @@ static int32_t step_host_impl(qlc_env* env, const uint8_t* actions_host, uint32_
     // page-locked outputs are written by the kernel itself (zero-copy stores over PCIe while it runs, UVA pointers);
     // pageable ones go through device staging + a device->host copy
     const bool zc_r = reward_host && pin_r && env->zero_copy, zc_d = done_host && pin_d && env->zero_copy;
-    rc = qlc_env_step(env, actions_dev, n_steps, zc_r ? reward_host : (float*)(dev + off_r), zc_d ? done_host : dev + off_d, s); if (rc) return rc;
+    rc = step_split(env, actions_dev, nullptr, n_steps, zc_r ? reward_host : (float*)(dev + off_r), zc_d ? done_host : dev + off_d, s); if (rc) return rc;
     if (reward_host && !zc_r) CUDA_TRY(cudaMemcpyAsync(pin_r ? (void*)reward_host : (void*)(pin + off_r), dev + off_r, n * 4, cudaMemcpyDeviceToHost, s));
     if (done_host && !zc_d) CUDA_TRY(cudaMemcpyAsync(pin_d ? (void*)done_host : (void*)(pin + off_d), dev + off_d, n, cudaMemcpyDeviceToHost, s));
     if (!wait) {
@@ -507,9 +534,11 @@ static int32_t step_host_impl(qlc_env* env, const uint8_t* actions_host, uint32_
         if (!ev) CUDA_TRY(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
         CUDA_TRY(cudaEventRecord(ev, s));
         ++env->submit_seq;
+        env->submits_pending = true;
         return QLC_OK;
     }
     CUDA_TRY(cudaStreamSynchronize(s));
+    env->submits_pending = false;                    // own_stream is idle: every submitted step has finished
     if (reward_host && !pin_r) memcpy(reward_host, pin + off_r, n * 4);
     if (done_host && !pin_d) memcpy(done_host, pin + off_d, n);
     return QLC_OK;
@@ -527,6 +556,7 @@ int32_t qlc_env_step_host_wait(qlc_env* env, uint32_t max_pending) {
     int32_t rc = set_device(env); if (rc) return rc;
     if (env->submit_seq <= max_pending) return QLC_OK;
     CUDA_TRY(cudaEventSynchronize(env->submit_done[(env->submit_seq - 1 - max_pending) % 8]));   // in-order stream: older submits are done too
+    if (max_pending == 0) env->submits_pending = false;
     return QLC_OK;
 }
 
@@ -616,7 +646,7 @@ int32_t qlc_env_obs(qlc_env* env, int32_t layout, void* out_dev, void* stream) {
     int32_t rc = set_device(env); if (rc) return rc;
     GatherParams g{}; fill_gather(env, g);
     g.mode = GATHER_CURRENT; g.n_items = env->cfg.n_envs; g.out_state = out_dev;
-    return launch_gather(env, g, layout, (cudaStream_t)stream);
+    return on_caller_stream(env, stream, [&] { return launch_gather(env, g, layout, (cudaStream_t)stream); });
 }
 
 // ---- state handles: what a cloned BreakoutState is on the host (state_as_rc / step_as_rc, prelude.rs:36,52-58) ----
@@ -628,7 +658,7 @@ int32_t qlc_obs_gather(qlc_env* env, const qlc_obs_handle* handles_dev, uint32_t
     static_assert(sizeof(qlc_obs_handle) == sizeof(ObsHandle), "handle layout");
     GatherParams g{}; fill_gather(env, g);
     g.mode = GATHER_HANDLES; g.handles = reinterpret_cast<const ObsHandle*>(handles_dev); g.n_items = n; g.out_state = out_dev;
-    return launch_gather(env, g, layout, (cudaStream_t)stream);
+    return on_caller_stream(env, stream, [&] { return launch_gather(env, g, layout, (cudaStream_t)stream); });
 }
 
 // a handle is usable while the frames it names are still in the ring (and it is not from the future)
@@ -718,17 +748,20 @@ static int32_t check_sample_args(qlc_env* env, uint32_t batch, uint64_t* len_out
     return QLC_OK;
 }
 
+static int32_t launch_sample(qlc_env* env, uint32_t batch, uint32_t n_batches, uint64_t len, uint64_t call_index, uint32_t* idx_dev, cudaStream_t s) {
+    if (batch >= SAMPLE_BLOCK_MIN_BATCH) replay_sample_kernel<8><<<n_batches, 256, 0, s>>>(idx_dev, batch, (uint32_t)len, env->cfg.seed, call_index);
+    else replay_sample_kernel<1><<<n_batches, 32, 0, s>>>(idx_dev, batch, (uint32_t)len, env->cfg.seed, call_index);
+    CUDA_TRY(cudaGetLastError());
+    return QLC_OK;
+}
+
 int32_t qlc_replay_sample(qlc_env* env, uint32_t batch, uint32_t n_batches, uint64_t call_index, uint32_t* idx_dev, void* stream) {
     QLC_RANGE("qlc_replay_sample");
     if (!env || !idx_dev) return fail(QLC_ERR_INVALID_ARG, "env/idx is null");
     uint64_t len = 0;
     int32_t rc = check_sample_args(env, batch, &len); if (rc) return rc;
     if (n_batches == 0) return QLC_OK;
-    rc = set_device(env); if (rc) return rc;
-    if (batch >= SAMPLE_BLOCK_MIN_BATCH) replay_sample_kernel<8><<<n_batches, 256, 0, (cudaStream_t)stream>>>(idx_dev, batch, (uint32_t)len, env->cfg.seed, call_index);
-    else replay_sample_kernel<1><<<n_batches, 32, 0, (cudaStream_t)stream>>>(idx_dev, batch, (uint32_t)len, env->cfg.seed, call_index);
-    CUDA_TRY(cudaGetLastError());
-    return QLC_OK;
+    return on_caller_stream(env, stream, [&] { return launch_sample(env, batch, n_batches, len, call_index, idx_dev, (cudaStream_t)stream); });
 }
 
 int32_t qlc_replay_gather(qlc_env* env, const uint32_t* idx_dev, uint32_t n, int32_t layout, void* state_dev, void* next_dev,
@@ -740,7 +773,7 @@ int32_t qlc_replay_gather(qlc_env* env, const uint32_t* idx_dev, uint32_t n, int
     GatherParams g{}; fill_gather(env, g);
     g.indices = idx_dev; g.n_items = n; g.out_state = state_dev; g.out_next = next_dev;
     g.reward = reward_dev; g.action = action_dev; g.done = done_dev;
-    return launch_gather(env, g, layout, (cudaStream_t)stream);
+    return on_caller_stream(env, stream, [&] { return launch_gather(env, g, layout, (cudaStream_t)stream); });
 }
 
 // sample + gather in ONE launch: every CTA of the gather kernel derives the index of its own item from the Philox stream
@@ -758,15 +791,18 @@ int32_t qlc_replay_sample_gather(qlc_env* env, uint32_t batch, uint32_t n_batche
     g.mode = GATHER_SAMPLE; g.sample_batch = batch; g.sample_len = (uint32_t)len; g.seed = env->cfg.seed; g.call0 = call_index; g.idx_out = idx_out_dev;
     g.n_items = batch * n_batches; g.out_state = state_dev; g.out_next = next_dev;
     g.reward = reward_dev; g.action = action_dev; g.done = done_dev;
-    return launch_gather(env, g, layout, (cudaStream_t)stream);
+    return on_caller_stream(env, stream, [&] { return launch_gather(env, g, layout, (cudaStream_t)stream); });
 }
 
 int32_t qlc_replay_sample_host(qlc_env* env, uint32_t batch, uint64_t call_index, uint32_t* idx_host) {
     QLC_RANGE("qlc_replay_sample_host");
     if (!env || !idx_host) return fail(QLC_ERR_INVALID_ARG, "env/idx is null");
-    int32_t rc = set_device(env); if (rc) return rc;
+    uint64_t len = 0;
+    int32_t rc = check_sample_args(env, batch, &len); if (rc) return rc;
+    rc = set_device(env); if (rc) return rc;
+    rc = after_caller_stream(env); if (rc) return rc;
     rc = ensure_dev_stage(env, (size_t)batch * 4); if (rc) return rc;
-    rc = qlc_replay_sample(env, batch, 1, call_index, (uint32_t*)env->dev_stage, env->own_stream); if (rc) return rc;
+    rc = launch_sample(env, batch, 1, len, call_index, (uint32_t*)env->dev_stage, env->own_stream); if (rc) return rc;
     CUDA_TRY(cudaMemcpyAsync(idx_host, env->dev_stage, (size_t)batch * 4, cudaMemcpyDeviceToHost, env->own_stream));
     CUDA_TRY(cudaStreamSynchronize(env->own_stream));
     return QLC_OK;
@@ -783,6 +819,7 @@ struct HostGather {
 
 static int32_t run_host_gather(qlc_env* env, HostGather& hg) {
     static const bool widen_on_host = getenv("QLC_HOST_WIDEN") ? atoi(getenv("QLC_HOST_WIDEN")) != 0 : true;
+    int32_t rc = after_caller_stream(env); if (rc) return rc;
     const uint32_t n = hg.n;
     const bool widen = hg.layout == QLC_LAYOUT_F32_BXYH && widen_on_host;
     const int32_t dev_layout = widen ? QLC_LAYOUT_U8_BXYH : hg.layout;
@@ -799,7 +836,7 @@ static int32_t run_host_gather(qlc_env* env, HostGather& hg) {
         static const bool timing = getenv("QLC_HOST_TIMING") != nullptr;
         const auto t0 = std::chrono::steady_clock::now();
         const size_t o_f = (total + 255) & ~(size_t)255, total_f = o_f + (size_t)n * 2 * 4 * sizeof(uint32_t);   // <= 4 CTAs per (item, s | s')
-        int32_t rc = ensure_pin(env, total_f); if (rc) return rc;
+        rc = ensure_pin(env, total_f); if (rc) return rc;
         uint8_t* pin = (uint8_t*)env->pin;
         cudaStream_t s = env->own_stream;
         if (hg.h2d_bytes) memcpy(pin + o_in, hg.h2d_src, hg.h2d_bytes);
@@ -872,7 +909,7 @@ static int32_t run_host_gather(qlc_env* env, HostGather& hg) {
         if (hg.idx_out_host) memcpy(hg.idx_out_host, pin + o_i, (size_t)n * 4);
         return QLC_OK;
     }
-    int32_t rc = ensure_dev_stage(env, 2 * ib * n); if (rc) return rc;
+    rc = ensure_dev_stage(env, 2 * ib * n); if (rc) return rc;
     rc = ensure_pin(env, total); if (rc) return rc;
     uint8_t* dev = (uint8_t*)env->dev_stage; uint8_t* pin = (uint8_t*)env->pin;
     uint8_t* dev_s = dev; uint8_t* dev_n = dev + ib * n;
@@ -1010,10 +1047,11 @@ int32_t qlc_stats_read(qlc_env* env, qlc_episode_stats* out) {
 }
 int32_t qlc_stats_export(qlc_env* env, double* out_dev, void* stream) {
     if (!env || !out_dev) return fail(QLC_ERR_INVALID_ARG, "env/out is null");
-    int32_t rc = set_device(env); if (rc) return rc;
-    stats_export_kernel<<<1, 1, 0, (cudaStream_t)stream>>>(env->stats, env->t * env->cfg.n_envs, out_dev);
-    CUDA_TRY(cudaGetLastError());
-    return QLC_OK;
+    return on_caller_stream(env, stream, [&] {
+        stats_export_kernel<<<1, 1, 0, (cudaStream_t)stream>>>(env->stats, env->t * env->cfg.n_envs, out_dev);
+        CUDA_TRY(cudaGetLastError());
+        return QLC_OK;
+    });
 }
 // ---------------- statistics reduction over the env shards: NCCL behind the C ABI, on a side stream ----------------
 int32_t qlc_comm_unique_id(uint8_t* id128) {
@@ -1263,6 +1301,8 @@ int32_t qlc_env_load(qlc_env* env, const char* path) {
     fclose(f);
     ++env->generation;                               // the ring may have been (partly) overwritten, whether or not the load succeeds
     if (ok) ok = cudaMemcpy(env->stats, &h.stats, sizeof h.stats, cudaMemcpyHostToDevice) == cudaSuccess;
+    // a pageable host-to-device copy may return before its DMA lands: done before a step or an export on a non-blocking stream
+    if (ok) ok = cudaDeviceSynchronize() == cudaSuccess;
     if (!ok) return fail(QLC_ERR_CUDA, std::string("reading checkpoint failed (the env state is now undefined): ") + path);
     env->t = h.t; env->window = window;
     if (env->comm) env->comm->have_snap = false;     // the snapshots belong to the run that was replaced
@@ -1613,7 +1653,9 @@ static int32_t qnet_forward(qlc_qnet* q, const uint32_t* idx_dev, uint32_t n, in
 
 extern "C" int32_t qlc_qnet_forward(qlc_qnet* q, const uint32_t* idx_dev, uint32_t n, int32_t which, float* q_dev, uint8_t* action_dev, float* max_q_dev, void* stream) {
     QLC_RANGE("qlc_qnet_forward");
-    return qnet_forward(q, idx_dev, n, which, q_dev, action_dev, max_q_dev, false, stream);
+    if (!q) return fail(QLC_ERR_INVALID_ARG, "qnet is null");
+    if (!q->env) return fail(QLC_ERR_INVALID_ARG, "the environment of this Q-network has been destroyed");
+    return on_caller_stream(q->env, stream, [&] { return qnet_forward(q, idx_dev, n, which, q_dev, action_dev, max_q_dev, false, stream); });
 }
 
 extern "C" {
@@ -1627,12 +1669,13 @@ int32_t qlc_qnet_forward_host(qlc_qnet* q, const uint32_t* idx_host, uint32_t n,
     if (!idx_host) n = env->cfg.n_envs;
     if (n == 0) return QLC_OK;
     if (idx_host) { const uint64_t len = replay_len(env); for (uint32_t i = 0; i < n; ++i) if (idx_host[i] >= len) return fail(QLC_ERR_OUT_OF_RANGE, "replay index out of range"); }
+    rc = after_caller_stream(env); if (rc) return rc;
     const size_t o_idx = 0, o_q = ((size_t)n * 4 + 255) & ~(size_t)255, o_m = o_q + (size_t)n * 12, o_a = o_m + (size_t)n * 4, total = o_a + n;
     rc = ensure_dev_stage(env, total); if (rc) return rc;
     uint8_t* dev = (uint8_t*)env->dev_stage;
     cudaStream_t s = env->own_stream;
     if (idx_host) CUDA_TRY(cudaMemcpyAsync(dev + o_idx, idx_host, (size_t)n * 4, cudaMemcpyHostToDevice, s));
-    rc = qlc_qnet_forward(q, idx_host ? (const uint32_t*)(dev + o_idx) : nullptr, n, which, (float*)(dev + o_q), dev + o_a, (float*)(dev + o_m), s); if (rc) return rc;
+    rc = qnet_forward(q, idx_host ? (const uint32_t*)(dev + o_idx) : nullptr, n, which, (float*)(dev + o_q), dev + o_a, (float*)(dev + o_m), false, s); if (rc) return rc;
     if (q_host) CUDA_TRY(cudaMemcpyAsync(q_host, dev + o_q, (size_t)n * 12, cudaMemcpyDeviceToHost, s));
     if (max_q_host) CUDA_TRY(cudaMemcpyAsync(max_q_host, dev + o_m, (size_t)n * 4, cudaMemcpyDeviceToHost, s));
     if (action_host) CUDA_TRY(cudaMemcpyAsync(action_host, dev + o_a, n, cudaMemcpyDeviceToHost, s));
@@ -1789,13 +1832,10 @@ static int32_t check_train_args(qlc_qnet* q, const void* idx, uint32_t batch, ui
     return QLC_OK;
 }
 
-int32_t qlc_qnet_train_weighted(qlc_qnet* q, const uint32_t* idx_dev, const float* weight_dev, uint32_t batch, uint32_t n_batches, const float* target_dev,
-                                qlc_qnet* target_net, float gamma, float* loss_dev, float* td_dev, void* stream) {
-    QLC_RANGE("qlc_qnet_train_weighted");
-    int32_t rc = check_train_args(q, idx_dev, batch, n_batches, target_dev, target_net); if (rc) return rc;
-    if (n_batches == 0) return QLC_OK;
-    rc = set_device(q->env); if (rc) return rc;
-    cudaStream_t s = (cudaStream_t)stream;
+// the updates of one qlc_qnet_train(_weighted) call on `s` (arguments checked, n_batches > 0)
+static int32_t qnet_train_calls(qlc_qnet* q, const uint32_t* idx_dev, const float* weight_dev, uint32_t batch, uint32_t n_batches, const float* target_dev,
+                                qlc_qnet* target_net, float gamma, float* loss_dev, float* td_dev, cudaStream_t s) {
+    int32_t rc = QLC_OK;
     const uint32_t n = batch * n_batches;
     const float* y = target_dev;
     if (!y) {
@@ -1821,6 +1861,16 @@ int32_t qlc_qnet_train_weighted(qlc_qnet* q, const uint32_t* idx_dev, const floa
         if (rc) return rc;
     }
     return QLC_OK;
+}
+
+int32_t qlc_qnet_train_weighted(qlc_qnet* q, const uint32_t* idx_dev, const float* weight_dev, uint32_t batch, uint32_t n_batches, const float* target_dev,
+                                qlc_qnet* target_net, float gamma, float* loss_dev, float* td_dev, void* stream) {
+    QLC_RANGE("qlc_qnet_train_weighted");
+    int32_t rc = check_train_args(q, idx_dev, batch, n_batches, target_dev, target_net); if (rc) return rc;
+    if (n_batches == 0) return QLC_OK;
+    return on_caller_stream(q->env, stream, [&] {
+        return qnet_train_calls(q, idx_dev, weight_dev, batch, n_batches, target_dev, target_net, gamma, loss_dev, td_dev, (cudaStream_t)stream);
+    });
 }
 
 int32_t qlc_qnet_train(qlc_qnet* q, const uint32_t* idx_dev, uint32_t batch, uint32_t n_batches, const float* target_dev, qlc_qnet* target_net,
@@ -1853,10 +1903,11 @@ int32_t qlc_qnet_train_host(qlc_qnet* q, const uint32_t* idx_host, uint32_t batc
     int32_t rc = check_train_args(q, idx_host, batch, n_batches, target_host, target_net); if (rc) return rc;
     if (n_batches == 0) return QLC_OK;
     rc = set_device(q->env); if (rc) return rc;
+    rc = after_caller_stream(q->env); if (rc) return rc;
     uint32_t* idx_dev; float *y_dev, *w_dev, *loss_dev, *td_dev;
     rc = stage_train_inputs(q, idx_host, batch * n_batches, target_host, nullptr, n_batches, &idx_dev, &y_dev, &w_dev, &loss_dev, &td_dev); if (rc) return rc;
     cudaStream_t s = q->env->own_stream;
-    rc = qlc_qnet_train(q, idx_dev, batch, n_batches, y_dev, target_net, gamma, loss_host ? loss_dev : nullptr, s); if (rc) return rc;
+    rc = qnet_train_calls(q, idx_dev, nullptr, batch, n_batches, y_dev, target_net, gamma, loss_host ? loss_dev : nullptr, nullptr, s); if (rc) return rc;
     if (loss_host) CUDA_TRY(cudaMemcpyAsync(loss_host, loss_dev, (size_t)n_batches * 4, cudaMemcpyDeviceToHost, s));
     CUDA_TRY(cudaStreamSynchronize(s));
     uint32_t herr = 0;
@@ -1873,6 +1924,7 @@ int32_t qlc_qnet_debug_grads_weighted(qlc_qnet* q, const uint32_t* idx_host, uin
     weight_ptrs(grads_out, dst);
     for (int i = 0; i < qnet::NVARS; ++i) if (!dst[i]) return fail(QLC_ERR_INVALID_ARG, "a gradient pointer is null");
     rc = set_device(q->env); if (rc) return rc;
+    rc = after_caller_stream(q->env); if (rc) return rc;
     uint32_t* idx_dev; float *y_dev, *w_dev, *loss_dev, *td_dev;
     rc = stage_train_inputs(q, idx_host, n, target_host, weight_host, 1, &idx_dev, &y_dev, &w_dev, &loss_dev, &td_dev); if (rc) return rc;
     cudaStream_t s = q->env->own_stream;
@@ -2071,15 +2123,16 @@ int32_t qlc_per_sample(qlc_per* p, uint32_t batch, uint32_t n_batches, uint64_t 
     if (len == 0) return fail(QLC_ERR_NOT_ENOUGH, "the replay is empty");
     if (len >= 0xFFFFFFFFull) return fail(QLC_ERR_INVALID_ARG, "replay longer than 2^32-2 transitions");
     if (n_batches == 0) return QLC_OK;
-    rc = set_device(env); if (rc) return rc;
-    cudaStream_t s = (cudaStream_t)stream;
-    rc = per_sync(p, s); if (rc) return rc;
-    const uint32_t n = batch * n_batches;
-    const uint64_t oldest = env->t > env->t_cap ? env->t - env->t_cap : 0;
-    CUDA_TRY(launch_pdl(per::per_sample_kernel, dim3((n + 127) / 128), dim3(128), 0, s, p->tree, batch, n, call_index, env->cfg.seed, env->t, oldest,
-                        idx_dev, weight_dev));
-    if (weight_dev) CUDA_TRY(launch_pdl(per::per_weight_kernel, dim3(n_batches), dim3(256), 0, s, weight_dev, batch, beta));
-    return QLC_OK;
+    return on_caller_stream(env, stream, [&] {
+        cudaStream_t s = (cudaStream_t)stream;
+        int32_t rc = per_sync(p, s); if (rc) return rc;
+        const uint32_t n = batch * n_batches;
+        const uint64_t oldest = env->t > env->t_cap ? env->t - env->t_cap : 0;
+        CUDA_TRY(launch_pdl(per::per_sample_kernel, dim3((n + 127) / 128), dim3(128), 0, s, p->tree, batch, n, call_index, env->cfg.seed, env->t, oldest,
+                            idx_dev, weight_dev));
+        if (weight_dev) CUDA_TRY(launch_pdl(per::per_weight_kernel, dim3(n_batches), dim3(256), 0, s, weight_dev, batch, beta));
+        return QLC_OK;
+    });
 }
 
 int32_t qlc_per_update(qlc_per* p, const uint32_t* idx_dev, const float* td_dev, uint32_t n, void* stream) {
@@ -2089,17 +2142,18 @@ int32_t qlc_per_update(qlc_per* p, const uint32_t* idx_dev, const float* td_dev,
     qlc_env* env = p->env;
     const uint64_t len = replay_len(env);
     if (len >= 0xFFFFFFFFull) return fail(QLC_ERR_INVALID_ARG, "replay longer than 2^32-2 transitions");
-    rc = set_device(env); if (rc) return rc;
-    cudaStream_t s = (cudaStream_t)stream;
-    rc = per_sync(p, s); if (rc) return rc;
-    if (n == 0) return QLC_OK;
-    const uint64_t oldest = env->t > env->t_cap ? env->t - env->t_cap : 0;
-    const dim3 grid((n + 255) / 256);
-    CUDA_TRY(launch_pdl(per::per_update_clear_kernel, grid, dim3(256), 0, s, p->tree, idx_dev, td_dev, n, (uint32_t)len, oldest, p->alpha, p->epsilon));
-    CUDA_TRY(launch_pdl(per::per_update_set_kernel, grid, dim3(256), 0, s, p->tree, idx_dev, td_dev, n, (uint32_t)len, oldest, p->alpha, p->epsilon));
-    for (uint32_t level = 1; level <= p->tree.depth; ++level)
-        CUDA_TRY(launch_pdl(per::per_resum_items_kernel, grid, dim3(256), 0, s, p->tree, level, idx_dev, n, (uint32_t)len, oldest));
-    return QLC_OK;
+    return on_caller_stream(env, stream, [&] {
+        cudaStream_t s = (cudaStream_t)stream;
+        int32_t rc = per_sync(p, s); if (rc) return rc;
+        if (n == 0) return QLC_OK;
+        const uint64_t oldest = env->t > env->t_cap ? env->t - env->t_cap : 0;
+        const dim3 grid((n + 255) / 256);
+        CUDA_TRY(launch_pdl(per::per_update_clear_kernel, grid, dim3(256), 0, s, p->tree, idx_dev, td_dev, n, (uint32_t)len, oldest, p->alpha, p->epsilon));
+        CUDA_TRY(launch_pdl(per::per_update_set_kernel, grid, dim3(256), 0, s, p->tree, idx_dev, td_dev, n, (uint32_t)len, oldest, p->alpha, p->epsilon));
+        for (uint32_t level = 1; level <= p->tree.depth; ++level)
+            CUDA_TRY(launch_pdl(per::per_resum_items_kernel, grid, dim3(256), 0, s, p->tree, level, idx_dev, n, (uint32_t)len, oldest));
+        return QLC_OK;
+    });
 }
 
 int32_t qlc_per_read_host(qlc_per* p, float* leaves_host, double* total_host, float* max_priority_host) {
