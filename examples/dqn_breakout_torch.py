@@ -70,7 +70,8 @@ class TorchDQNModel:
 
 
 def run(n_envs=1024, iterations=200, batch=32, minibatches_per_call=None, seed=0, device=0, quiet=False, tensor_core_actor=False, actor_sync_every=10,
-        env_id_base=0, skip_model=False, random_phase_steps=None, tensor_core_learner=False, target_sync_every=250, prioritized=False):
+        env_id_base=0, skip_model=False, random_phase_steps=None, tensor_core_learner=False, target_sync_every=250, prioritized=False,
+        n_step=1, double_dqn=False):
     """Device-resident variant of learner.SelfDrivingQLearner.learn_iteration: same rules, tensors never leave the GPU.
     skip_model: run the data path only (step, replay insert, sample + gather, TD-target inputs) without the network calls —
     what is left of an iteration when the learner costs nothing (bench.py uses it to attribute the iteration time).
@@ -80,7 +81,11 @@ def run(n_envs=1024, iterations=200, batch=32, minibatches_per_call=None, seed=0
     network, which follows every `target_sync_every` iterations.
     prioritized (with tensor_core_learner): proportional prioritized replay (alpha 0.6) instead of uniform minibatches — one
     stratified minibatch of the same nb * batch items per iteration, importance weights with beta annealed linearly from 0.4 to
-    1.0 over the run, priorities updated from the TD errors of the update."""
+    1.0 over the run, priorities updated from the TD errors of the update.
+    n_step, double_dqn: TD targets from n-step returns read from the replay ring (qlc_replay_nstep), bootstrapped from the
+    state_next of the last transition walked; double_dqn takes Q_target there at the online network's greedy action instead of
+    max Q_target. The tensor-core learner computes them on the device; the torch learner gathers the bootstrap states and forms
+    y = G + disc * Q_boot in torch. n_step=1 without double_dqn is the one-step target above."""
     if prioritized and not tensor_core_learner:
         raise ValueError("prioritized replay runs on the tensor-core learner (tensor_core_learner=True)")
     dev = torch.device("cuda", device)
@@ -92,8 +97,8 @@ def run(n_envs=1024, iterations=200, batch=32, minibatches_per_call=None, seed=0
     rb = q.ReplayBuffer(env)
     model, target = TorchDQNModel(dev), TorchDQNModel(dev)
     target.load_from(model)
-    learner = tio.TensorCoreLearner(env, tio.keras_weights_from_torch(model.net), gamma=p.gamma.item(), per_alpha=0.6 if prioritized else None) \
-        if tensor_core_learner else None
+    learner = tio.TensorCoreLearner(env, tio.keras_weights_from_torch(model.net), gamma=p.gamma.item(), per_alpha=0.6 if prioritized else None,
+                                    n_step=n_step, double_dqn=double_dqn) if tensor_core_learner else None
     # optional: action selection on the library's tcgen05 Q-network, reading the frame ring directly (no f32 observation
     # is materialised); its weights follow the torch model every `actor_sync_every` iterations
     actor = tio.TensorCoreActor(env, model.net) if tensor_core_actor else None
@@ -101,6 +106,9 @@ def run(n_envs=1024, iterations=200, batch=32, minibatches_per_call=None, seed=0
     nb = minibatches_per_call or due_per_iter
     if learner is None:
         sampler = tio.DeviceSampler(rb, batch, nb, q.LAYOUT_F32_BXYH)
+        if n_step != 1 or double_dqn:
+            n_ret, n_disc = (torch.empty(nb * batch, dtype=torch.float32, device=dev) for _ in range(2))
+            n_boot = torch.empty(nb * batch, dtype=torch.int32, device=dev)
     else:
         idx = torch.empty((nb, batch), dtype=torch.int32, device=dev)
     gen = torch.Generator(device=dev); gen.manual_seed(seed)
@@ -146,9 +154,21 @@ def run(n_envs=1024, iterations=200, batch=32, minibatches_per_call=None, seed=0
                 st, nx = s.state.view(nb * batch, 84, 84, 4), s.state_next.view(nb * batch, 84, 84, 4)
                 if skip_model:
                     continue
-                max_future = target.batch_predict_max_future_reward(nx)
-                rwd, dn = s.reward.view(-1), s.done.view(-1)
-                updated_q = torch.where(dn != 0, rwd, rwd + p.gamma.item() * max_future)      # TD target (:192-199)
+                if n_step != 1 or double_dqn:
+                    # G, disc and the bootstrap index of every sampled transition; its state_next replaces the sampled one
+                    rb.nstep_device(s.indices.data_ptr(), nb * batch, n_step, p.gamma.item(), n_ret.data_ptr(), n_disc.data_ptr(), n_boot.data_ptr(), tio._stream())
+                    rb.gather_device(n_boot.data_ptr(), nb * batch, q.LAYOUT_F32_BXYH, None, s.state_next.data_ptr(), stream=tio._stream())
+                    with torch.no_grad():
+                        if double_dqn:
+                            a_star = model.predict_action(nx).long()
+                            q_boot = target.net(nx).gather(1, a_star.unsqueeze(1)).squeeze(1)
+                        else:
+                            q_boot = target.batch_predict_max_future_reward(nx)
+                    updated_q = n_ret + n_disc * q_boot
+                else:
+                    max_future = target.batch_predict_max_future_reward(nx)
+                    rwd, dn = s.reward.view(-1), s.done.view(-1)
+                    updated_q = torch.where(dn != 0, rwd, rwd + p.gamma.item() * max_future)      # TD target (:192-199)
                 model.train(st, s.action.view(-1), updated_q)
         if learner is not None and (it + 1) % target_sync_every == 0:
             learner.sync_target()
@@ -188,8 +208,10 @@ if __name__ == "__main__":
                     "on its tcgen05 Q-network, minibatches sampled as indices only")
     ap.add_argument("--tensor-core-actor", action="store_true", help="greedy actions from the library's tcgen05 Q-network (weights synced from the torch model)")
     ap.add_argument("--prioritized", action="store_true", help="with --tensor-core-learner: proportional prioritized replay (alpha 0.6, beta 0.4 -> 1.0)")
+    ap.add_argument("--n-step", type=int, default=1, help="TD targets from n-step returns read from the replay ring (1 = one-step)")
+    ap.add_argument("--double-dqn", action="store_true", help="double-DQN targets: Q_target at the online network's greedy action")
     args = ap.parse_args()
     if args.prioritized and not args.tensor_core_learner:
         ap.error("--prioritized needs --tensor-core-learner")
     print(run(args.envs, args.iterations, args.batch, tensor_core_actor=args.tensor_core_actor, tensor_core_learner=args.tensor_core_learner,
-              prioritized=args.prioritized))
+              prioritized=args.prioritized, n_step=args.n_step, double_dqn=args.double_dqn))

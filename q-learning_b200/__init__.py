@@ -56,6 +56,8 @@ ABI_SYMBOLS = [
     "qlc_qnet_train_weighted", "qlc_qnet_debug_grads_weighted",
     "qlc_per_create", "qlc_per_destroy", "qlc_per_sample", "qlc_per_update", "qlc_per_read_host",
 ]
+# the entry points include/ql_cuda_nstep.h declares (n-step returns and double-DQN targets)
+NSTEP_ABI_SYMBOLS = ["qlc_replay_nstep", "qlc_qnet_train_nstep"]
 
 
 class QlError(Exception):
@@ -203,6 +205,8 @@ def load_library(build_if_missing=True):
         "qlc_per_sample": (i32, [vp, u32, u32, u64, C.c_float, vp, vp, vp]),
         "qlc_per_update": (i32, [vp, vp, vp, u32, vp]),
         "qlc_per_read_host": (i32, [vp, vp, C.POINTER(C.c_double), C.POINTER(C.c_float)]),
+        "qlc_replay_nstep": (i32, [vp, vp, u32, u32, C.c_float, vp, vp, vp, vp]),
+        "qlc_qnet_train_nstep": (i32, [vp, vp, vp, u32, u32, vp, C.c_float, u32, i32, vp, vp, vp, vp]),
     }
     for name, (res, args) in sig.items():
         f = getattr(L, name)   # AttributeError if the library lacks a declared symbol
@@ -643,6 +647,11 @@ class ReplayBuffer:
     def gather_device(self, idx_ptr, n, layout, state_ptr, next_ptr, reward_ptr=None, action_ptr=None, done_ptr=None, stream=None):
         _check(self._L.qlc_replay_gather(self._env._h, idx_ptr, n, layout, state_ptr, next_ptr, reward_ptr, action_ptr, done_ptr, stream))
 
+    def nstep_device(self, idx_ptr, n, n_step, gamma, ret_ptr=None, disc_ptr=None, boot_ptr=None, stream=None):
+        """n-step returns of the n transitions idx_ptr (u32 logical indices): G f32 at ret_ptr, discount f32 at disc_ptr (gamma^m,
+        0 where terminal), and the logical index whose state_next bootstraps, u32 at boot_ptr (any may be None). Asynchronous."""
+        _check(self._L.qlc_replay_nstep(self._env._h, idx_ptr, n, n_step, gamma, ret_ptr, disc_ptr, boot_ptr, stream))
+
 
 def debug_collision_wall(which, center, radius, mv):
     """Run the DEVICE wall test on the GPU: (some, way, approximation, nx, ny, err)."""
@@ -800,6 +809,14 @@ class QNetwork:
         TD errors Q(s)[a] - y of every item written there (what PrioritizedReplay.update_device takes)."""
         _check(self._L.qlc_qnet_train_weighted(self._h, idx_ptr, weight_ptr, batch, n_batches, target_ptr, None if target_net is None else target_net._h,
                                                gamma, loss_ptr, td_ptr, stream))
+
+    def train_nstep_device(self, idx_ptr, weight_ptr, batch, n_batches, target_net, gamma=0.99, n_step=1, double_dqn=False, loss_ptr=None,
+                           td_ptr=None, y_ptr=None, stream=None):
+        """train_weighted_device with n-step targets (ReplayBuffer.nstep_device) bootstrapped from `target_net`: max_a Q_target,
+        or with `double_dqn` Q_target at the online network's greedy action. y_ptr (may be None) gets every item's target.
+        n_step=1, double_dqn=False is train_weighted_device's arithmetic."""
+        _check(self._L.qlc_qnet_train_nstep(self._h, idx_ptr, weight_ptr, batch, n_batches, target_net._h, gamma, n_step, 1 if double_dqn else 0,
+                                            loss_ptr, td_ptr, y_ptr, stream))
 
     def debug_grads_weighted(self, indices, targets, weights):
         """Forward + backward only of the loss mean(w * Huber): (gradients in the Keras layouts, TD errors f32 [n])."""

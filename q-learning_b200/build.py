@@ -19,9 +19,11 @@ HEADERS = [
     os.path.join(_HERE, "csrc", "qnet_conv.cuh"),
     os.path.join(_HERE, "csrc", "qnet_train.cuh"),
     os.path.join(_HERE, "csrc", "per.cuh"),
+    os.path.join(_HERE, "csrc", "nstep.cuh"),
     os.path.join(_HERE, "csrc", "host_pool.h"),
     os.path.join(_HERE, "csrc", "comm.h"),
     os.path.join(os.path.dirname(_HERE), "include", "ql_cuda.h"),
+    os.path.join(os.path.dirname(_HERE), "include", "ql_cuda_nstep.h"),
 ]
 # -fmad=false: the reference's Rust never contracts a*b+c; results must be bit-identical to that arithmetic.
 NVCC_FLAGS = [

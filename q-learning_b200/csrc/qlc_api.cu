@@ -1,11 +1,13 @@
 // qlc_api.cu — C ABI (include/ql_cuda.h) over the sm_100a kernels. No CPU fallback: every entry point that
 // computes needs a CUDA device and fails with QLC_ERR_NO_DEVICE / QLC_ERR_CUDA otherwise.
 #include "../../include/ql_cuda.h"
+#include "../../include/ql_cuda_nstep.h"
 #include "kernels.cuh"
 #include "qnet.cuh"
 #include "qnet_conv.cuh"
 #include "qnet_train.cuh"
 #include "per.cuh"
+#include "nstep.cuh"
 #include "host_pool.h"
 #include "comm.h"
 
@@ -1414,6 +1416,10 @@ struct qlc_qnet {
     float *t_q = nullptr, *t_dq = nullptr, *t_loss = nullptr, *t_dh = nullptr, *t_d3 = nullptr, *t_d2 = nullptr, *t_d1 = nullptr, *t_split = nullptr, *t_colsum = nullptr;
     __nv_bfloat16 *t_dh_bf = nullptr, *t_d3_bf = nullptr, *t_d2_bf = nullptr, *t_pack = nullptr;
     float *t_y = nullptr, *t_maxq = nullptr;
+    // n-step / double-DQN targets (qlc_qnet_train_nstep, sized for nstep_cap items): returns, discounts, bootstrap indices,
+    // target-network q [n][3], online greedy actions
+    uint32_t nstep_cap = 0;
+    float *t_ret = nullptr, *t_disc = nullptr, *t_tq = nullptr; uint32_t* t_boot = nullptr; uint8_t* t_act = nullptr;
     size_t split_floats = 0, pack_elems = 0;
 };
 
@@ -1427,6 +1433,8 @@ static void qnet_free_scratch(qlc_qnet* q) {
 // TD targets and target-network max-Q of one call (sized for y_cap items)
 static void qnet_free_targets(qlc_qnet* q) {
     cudaFree(q->t_y); cudaFree(q->t_maxq); q->t_y = q->t_maxq = nullptr; q->y_cap = 0;
+    cudaFree(q->t_ret); cudaFree(q->t_disc); cudaFree(q->t_tq); cudaFree(q->t_boot); cudaFree(q->t_act);
+    q->t_ret = q->t_disc = q->t_tq = nullptr; q->t_boot = nullptr; q->t_act = nullptr; q->nstep_cap = 0;
 }
 static void qnet_free_train(qlc_qnet* q) { qnet_free_scratch(q); qnet_free_targets(q); }
 
@@ -1943,6 +1951,103 @@ int32_t qlc_qnet_debug_grads(qlc_qnet* q, const uint32_t* idx_host, uint32_t n, 
 }
 
 // test hook: out[M][N] = act(bf16(a)[M][K] * bf16(w)[N][K]^T + bias) through the tcgen05 GEMM kernel (host f32 in / out)
+// ---------------- n-step returns and double-DQN targets (nstep.cuh, DESIGN §14) ----------------
+static int32_t check_nstep_args(uint32_t n_step, float gamma) {
+    if (n_step < 1 || n_step > QLC_NSTEP_MAX) return fail(QLC_ERR_INVALID_ARG, "n_step must be in [1, QLC_NSTEP_MAX]");
+    if (!(gamma >= 0.0f && gamma <= 1.0f)) return fail(QLC_ERR_INVALID_ARG, "gamma must be finite and in [0, 1]");
+    return QLC_OK;
+}
+// before anything reads a handle's env: a call that passes validation on a machine without a device fails here
+static int32_t check_device_present() {
+    int ndev = 0;
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) return fail(QLC_ERR_NO_DEVICE, "no CUDA device: ql_cuda has no CPU fallback");
+    return QLC_OK;
+}
+
+static cudaError_t launch_nstep(qlc_env* env, const uint32_t* idx_dev, uint32_t n, uint32_t n_step, float gamma, float* ret, float* disc, uint32_t* boot,
+                                cudaStream_t s) {
+    GatherParams g{}; fill_gather(env, g);
+    g.indices = idx_dev; g.n_items = n;
+    return launch_pdl(nstep::nstep_kernel, dim3((n + 127) / 128), dim3(128), 0, s, g, n_step, gamma, ret, disc, boot);
+}
+
+int32_t qlc_replay_nstep(qlc_env* env, const uint32_t* idx_dev, uint32_t n, uint32_t n_step, float gamma, float* return_dev, float* discount_dev,
+                         uint32_t* boot_idx_dev, void* stream) {
+    QLC_RANGE("qlc_replay_nstep");
+    int32_t rc = check_nstep_args(n_step, gamma); if (rc) return rc;
+    if (!env || !idx_dev) return fail(QLC_ERR_INVALID_ARG, "env/idx is null");
+    rc = check_device_present(); if (rc) return rc;
+    if (n == 0) return QLC_OK;
+    return on_caller_stream(env, stream, [&] {
+        CUDA_TRY(launch_nstep(env, idx_dev, n, n_step, gamma, return_dev, discount_dev, boot_idx_dev, (cudaStream_t)stream));
+        return QLC_OK;
+    });
+}
+
+// grows the n-step scratch (and t_y) to n items; allocation follows y_cap's rule: synchronise, free, allocate
+static int32_t qnet_nstep_alloc(qlc_qnet* q, uint32_t n) {
+    if (n > q->y_cap) {
+        CUDA_TRY(cudaDeviceSynchronize());
+        qnet_free_targets(q);
+        cudaError_t e = cudaMalloc(&q->t_y, (size_t)n * 4);
+        if (e == cudaSuccess) e = cudaMalloc(&q->t_maxq, (size_t)n * 4);
+        if (e != cudaSuccess) { cudaGetLastError(); qnet_free_targets(q); return fail(QLC_ERR_CUDA, std::string("qnet TD targets: ") + cudaGetErrorString(e)); }
+        q->y_cap = n;
+    }
+    if (n > q->nstep_cap) {
+        CUDA_TRY(cudaDeviceSynchronize());
+        cudaFree(q->t_ret); cudaFree(q->t_disc); cudaFree(q->t_tq); cudaFree(q->t_boot); cudaFree(q->t_act);
+        q->t_ret = q->t_disc = q->t_tq = nullptr; q->t_boot = nullptr; q->t_act = nullptr; q->nstep_cap = 0;
+        cudaError_t e = cudaMalloc(&q->t_ret, (size_t)n * 4);
+        if (e == cudaSuccess) e = cudaMalloc(&q->t_disc, (size_t)n * 4);
+        if (e == cudaSuccess) e = cudaMalloc(&q->t_boot, (size_t)n * 4);
+        if (e == cudaSuccess) e = cudaMalloc(&q->t_tq, (size_t)n * 12);
+        if (e == cudaSuccess) e = cudaMalloc(&q->t_act, (size_t)n);
+        if (e != cudaSuccess) { cudaGetLastError(); qnet_free_targets(q); return fail(QLC_ERR_CUDA, std::string("qnet n-step targets: ") + cudaGetErrorString(e)); }
+        q->nstep_cap = n;
+    }
+    return QLC_OK;
+}
+
+int32_t qlc_qnet_train_nstep(qlc_qnet* q, const uint32_t* idx_dev, const float* weight_dev, uint32_t batch, uint32_t n_batches, qlc_qnet* target_net,
+                             float gamma, uint32_t n_step, int32_t double_dqn, float* loss_dev, float* td_dev, float* y_dev, void* stream) {
+    QLC_RANGE("qlc_qnet_train_nstep");
+    int32_t rc = check_nstep_args(n_step, gamma); if (rc) return rc;
+    if (double_dqn != 0 && double_dqn != 1) return fail(QLC_ERR_INVALID_ARG, "double_dqn must be 0 or 1");
+    if (!target_net) return fail(QLC_ERR_INVALID_ARG, "target_net is null");
+    rc = check_train_args(q, idx_dev, batch, n_batches, nullptr, target_net); if (rc) return rc;
+    rc = check_device_present(); if (rc) return rc;
+    if (n_batches == 0) return QLC_OK;
+    return on_caller_stream(q->env, stream, [&] {
+        const cudaStream_t s = (cudaStream_t)stream;
+        const uint32_t n = batch * n_batches;
+        int32_t rc = qnet_nstep_alloc(q, n); if (rc) return rc;
+        float* const y = y_dev ? y_dev : q->t_y;
+        // G, disc, boot of the whole call; then the target network once, on the bootstrap states
+        CUDA_TRY(launch_nstep(q->env, idx_dev, n, n_step, gamma, q->t_ret, q->t_disc, q->t_boot, s));
+        rc = qnet_forward(target_net, q->t_boot, n, 1, double_dqn ? q->t_tq : nullptr, nullptr, double_dqn ? nullptr : q->t_maxq, false, s); if (rc) return rc;
+        GatherParams gp{}; fill_gather(q->env, gp);
+        gp.indices = q->t_boot; gp.n_items = n;
+        if (!double_dqn)
+            CUDA_TRY(launch_pdl(nstep::nstep_target_kernel, dim3((n + 255) / 256), dim3(256), 0, s, gp, (const float*)q->t_ret, (const float*)q->t_disc,
+                                (const float*)q->t_maxq, (const float*)nullptr, (const uint8_t*)nullptr, y));
+        for (uint32_t j = 0; j < n_batches; ++j) {
+            const size_t o = (size_t)j * batch;
+            if (double_dqn) {
+                // a* from the online weights after updates 0 .. j-1, so n_batches = k is k calls
+                rc = qnet_forward(q, q->t_boot + o, batch, 1, nullptr, q->t_act, nullptr, false, s); if (rc) return rc;
+                gp.indices = q->t_boot + o; gp.n_items = batch;
+                CUDA_TRY(launch_pdl(nstep::nstep_target_kernel, dim3((batch + 255) / 256), dim3(256), 0, s, gp, (const float*)q->t_ret + o,
+                                    (const float*)q->t_disc + o, (const float*)nullptr, (const float*)q->t_tq + o * 3, (const uint8_t*)q->t_act, y + o));
+            }
+            rc = qnet_train_step(q, idx_dev + o, batch, y + o, weight_dev ? weight_dev + o : nullptr, loss_dev ? loss_dev + j : nullptr,
+                                 td_dev ? td_dev + o : nullptr, true, s);
+            if (rc) return rc;
+        }
+        return QLC_OK;
+    });
+}
+
 int32_t qlc_debug_gemm_bf16(const float* a_host, const float* w_host, const float* bias_host, int32_t relu, float* out_host, uint32_t m, uint32_t n, uint32_t k) {
     if (!a_host || !w_host || !bias_host || !out_host) return fail(QLC_ERR_INVALID_ARG, "null pointer");
     if (k % qnet::KC != 0 || !(n == 32 || n == 64 || n == 128 || n == 256 || n == 512) || m == 0) return fail(QLC_ERR_INVALID_ARG, "need K % 64 == 0 and N in {32, 64, 128, 256, 512}");

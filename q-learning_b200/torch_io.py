@@ -125,11 +125,13 @@ class TensorCoreLearner:
     y = r + max Q_target(s') * gamma (y = r where done) computed on the device — and `sync_target()`. No state tensor is
     materialised anywhere: the kernels read the u8 frames where the step kernel wrote them. `weights`: Keras-layout f32 arrays
     (QNET_SHAPES) for both networks. `per_alpha` (not None): prioritized replay over the same ring (PrioritizedReplay), used by
-    `train_prioritized()`."""
+    `train_prioritized()`. `n_step` > 1 and `double_dqn`: both training calls bootstrap from n-step returns read from the ring
+    (DESIGN.md §14) and, with `double_dqn`, take Q_target at the online network's greedy action instead of max Q_target."""
 
-    def __init__(self, env, weights, gamma=0.99, lr=2.5e-4, clipnorm=1.0, per_alpha=None, per_epsilon=1e-6):
+    def __init__(self, env, weights, gamma=0.99, lr=2.5e-4, clipnorm=1.0, per_alpha=None, per_epsilon=1e-6, n_step=1, double_dqn=False):
         from . import PrioritizedReplay, QNetwork
         self.env, self.gamma = env, float(gamma)
+        self.n_step, self.double_dqn = int(n_step), bool(double_dqn)
         self.online = QNetwork(env, weights)
         self.target = QNetwork(env, weights)
         self.online.set_adam(lr=lr, clipnorm=clipnorm)
@@ -151,7 +153,11 @@ class TensorCoreLearner:
             raise QlError("indices must be a contiguous int32 CUDA tensor [n_batches][batch]")
         nb, batch = indices.shape
         loss = torch.empty(nb, dtype=torch.float32, device=indices.device)
-        self.online.train_device(indices.data_ptr(), batch, nb, None, self.target, self.gamma, loss.data_ptr(), _stream())
+        if self._nstep_targets():
+            self.online.train_nstep_device(indices.data_ptr(), None, batch, nb, self.target, self.gamma, self.n_step, self.double_dqn, loss.data_ptr(),
+                                           None, None, _stream())
+        else:
+            self.online.train_device(indices.data_ptr(), batch, nb, None, self.target, self.gamma, loss.data_ptr(), _stream())
         self.losses.append(loss)
         return loss
 
@@ -169,10 +175,17 @@ class TensorCoreLearner:
         s = _stream()
         loss = torch.empty(n_batches, dtype=torch.float32, device=dev)
         self.per.sample_device(batch, n_batches, call_index, beta, idx.data_ptr(), w.data_ptr(), s)
-        self.online.train_weighted_device(idx.data_ptr(), w.data_ptr(), batch, n_batches, None, self.target, self.gamma, loss.data_ptr(), td.data_ptr(), s)
+        if self._nstep_targets():
+            self.online.train_nstep_device(idx.data_ptr(), w.data_ptr(), batch, n_batches, self.target, self.gamma, self.n_step, self.double_dqn,
+                                           loss.data_ptr(), td.data_ptr(), None, s)
+        else:
+            self.online.train_weighted_device(idx.data_ptr(), w.data_ptr(), batch, n_batches, None, self.target, self.gamma, loss.data_ptr(), td.data_ptr(), s)
         self.per.update_device(idx.data_ptr(), td.data_ptr(), batch * n_batches, s)
         self.losses.append(loss)
         return loss
+
+    def _nstep_targets(self):
+        return self.n_step != 1 or self.double_dqn
 
     def sync_target(self):
         """target <- online (get + set of the f32 master weights)."""
