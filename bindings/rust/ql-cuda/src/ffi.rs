@@ -11,6 +11,7 @@ pub const QLC_COMM_ID_BYTES: usize = 128;
 pub const QLC_FRAME_W: usize = 84;
 pub const QLC_FRAME_H: usize = 84;
 pub const QLC_NUM_FRAMES: usize = 4;
+pub const QLC_NSTEP_MAX: u32 = 64;
 
 #[repr(C)]
 pub struct qlc_env {
@@ -206,6 +207,10 @@ extern "C" {
                                    target_net: *mut qlc_qnet, gamma: f32, loss_dev: *mut f32, td_dev: *mut f32, stream: *mut c_void) -> i32;
     pub fn qlc_qnet_debug_grads_weighted(qnet: *mut qlc_qnet, idx_host: *const u32, n: u32, target_host: *const f32, weight_host: *const f32,
                                          grads_out_host: *const qlc_qnet_weights, td_out_host: *mut f32) -> i32;
+    pub fn qlc_replay_nstep(env: *mut qlc_env, idx_dev: *const u32, n: u32, n_step: u32, gamma: f32, return_dev: *mut f32, discount_dev: *mut f32,
+                            boot_idx_dev: *mut u32, stream: *mut c_void) -> i32;
+    pub fn qlc_qnet_train_nstep(qnet: *mut qlc_qnet, idx_dev: *const u32, weight_dev: *const f32, batch: u32, n_batches: u32, target_net: *mut qlc_qnet,
+                                gamma: f32, n_step: u32, double_dqn: i32, loss_dev: *mut f32, td_dev: *mut f32, y_dev: *mut f32, stream: *mut c_void) -> i32;
     pub fn qlc_per_create(env: *mut qlc_env, alpha: f32, epsilon: f32, out: *mut *mut qlc_per) -> i32;
     pub fn qlc_per_destroy(per: *mut qlc_per) -> i32;
     pub fn qlc_per_sample(per: *mut qlc_per, batch: u32, n_batches: u32, call_index: u64, beta: f32, idx_dev: *mut u32, weight_dev: *mut f32,

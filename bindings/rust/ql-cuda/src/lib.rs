@@ -12,7 +12,6 @@
 //!   `self_driving_tf_q_learner.rs` is not touched at all — not even its `use` lines.
 //! * [`TensorCoreQModel`]: optional inference half of `DeepQLearningModel` on the library's tcgen05 Q-network.
 pub mod ffi;
-pub mod nstep_ffi;
 
 mod env;
 mod model;

@@ -53,11 +53,9 @@ ABI_SYMBOLS = [
     "qlc_debug_collision_wall", "qlc_debug_collision_rect", "qlc_debug_collision_rect_batch", "qlc_debug_gemm_bf16",
     "qlc_qnet_create", "qlc_qnet_set_weights", "qlc_qnet_destroy", "qlc_qnet_error", "qlc_qnet_forward", "qlc_qnet_forward_host",
     "qlc_qnet_set_adam", "qlc_qnet_get_weights", "qlc_qnet_train", "qlc_qnet_train_host", "qlc_qnet_debug_grads",
-    "qlc_qnet_train_weighted", "qlc_qnet_debug_grads_weighted",
+    "qlc_qnet_train_weighted", "qlc_qnet_debug_grads_weighted", "qlc_replay_nstep", "qlc_qnet_train_nstep",
     "qlc_per_create", "qlc_per_destroy", "qlc_per_sample", "qlc_per_update", "qlc_per_read_host",
 ]
-# the entry points include/ql_cuda_nstep.h declares (n-step returns and double-DQN targets)
-NSTEP_ABI_SYMBOLS = ["qlc_replay_nstep", "qlc_qnet_train_nstep"]
 
 
 class QlError(Exception):

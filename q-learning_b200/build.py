@@ -23,7 +23,6 @@ HEADERS = [
     os.path.join(_HERE, "csrc", "host_pool.h"),
     os.path.join(_HERE, "csrc", "comm.h"),
     os.path.join(os.path.dirname(_HERE), "include", "ql_cuda.h"),
-    os.path.join(os.path.dirname(_HERE), "include", "ql_cuda_nstep.h"),
 ]
 # -fmad=false: the reference's Rust never contracts a*b+c; results must be bit-identical to that arithmetic.
 NVCC_FLAGS = [

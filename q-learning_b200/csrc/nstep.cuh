@@ -4,7 +4,8 @@
 // strided walk over the u32 records [time_slots][N]. The walk over R_j = record (T + j, e) stops at the first j where R_j is done
 // (terminal), R_j is truncated, j = n_step - 1, T + j is the newest time in the replay, or R_{j+1} starts an episode
 // (min(k,4) = 0: a reset by the caller). Then m = j + 1, G = sum_j gamma^j r_j, disc = gamma^m (0 where terminal) and the
-// bootstrap state is state_next of boot = i + (m - 1) N. Both kernels are elementwise and use no atomics: deterministic.
+// bootstrap state is state_next of boot = i + (m - 1) N. The kernel is elementwise and uses no atomics: deterministic. The
+// targets y are formed by qnet::target_kernel (qnet_train.cuh).
 #pragma once
 #include "kernels.cuh"
 #include "qnet_conv.cuh"     // pdl_wait / pdl_launch_dependents
@@ -61,20 +62,6 @@ __global__ void nstep_kernel(GatherParams g, uint32_t n_step, float gamma, float
     if (ret) ret[i] = G;
     if (disc) disc[i] = d;
     if (boot) boot[i] = idx + (m - 1u) * g.n_envs;
-}
-
-// y [n] = G where terminal, else G + Q_boot * disc; g.indices = boot (its record's done bit is R_{m-1}'s: terminal). Q_boot is
-// max_q [n] (vanilla), or q [n][3] of the target network at the online network's greedy action [n] (double DQN, max_q NULL).
-__global__ void nstep_target_kernel(GatherParams g, const float* __restrict__ ret, const float* __restrict__ disc, const float* __restrict__ max_q,
-                                    const float* __restrict__ q, const uint8_t* __restrict__ action, float* __restrict__ y) {
-    pdl_launch_dependents(); pdl_wait();
-    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= g.n_items) return;
-    uint64_t T; uint32_t e, k, rec;
-    locate(g, i, g.indices[i], T, e, k, rec);
-    const float qb = max_q ? max_q[i] : q[(size_t)i * 3 + action[i]];
-    const float fut = qb * disc[i];
-    y[i] = ((rec >> 2) & 1u) ? ret[i] : ret[i] + fut;
 }
 
 }  // namespace nstep

@@ -1,7 +1,6 @@
 // qlc_api.cu — C ABI (include/ql_cuda.h) over the sm_100a kernels. No CPU fallback: every entry point that
 // computes needs a CUDA device and fails with QLC_ERR_NO_DEVICE / QLC_ERR_CUDA otherwise.
 #include "../../include/ql_cuda.h"
-#include "../../include/ql_cuda_nstep.h"
 #include "kernels.cuh"
 #include "qnet.cuh"
 #include "qnet_conv.cuh"
@@ -1415,11 +1414,10 @@ struct qlc_qnet {
     uint32_t train_cap = 0, y_cap = 0;
     float *t_q = nullptr, *t_dq = nullptr, *t_loss = nullptr, *t_dh = nullptr, *t_d3 = nullptr, *t_d2 = nullptr, *t_d1 = nullptr, *t_split = nullptr, *t_colsum = nullptr;
     __nv_bfloat16 *t_dh_bf = nullptr, *t_d3_bf = nullptr, *t_d2_bf = nullptr, *t_pack = nullptr;
-    float *t_y = nullptr, *t_maxq = nullptr;
-    // n-step / double-DQN targets (qlc_qnet_train_nstep, sized for nstep_cap items): returns, discounts, bootstrap indices,
-    // target-network q [n][3], online greedy actions
-    uint32_t nstep_cap = 0;
-    float *t_ret = nullptr, *t_disc = nullptr, *t_tq = nullptr; uint32_t* t_boot = nullptr; uint8_t* t_act = nullptr;
+    // targets of one call, sized for y_cap items: y, target-network max-Q; for n-step / double DQN also returns, discounts,
+    // bootstrap indices, target-network q [n][3], online greedy actions. All seven grow together, so a one-step call also holds
+    // the n-step arrays (25 bytes per item: 0.8 MB at 32,768 items) in exchange for one allocation rule.
+    float *t_y = nullptr, *t_maxq = nullptr, *t_ret = nullptr, *t_disc = nullptr, *t_tq = nullptr; uint32_t* t_boot = nullptr; uint8_t* t_act = nullptr;
     size_t split_floats = 0, pack_elems = 0;
 };
 
@@ -1430,11 +1428,10 @@ static void qnet_free_scratch(qlc_qnet* q) {
     q->t_q = q->t_dq = q->t_loss = q->t_dh = q->t_d3 = q->t_d2 = q->t_d1 = q->t_split = q->t_colsum = nullptr;
     q->t_dh_bf = q->t_d3_bf = q->t_d2_bf = q->t_pack = nullptr; q->train_cap = 0; q->split_floats = 0; q->pack_elems = 0;
 }
-// TD targets and target-network max-Q of one call (sized for y_cap items)
+// targets of one call (sized for y_cap items)
 static void qnet_free_targets(qlc_qnet* q) {
-    cudaFree(q->t_y); cudaFree(q->t_maxq); q->t_y = q->t_maxq = nullptr; q->y_cap = 0;
-    cudaFree(q->t_ret); cudaFree(q->t_disc); cudaFree(q->t_tq); cudaFree(q->t_boot); cudaFree(q->t_act);
-    q->t_ret = q->t_disc = q->t_tq = nullptr; q->t_boot = nullptr; q->t_act = nullptr; q->nstep_cap = 0;
+    cudaFree(q->t_y); cudaFree(q->t_maxq); cudaFree(q->t_ret); cudaFree(q->t_disc); cudaFree(q->t_tq); cudaFree(q->t_boot); cudaFree(q->t_act);
+    q->t_y = q->t_maxq = q->t_ret = q->t_disc = q->t_tq = nullptr; q->t_boot = nullptr; q->t_act = nullptr; q->y_cap = 0;
 }
 static void qnet_free_train(qlc_qnet* q) { qnet_free_scratch(q); qnet_free_targets(q); }
 
@@ -1840,31 +1837,78 @@ static int32_t check_train_args(qlc_qnet* q, const void* idx, uint32_t batch, ui
     return QLC_OK;
 }
 
-// the updates of one qlc_qnet_train(_weighted) call on `s` (arguments checked, n_batches > 0)
-static int32_t qnet_train_calls(qlc_qnet* q, const uint32_t* idx_dev, const float* weight_dev, uint32_t batch, uint32_t n_batches, const float* target_dev,
-                                qlc_qnet* target_net, float gamma, float* loss_dev, float* td_dev, cudaStream_t s) {
+// where the targets of a training call come from: given (y [n]), or from target_net (same env) as the one-step TD target of
+// the items' records (n_step = 0) or through the n-step walk (n_step >= 1; nstep.cuh, DESIGN §14), optionally double DQN
+struct TargetSource {
+    const float* y;
+    qlc_qnet* target_net;
+    float gamma;
+    uint32_t n_step;
+    bool double_dqn;
+};
+
+// grows the targets of one call to n items: synchronise, free, allocate (a failed allocation leaves y_cap = 0 and no stale pointers)
+static int32_t qnet_targets_alloc(qlc_qnet* q, uint32_t n) {
+    if (n <= q->y_cap) return QLC_OK;
+    CUDA_TRY(cudaDeviceSynchronize());
+    qnet_free_targets(q);
+    const size_t m = n;
+    cudaError_t e = cudaSuccess;
+    auto A = [&](void** p, size_t bytes) { if (e == cudaSuccess) e = cudaMalloc(p, bytes); };
+    A((void**)&q->t_y, m * 4); A((void**)&q->t_maxq, m * 4); A((void**)&q->t_ret, m * 4); A((void**)&q->t_disc, m * 4);
+    A((void**)&q->t_boot, m * 4); A((void**)&q->t_tq, m * 12); A((void**)&q->t_act, m);
+    if (e != cudaSuccess) { cudaGetLastError(); qnet_free_targets(q); return fail(QLC_ERR_CUDA, std::string("qnet TD targets: ") + cudaGetErrorString(e)); }
+    q->y_cap = n;
+    return QLC_OK;
+}
+
+static cudaError_t launch_nstep(qlc_env* env, const uint32_t* idx_dev, uint32_t n, uint32_t n_step, float gamma, float* ret, float* disc, uint32_t* boot,
+                                cudaStream_t s) {
+    GatherParams g{}; fill_gather(env, g);
+    g.indices = idx_dev; g.n_items = n;
+    return launch_pdl(nstep::nstep_kernel, dim3((n + 127) / 128), dim3(128), 0, s, g, n_step, gamma, ret, disc, boot);
+}
+
+// the updates of one training call on `s` (arguments checked, n_batches > 0). Computed targets are written to y_out [n] if it
+// is given, else to the network's scratch. The target network runs once per call; with double DQN the online network's
+// greedy action for minibatch j comes from the weights after updates 0 .. j-1, so n_batches = k is k calls.
+static int32_t qnet_train_calls(qlc_qnet* q, const uint32_t* idx_dev, const float* weight_dev, uint32_t batch, uint32_t n_batches, const TargetSource& t,
+                                float* loss_dev, float* td_dev, float* y_out, cudaStream_t s) {
     int32_t rc = QLC_OK;
     const uint32_t n = batch * n_batches;
-    const float* y = target_dev;
-    if (!y) {
-        // TD targets of the whole call from the (fixed) target network: max_a Q_target(state_next), then r / done of the records
-        if (n > q->y_cap) {
-            CUDA_TRY(cudaDeviceSynchronize());
-            qnet_free_targets(q);
-            cudaError_t e = cudaMalloc(&q->t_y, (size_t)n * 4);
-            if (e == cudaSuccess) e = cudaMalloc(&q->t_maxq, (size_t)n * 4);
-            if (e != cudaSuccess) { cudaGetLastError(); qnet_free_targets(q); return fail(QLC_ERR_CUDA, std::string("qnet TD targets: ") + cudaGetErrorString(e)); }
-            q->y_cap = n;
+    GatherParams gp{}; fill_gather(q->env, gp);
+    // y [m] = target_kernel over gp.indices [m]: G = ret or r of the record, d = disc or gamma, Q_boot = max_q or tq at t_act
+    auto target = [&](uint32_t m, const float* ret, const float* disc, const float* max_q, const float* tq, float* y) {
+        gp.n_items = m;
+        return launch_pdl(qnet::target_kernel, dim3((m + 255) / 256), dim3(256), 0, s, gp, ret, disc, t.gamma, max_q, tq,
+                          (const uint8_t*)(tq ? q->t_act : nullptr), y);
+    };
+    float* y = nullptr;
+    if (!t.y) {
+        rc = qnet_targets_alloc(q, n); if (rc) return rc;
+        y = y_out ? y_out : q->t_y;
+        if (t.n_step == 0) {
+            rc = qnet_forward(t.target_net, idx_dev, n, 1, nullptr, nullptr, q->t_maxq, false, s); if (rc) return rc;
+            gp.indices = idx_dev;
+            CUDA_TRY(target(n, nullptr, nullptr, q->t_maxq, nullptr, y));
+        } else {
+            // G, disc, boot of the whole call; then the target network on the bootstrap states
+            CUDA_TRY(launch_nstep(q->env, idx_dev, n, t.n_step, t.gamma, q->t_ret, q->t_disc, q->t_boot, s));
+            rc = qnet_forward(t.target_net, q->t_boot, n, 1, t.double_dqn ? q->t_tq : nullptr, nullptr, t.double_dqn ? nullptr : q->t_maxq, false, s);
+            if (rc) return rc;
+            gp.indices = q->t_boot;
+            if (!t.double_dqn) CUDA_TRY(target(n, q->t_ret, q->t_disc, q->t_maxq, nullptr, y));
         }
-        rc = qnet_forward(target_net, idx_dev, n, 1, nullptr, nullptr, q->t_maxq, false, s); if (rc) return rc;
-        GatherParams gp{}; fill_gather(q->env, gp);
-        gp.indices = idx_dev; gp.n_items = n; gp.mode = GATHER_INDICES;
-        CUDA_TRY(launch_pdl(qnet::td_target_kernel, dim3((n + 255) / 256), dim3(256), 0, s, gp, (const float*)q->t_maxq, gamma, q->t_y));
-        y = q->t_y;
     }
+    const float* const y_in = t.y ? t.y : y;
     for (uint32_t j = 0; j < n_batches; ++j) {
         const size_t o = (size_t)j * batch;
-        rc = qnet_train_step(q, idx_dev + o, batch, y + o, weight_dev ? weight_dev + o : nullptr, loss_dev ? loss_dev + j : nullptr,
+        if (t.double_dqn) {
+            rc = qnet_forward(q, q->t_boot + o, batch, 1, nullptr, q->t_act, nullptr, false, s); if (rc) return rc;
+            gp.indices = q->t_boot + o;
+            CUDA_TRY(target(batch, q->t_ret + o, q->t_disc + o, nullptr, q->t_tq + o * 3, y + o));
+        }
+        rc = qnet_train_step(q, idx_dev + o, batch, y_in + o, weight_dev ? weight_dev + o : nullptr, loss_dev ? loss_dev + j : nullptr,
                              td_dev ? td_dev + o : nullptr, true, s);
         if (rc) return rc;
     }
@@ -1877,7 +1921,8 @@ int32_t qlc_qnet_train_weighted(qlc_qnet* q, const uint32_t* idx_dev, const floa
     int32_t rc = check_train_args(q, idx_dev, batch, n_batches, target_dev, target_net); if (rc) return rc;
     if (n_batches == 0) return QLC_OK;
     return on_caller_stream(q->env, stream, [&] {
-        return qnet_train_calls(q, idx_dev, weight_dev, batch, n_batches, target_dev, target_net, gamma, loss_dev, td_dev, (cudaStream_t)stream);
+        return qnet_train_calls(q, idx_dev, weight_dev, batch, n_batches, TargetSource{target_dev, target_net, gamma, 0, false}, loss_dev, td_dev, nullptr,
+                                (cudaStream_t)stream);
     });
 }
 
@@ -1915,7 +1960,9 @@ int32_t qlc_qnet_train_host(qlc_qnet* q, const uint32_t* idx_host, uint32_t batc
     uint32_t* idx_dev; float *y_dev, *w_dev, *loss_dev, *td_dev;
     rc = stage_train_inputs(q, idx_host, batch * n_batches, target_host, nullptr, n_batches, &idx_dev, &y_dev, &w_dev, &loss_dev, &td_dev); if (rc) return rc;
     cudaStream_t s = q->env->own_stream;
-    rc = qnet_train_calls(q, idx_dev, nullptr, batch, n_batches, y_dev, target_net, gamma, loss_host ? loss_dev : nullptr, nullptr, s); if (rc) return rc;
+    rc = qnet_train_calls(q, idx_dev, nullptr, batch, n_batches, TargetSource{y_dev, target_net, gamma, 0, false}, loss_host ? loss_dev : nullptr, nullptr,
+                          nullptr, s);
+    if (rc) return rc;
     if (loss_host) CUDA_TRY(cudaMemcpyAsync(loss_host, loss_dev, (size_t)n_batches * 4, cudaMemcpyDeviceToHost, s));
     CUDA_TRY(cudaStreamSynchronize(s));
     uint32_t herr = 0;
@@ -1950,7 +1997,6 @@ int32_t qlc_qnet_debug_grads(qlc_qnet* q, const uint32_t* idx_host, uint32_t n, 
     return qlc_qnet_debug_grads_weighted(q, idx_host, n, target_host, nullptr, grads_out, nullptr);
 }
 
-// test hook: out[M][N] = act(bf16(a)[M][K] * bf16(w)[N][K]^T + bias) through the tcgen05 GEMM kernel (host f32 in / out)
 // ---------------- n-step returns and double-DQN targets (nstep.cuh, DESIGN §14) ----------------
 static int32_t check_nstep_args(uint32_t n_step, float gamma) {
     if (n_step < 1 || n_step > QLC_NSTEP_MAX) return fail(QLC_ERR_INVALID_ARG, "n_step must be in [1, QLC_NSTEP_MAX]");
@@ -1962,13 +2008,6 @@ static int32_t check_device_present() {
     int ndev = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) return fail(QLC_ERR_NO_DEVICE, "no CUDA device: ql_cuda has no CPU fallback");
     return QLC_OK;
-}
-
-static cudaError_t launch_nstep(qlc_env* env, const uint32_t* idx_dev, uint32_t n, uint32_t n_step, float gamma, float* ret, float* disc, uint32_t* boot,
-                                cudaStream_t s) {
-    GatherParams g{}; fill_gather(env, g);
-    g.indices = idx_dev; g.n_items = n;
-    return launch_pdl(nstep::nstep_kernel, dim3((n + 127) / 128), dim3(128), 0, s, g, n_step, gamma, ret, disc, boot);
 }
 
 int32_t qlc_replay_nstep(qlc_env* env, const uint32_t* idx_dev, uint32_t n, uint32_t n_step, float gamma, float* return_dev, float* discount_dev,
@@ -1984,31 +2023,6 @@ int32_t qlc_replay_nstep(qlc_env* env, const uint32_t* idx_dev, uint32_t n, uint
     });
 }
 
-// grows the n-step scratch (and t_y) to n items; allocation follows y_cap's rule: synchronise, free, allocate
-static int32_t qnet_nstep_alloc(qlc_qnet* q, uint32_t n) {
-    if (n > q->y_cap) {
-        CUDA_TRY(cudaDeviceSynchronize());
-        qnet_free_targets(q);
-        cudaError_t e = cudaMalloc(&q->t_y, (size_t)n * 4);
-        if (e == cudaSuccess) e = cudaMalloc(&q->t_maxq, (size_t)n * 4);
-        if (e != cudaSuccess) { cudaGetLastError(); qnet_free_targets(q); return fail(QLC_ERR_CUDA, std::string("qnet TD targets: ") + cudaGetErrorString(e)); }
-        q->y_cap = n;
-    }
-    if (n > q->nstep_cap) {
-        CUDA_TRY(cudaDeviceSynchronize());
-        cudaFree(q->t_ret); cudaFree(q->t_disc); cudaFree(q->t_tq); cudaFree(q->t_boot); cudaFree(q->t_act);
-        q->t_ret = q->t_disc = q->t_tq = nullptr; q->t_boot = nullptr; q->t_act = nullptr; q->nstep_cap = 0;
-        cudaError_t e = cudaMalloc(&q->t_ret, (size_t)n * 4);
-        if (e == cudaSuccess) e = cudaMalloc(&q->t_disc, (size_t)n * 4);
-        if (e == cudaSuccess) e = cudaMalloc(&q->t_boot, (size_t)n * 4);
-        if (e == cudaSuccess) e = cudaMalloc(&q->t_tq, (size_t)n * 12);
-        if (e == cudaSuccess) e = cudaMalloc(&q->t_act, (size_t)n);
-        if (e != cudaSuccess) { cudaGetLastError(); qnet_free_targets(q); return fail(QLC_ERR_CUDA, std::string("qnet n-step targets: ") + cudaGetErrorString(e)); }
-        q->nstep_cap = n;
-    }
-    return QLC_OK;
-}
-
 int32_t qlc_qnet_train_nstep(qlc_qnet* q, const uint32_t* idx_dev, const float* weight_dev, uint32_t batch, uint32_t n_batches, qlc_qnet* target_net,
                              float gamma, uint32_t n_step, int32_t double_dqn, float* loss_dev, float* td_dev, float* y_dev, void* stream) {
     QLC_RANGE("qlc_qnet_train_nstep");
@@ -2019,34 +2033,12 @@ int32_t qlc_qnet_train_nstep(qlc_qnet* q, const uint32_t* idx_dev, const float* 
     rc = check_device_present(); if (rc) return rc;
     if (n_batches == 0) return QLC_OK;
     return on_caller_stream(q->env, stream, [&] {
-        const cudaStream_t s = (cudaStream_t)stream;
-        const uint32_t n = batch * n_batches;
-        int32_t rc = qnet_nstep_alloc(q, n); if (rc) return rc;
-        float* const y = y_dev ? y_dev : q->t_y;
-        // G, disc, boot of the whole call; then the target network once, on the bootstrap states
-        CUDA_TRY(launch_nstep(q->env, idx_dev, n, n_step, gamma, q->t_ret, q->t_disc, q->t_boot, s));
-        rc = qnet_forward(target_net, q->t_boot, n, 1, double_dqn ? q->t_tq : nullptr, nullptr, double_dqn ? nullptr : q->t_maxq, false, s); if (rc) return rc;
-        GatherParams gp{}; fill_gather(q->env, gp);
-        gp.indices = q->t_boot; gp.n_items = n;
-        if (!double_dqn)
-            CUDA_TRY(launch_pdl(nstep::nstep_target_kernel, dim3((n + 255) / 256), dim3(256), 0, s, gp, (const float*)q->t_ret, (const float*)q->t_disc,
-                                (const float*)q->t_maxq, (const float*)nullptr, (const uint8_t*)nullptr, y));
-        for (uint32_t j = 0; j < n_batches; ++j) {
-            const size_t o = (size_t)j * batch;
-            if (double_dqn) {
-                // a* from the online weights after updates 0 .. j-1, so n_batches = k is k calls
-                rc = qnet_forward(q, q->t_boot + o, batch, 1, nullptr, q->t_act, nullptr, false, s); if (rc) return rc;
-                gp.indices = q->t_boot + o; gp.n_items = batch;
-                CUDA_TRY(launch_pdl(nstep::nstep_target_kernel, dim3((batch + 255) / 256), dim3(256), 0, s, gp, (const float*)q->t_ret + o,
-                                    (const float*)q->t_disc + o, (const float*)nullptr, (const float*)q->t_tq + o * 3, (const uint8_t*)q->t_act, y + o));
-            }
-            rc = qnet_train_step(q, idx_dev + o, batch, y + o, weight_dev ? weight_dev + o : nullptr, loss_dev ? loss_dev + j : nullptr,
-                                 td_dev ? td_dev + o : nullptr, true, s);
-            if (rc) return rc;
-        }
-        return QLC_OK;
+        return qnet_train_calls(q, idx_dev, weight_dev, batch, n_batches, TargetSource{nullptr, target_net, gamma, n_step, double_dqn != 0}, loss_dev, td_dev,
+                                y_dev, (cudaStream_t)stream);
     });
 }
+
+// test hook: out[M][N] = act(bf16(a)[M][K] * bf16(w)[N][K]^T + bias) through the tcgen05 GEMM kernel (host f32 in / out)
 
 int32_t qlc_debug_gemm_bf16(const float* a_host, const float* w_host, const float* bias_host, int32_t relu, float* out_host, uint32_t m, uint32_t n, uint32_t k) {
     if (!a_host || !w_host || !bias_host || !out_host) return fail(QLC_ERR_INVALID_ARG, "null pointer");

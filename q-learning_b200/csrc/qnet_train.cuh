@@ -189,16 +189,22 @@ __global__ void colsum_final_kernel(const float* __restrict__ partial, uint32_t 
     out[col] = t / div;
 }
 
-// ---- TD target: y = r + maxQ_target(s') * gamma, y = r where done (learner.py; -fmad=false: the multiply rounds first) ----
-__global__ void td_target_kernel(GatherParams g, const float* __restrict__ max_q, float gamma, float* __restrict__ y) {
+// ---- target: y [n] = G where the record of g.indices [i] is done, else G + Q_boot * d (-fmad=false: the multiply rounds first).
+// One-step TD target (learner.py): g.indices = the items, ret = disc = NULL, so G = r of their record and d = gamma. n-step
+// (nstep.cuh, DESIGN §14): g.indices = boot, whose record's done bit is R_{m-1}'s (terminal), G = ret [n], d = disc [n].
+// Q_boot is max_q [n], or q [n][3] of the target network at the online network's greedy action [n] (double DQN, max_q NULL). ----
+__global__ void target_kernel(GatherParams g, const float* __restrict__ ret, const float* __restrict__ disc, float gamma, const float* __restrict__ max_q,
+                              const float* __restrict__ q, const uint8_t* __restrict__ action, float* __restrict__ y) {
     pdl_launch_dependents(); pdl_wait();
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= g.n_items) return;
     uint64_t T; uint32_t e, k, rec;
     locate(g, i, g.indices[i], T, e, k, rec);
-    const float r = (float)((rec >> 8) & 0xFFu);
-    const float fut = max_q[i] * gamma;
-    y[i] = ((rec >> 2) & 1u) ? r : r + fut;
+    const float G = ret ? ret[i] : (float)((rec >> 8) & 0xFFu);
+    const float d = disc ? disc[i] : gamma;
+    const float qb = max_q ? max_q[i] : q[(size_t)i * 3 + action[i]];
+    const float fut = qb * d;
+    y[i] = ((rec >> 2) & 1u) ? G : G + fut;
 }
 
 // ---- head backward (CUDA cores, one warp per item): Huber(delta 1) on Q(s)[a], weighted by w [B] (NULL = 1), averaged over

@@ -3,7 +3,8 @@ against the numpy model of tests/test_nstep_abi.py, bit for bit:
 
 1. qlc_replay_nstep for every logical index of wrapped rings (1, 37 and 4,096 envs), auto-reset on and off with resets by the
    caller, truncating episode limits, n_step 1 to 64, gamma 0 to 1, and indices >= len.
-2. n_step = 1 without double DQN is qlc_qnet_train_weighted (weighted and unweighted) and qlc_qnet_train.
+2. n_step = 1 without double DQN is qlc_qnet_train_weighted (weighted and unweighted) and qlc_qnet_train, except at an index
+   >= len, where the one-step target bootstraps from the zero stack and the n-step target is 0.
 3. The targets equal the model's y built from qlc_replay_nstep and qlc_qnet_forward on the bootstrap states.
 4. Each minibatch is qlc_qnet_train_weighted on the targets y_dev reports; n_batches = 3 is 3 calls; runs repeat bit for bit.
 5. The prioritized learner feeds its n-step double-DQN TD errors to the tree.
@@ -171,6 +172,35 @@ def test_one_step_is_the_weighted_update(qlb):
         for n in (a, b, c):
             n.close()
     target.close(); env.close()
+
+
+def test_one_step_target_of_an_index_beyond_len(qlb):
+    """Where the one-step and the n-step targets differ: an index >= len has record 0 and the all-zero stacks. The one-step
+    target is then y = 0 + maxQ_target(zero stack)·gamma with action 0, so td = Q_online(zero stack)[0] - y; the n-step walk
+    gives G = 0, disc = 0, so y = 0."""
+    env, rb = _setup(qlb, seed=8)
+    w0, w1 = _random_weights(qlb, 51), _random_weights(qlb, 52)
+    target = qlb.QNetwork(env, w1)
+    batch, gamma, k = 32, 0.99, 7
+    idx_np = np.random.default_rng(5).integers(0, rb.len(), size=batch).astype(np.uint32)
+    idx_np[k] = rb.len() + 5
+    idx = _dev_idx(idx_np)
+    a, b = _nets(qlb, env, w0, 2)
+    q_on, max_t = torch.empty((batch, 3), dtype=torch.float32, device="cuda"), torch.empty(batch, dtype=torch.float32, device="cuda")
+    a.forward_device(idx.data_ptr(), batch, 0, q_on.data_ptr(), None, None, _s())          # the online weights before the update
+    target.forward_device(idx.data_ptr(), batch, 1, None, None, max_t.data_ptr(), _s())
+    loss, td, y = _bufs(1, batch)
+    a.train_weighted_device(idx.data_ptr(), None, batch, 1, None, target, gamma, loss.data_ptr(), td.data_ptr(), _s())
+    b.train_nstep_device(idx.data_ptr(), None, batch, 1, target, gamma, 1, False, None, None, y.data_ptr(), _s())
+    torch.cuda.synchronize()
+    assert a.error() == 0 and b.error() == 0
+    q0, mt = q_on.cpu().numpy()[k, 0], max_t.cpu().numpy()[k]
+    want = np.float32(q0 - np.float32(mt * np.float32(gamma)))
+    assert _bits(td.cpu().numpy()[k]) == _bits(want), (td.cpu().numpy()[k], want)
+    assert y.cpu().numpy()[k] == 0.0
+    for n in (a, b, target):
+        n.close()
+    env.close()
 
 
 # ---------------------------------------------------------------- 3. targets

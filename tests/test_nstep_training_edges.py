@@ -11,10 +11,8 @@ for bit, +0 and -0 equal. td is compared bit for bit with Q(s)[a] - y from the f
    minibatch each) on either side of the narrow / wide boundary, and 32,768 items on a 1 M-transition ring.
 3. Scratch growth and reuse: n-step, plain and weighted calls of one network on a side stream at growing and shrinking sizes,
    each equal to a fresh twin that makes only that call.
-4. Stream order of include/ql_cuda_nstep.h: every entry point has a rule; both calls see submitted host steps; host calls of
-   the network wait for an n-step update queued behind a sleep."""
-import os
-import re
+4. Stream order of the two n-step calls: both are under test_stream_order.py's asynchronous rule and see submitted host steps;
+   host calls of the network wait for an n-step update queued behind a sleep."""
 import time
 from types import SimpleNamespace
 
@@ -28,8 +26,6 @@ from test_qnet_batch_edges import _random_weights, _size
 
 torch = pytest.importorskip("torch")
 gpu = pytest.mark.gpu
-
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 DONE, TRUNCATION, RESET, NEWEST, N_STEP = range(5)
 KINDS = ("done", "truncation", "reset by the caller", "newest time", "n_step reached")
@@ -153,22 +149,11 @@ def test_dense_shapes_straddle_the_boundary(sm):
     assert sides == [(False, True), (False, True), (False, False), (False, False)]
 
 
-# ---------------------------------------------------------------- 4a. every entry point of ql_cuda_nstep.h has an ordering rule
-RULES = {   # the rule names of test_stream_order.py's tables
-    "qlc_replay_nstep": "async",          # queued on the caller's stream after submitted host steps; caller_done recorded after
-    "qlc_qnet_train_nstep": "async",
-}
-
-
-def test_every_nstep_entry_point_has_an_ordering_rule(qlb):
-    """A new qlc_* function in include/ql_cuda_nstep.h must be placed in RULES, and have a consumer test below if it is
-    asynchronous."""
-    text = re.sub(r"/\*.*?\*/", " ", open(os.path.join(ROOT, "include", "ql_cuda_nstep.h")).read(), flags=re.S)
-    declared = set(re.findall(r"\b(qlc_\w+)\s*\(", text))
-    assert declared == set(RULES) == set(qlb.NSTEP_ABI_SYMBOLS)
-    assert set(RULES.values()) <= {"async", "host_ordered", "synchronises", "exempt"}
-    assert not set(RULES) & (so.ASYNC | so.HOST_ORDERED | so.SYNCHRONISES | set(so.EXEMPT)), "listed in both files"
-    assert {s for s, r in RULES.items() if r == "async"} == set(SUBMITTED_CONSUMERS.values())
+# ---------------------------------------------------------------- 4a. both n-step calls are asynchronous and have a consumer test
+def test_every_nstep_entry_point_has_an_ordering_rule():
+    """test_stream_order.py places both calls under its asynchronous rule; each has a submitted-steps consumer case below."""
+    assert {"qlc_replay_nstep", "qlc_qnet_train_nstep"} <= so.ASYNC
+    assert {"qlc_replay_nstep", "qlc_qnet_train_nstep"} == set(SUBMITTED_CONSUMERS.values())
 
 
 # ---------------------------------------------------------------- GPU helpers

@@ -30,7 +30,7 @@ BIG_N, BIG_T_CAP = 16384, 8               # pipelined submits: above 96 x SMs, s
 ASYNC = {   # queued on the caller's stream after submitted host steps; caller_done recorded after the launches
     "qlc_env_step", "qlc_env_step_random", "qlc_env_obs", "qlc_obs_gather", "qlc_replay_sample", "qlc_replay_gather",
     "qlc_replay_sample_gather", "qlc_stats_export", "qlc_qnet_forward", "qlc_qnet_train", "qlc_qnet_train_weighted",
-    "qlc_per_sample", "qlc_per_update",
+    "qlc_per_sample", "qlc_per_update", "qlc_replay_nstep", "qlc_qnet_train_nstep",
 }
 HOST_ORDERED = {   # host buffers on the env's own stream, which first waits for caller_done
     "qlc_env_step_host", "qlc_env_step_host_submit", "qlc_env_obs_host", "qlc_obs_gather_host", "qlc_replay_sample_host",
